@@ -11,7 +11,7 @@ step path).  One "step" = one time step of all members of the batch:
 convection re-evaluation (K1a), right-hand side (K2), saddle-point solve (K3).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--members B]
-                    [--mesh 4] [--impl ours|reference]
+                    [--mesh 4] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `--impl reference` times the CPU restatement of
 the reference's scipy path (oracle/: SuperLU + compiled cell loop) on the box's
@@ -67,7 +67,13 @@ def parse():
                     help='do not pin the ranks of a multi-GPU run to the cores next to their GPU')
     ap.add_argument('--no-parity', action='store_true',
                     help='skip the CPU-oracle check of the measured trajectory')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the state (v, p of every member) after the last timed step as DIR/v.npy, '
+                         'DIR/p.npy (float64, at most 64 MB together), to compare builds output for output')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the device path computed: use it with --impl ours')
+    return args
 
 
 # --------------------------------------------------------------------------
@@ -565,6 +571,40 @@ def secondary_records(args, ctx):
 # --------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------
+DUMP_BYTES = 64*10**6
+
+
+def gather_members(a, world):
+    """(n, members of this rank) -> (n, members of every rank) in rank order;
+    every rank holds the same number of members"""
+    if world == 1:
+        return a
+    import torch
+    import torch.distributed as dist
+    t = torch.from_numpy(np.ascontiguousarray(a)).cuda()
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t)
+    return torch.cat(parts, dim=1).cpu().numpy()
+
+
+def dump_outputs(dirname, arrays):
+    """``arrays``: name -> (n, members) float64.  Above DUMP_BYTES in all, a
+    fixed seeded sample of the members (the same columns of every array) is
+    written, so that runs with the same arguments write the same entries."""
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 4096             # room for the .npy headers
+    ncols = next(iter(arrays.values())).shape[1]
+    cols = slice(None)
+    if total > budget:
+        keep = max(1, ncols*budget//total)
+        cols = np.sort(np.random.default_rng(0).choice(ncols, keep, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        out = np.ascontiguousarray(a[:, cols], dtype=np.float64)
+        np.save(os.path.join(dirname, name + '.npy'), out)
+        print('dump-outputs: %s.npy %s' % (name, out.shape), file=sys.stderr)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -623,9 +663,14 @@ def run_ours(args, rank, world, local_rank):
     value = units/(dev_ms_max*1e-3)
     # state after spin-up + warm-up + timed steps: checked against the CPU
     # oracle (first and last member of rank 0's shard) once the timing is over
+    if args.dump_outputs or (rank == 0 and not args.no_parity):
+        Vd, Pd = integ.state()
+    if args.dump_outputs:
+        Vall, Pall = gather_members(Vd, world), gather_members(Pd, world)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dict(v=Vall, p=Pall))
     parity_job = None
     if rank == 0 and not args.no_parity:
-        Vd, Pd = integ.state()
         sel = [0, nb - 1] if nb > 1 else [0]
         parity_job = dict(mesh=args.mesh, dt=1./args.nts, nsteps=nwarm + args.steps,
                           nus=[float(info['nus'][k]) for k in sel],

@@ -112,11 +112,36 @@ def golden_dfg():
                                              0.11752016697]))
 
 
+def golden_live_cases():
+    """what the oracle and the package return for the inputs of the tests
+    that run the live reference (`tests/live_cases.py`): the always-run part
+    of those tests compares with these, the live part with the reference"""
+    sys.path.insert(0, os.path.dirname(HERE))
+    import live_cases as lc
+    from dolfin_navier_scipy_b200 import time_int_utils as tiu
+    out = osnu.solve_nse(**dict(lc.bcrob_soldict(1, lc.CNAB_RE), **lc.CNAB_KW))
+    ts = sorted(out.keys())
+    femp, sm, rhsd = cyl(1, 60)
+    (vb, pb), ffb = osnu.solve_nse(**soldict(femp, sm, rhsd, **lc.BLOWUP_KW))
+    inp = lc.observer_inputs()
+    ab, abkeys = lc.observer_trail(tiu.get_heunab_lti, inp)
+    tz, tzkeys = lc.observer_trail(tiu.get_heuntrpz_lti, inp,
+                                   constdt=inp['ts'][1] - inp['ts'][0])
+    np.savez_compressed(
+        os.path.join(HERE, 'live_cases_cyl1.npz'), cnab_t=np.array(ts),
+        cnab_v=np.hstack([out[t]['v'] for t in ts]),
+        cnab_p=np.hstack([out[t]['p'] for t in ts]),
+        blowup_ff=np.array(ffb), blowup_v=vb, blowup_p=pb,
+        heunab_out=ab, heunab_keys=np.array(abkeys),
+        heuntrpz_out=tz, heuntrpz_keys=np.array(tzkeys))
+
+
 if __name__ == '__main__':
     golden_convection()
     golden_cnab()
     golden_newton_cn()
     golden_dfg()
+    golden_live_cases()
     for f in sorted(os.listdir(HERE)):
         if f.endswith('.npz'):
             print(f, os.path.getsize(os.path.join(HERE, f)), 'bytes')

@@ -1,18 +1,20 @@
 #!/usr/bin/env python
 """Reference-RUN golden vectors: outputs of the reference's own code.
 
-Runs the UNMODIFIED modules of /root/reference (`time_int_utils.py`,
-`stokes_navier_utils.py`, `dolfin_to_sparrays.py` condensation helpers,
-`data_output_utils.py`) in this container through `tests/refharness.py`
+Runs the UNMODIFIED modules of the reference checkout that
+``DNS_REFERENCE_ROOT`` names (`time_int_utils.py`, `stokes_navier_utils.py`,
+`dolfin_to_sparrays.py` condensation helpers, `data_output_utils.py`) through
+`tests/refharness.py`
 (stub `dolfin` carrier objects, exact sparse solve for the un-vendored
 `sadptprj_riclyap_adi.lin_alg_utils.solve_sadpnt_smw`, quadrature for the two
 FFC-assembled convection forms) on the operators of the package's host shim,
-and stores what they return.  The reference cannot travel to the GPU box, so
-these small `.npz` files are what pins (a) the oracle (`tests/
+and stores what they return.  The reference is not part of this repository,
+so these small `.npz` files are what pins (a) the oracle (`tests/
 test_reference_pin.py`, CPU) and (b) the CUDA path (`tests/test_gpu_parity.py`,
 GPU) to reference-run numbers.
 
-    python tests/golden/make_reference_golden.py    # rewrites tests/golden/ref_*.npz
+    DNS_REFERENCE_ROOT=<checkout> python tests/golden/make_reference_golden.py
+                                            # rewrites tests/golden/ref_*.npz
 """
 import os
 import shutil

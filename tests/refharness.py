@@ -1,4 +1,7 @@
-"""Run the UNMODIFIED reference modules of /root/reference in this container.
+"""Run the UNMODIFIED reference modules of a `dolfin_navier_scipy` checkout.
+
+The checkout is not part of this repository: ``DNS_REFERENCE_ROOT`` names its
+root directory (the one that holds the `dolfin_navier_scipy` package).
 
 TEST INFRASTRUCTURE.  The reference is pure Python, but its modules import
 three things that are not installable here: `dolfin` (FEniCS), the un-vendored
@@ -24,7 +27,7 @@ condense_velmatsbybcs/condense_sysmatsbybcs/append_bcs_vec/unroll_dlfn_dbcs`,
 from the files where they lie and executed unchanged.  `load()` returns the
 modules; `tests/golden/make_reference_golden.py` uses them to write the
 reference-run fixtures, `tests/test_reference_pin.py` to compare the oracle
-with the live reference whenever /root/reference exists.
+with the live reference whenever ``DNS_REFERENCE_ROOT`` is set.
 
 Nothing here is imported by the product or by the `-m gpu` tests.
 """
@@ -36,12 +39,13 @@ import types
 
 import numpy as np
 
-REFROOT = os.environ.get('DNS_REFERENCE_ROOT', '/root/reference')
+REFROOT = os.environ.get('DNS_REFERENCE_ROOT', '')
 REFPKG = os.path.join(REFROOT, 'dolfin_navier_scipy')
 
 
 def available():
-    return os.path.isfile(os.path.join(REFPKG, 'time_int_utils.py'))
+    return bool(REFROOT) and \
+        os.path.isfile(os.path.join(REFPKG, 'time_int_utils.py'))
 
 
 class _Vector(object):

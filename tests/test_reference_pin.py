@@ -5,12 +5,11 @@ Two layers:
  * `tests/golden/ref_*.npz` were written by `tests/golden/
    make_reference_golden.py`, which executes the unmodified reference modules
    (`time_int_utils.py`, `stokes_navier_utils.py`, the condensation helpers of
-   `dolfin_to_sparrays.py`) from /root/reference through `tests/refharness.py`.
-   The oracle must reproduce them -- always checked, also where the reference
-   is absent (GPU box).
- * where /root/reference exists (the build container) the reference is run
-   LIVE beside the oracle on fresh inputs, so neither the fixtures nor the
-   oracle can drift.
+   `dolfin_to_sparrays.py`) through `tests/refharness.py`.  The oracle must
+   reproduce them -- always checked, also where the reference is absent.
+ * where ``DNS_REFERENCE_ROOT`` names a checkout of the reference, the
+   reference is run LIVE beside the oracle on fresh inputs, so neither the
+   fixtures nor the oracle can drift.
 
 Tolerance 1e-13 relative (measured: 0.0 -- the oracle performs the same
 floating-point operations in the same order).
@@ -20,14 +19,17 @@ import os
 import numpy as np
 import pytest
 
+import live_cases as lc
 import refharness as rh
 from conftest import soldict
+from live_cases import bcrob_soldict
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 TOL = 1e-13
 
-needs_ref = pytest.mark.skipif(not rh.available(),
-                               reason='/root/reference is not on this box')
+needs_ref = pytest.mark.skipif(
+    not rh.available(), reason='needs a checkout of the reference '
+    'dolfin_navier_scipy: set DNS_REFERENCE_ROOT to its root directory')
 
 
 def _rel(a, b):
@@ -44,21 +46,6 @@ def _cyl(level, Re):
     return dnsps.get_sysmats(problem='cylinderwake', Re=Re, scheme='TH',
                              mergerhs=True,
                              meshparams=dict(refinement_level=level))
-
-
-def bcrob_soldict(level, Re, palpha=1e-5):
-    """`tests/time_dep_nse_bcrob.py:14-34` on the host shim's operators"""
-    from dolfin_navier_scipy_b200 import problem_setups as dnsps
-    femp, sm, rv, rb = dnsps.get_sysmats(
-        problem='cylinderwake', Re=Re, bccontrol=True, scheme='TH',
-        meshparams=dict(refinement_level=level))
-    Brob = sm['Brob']/palpha
-    bdiff = np.asarray(Brob[:, :1] - Brob[:, 1:]).reshape(-1, 1)
-    return dict(A=sm['A'] + sm['Arob']/palpha, M=sm['M'], J=sm['J'],
-                JT=sm['JT'], fv=rb['fv'] + rv['fv'], fp=rb['fp'] + rv['fp'],
-                fvtd=lambda t: np.sin(t)*bdiff, V=femp['V'],
-                invinds=femp['invinds'], dbcinds=femp['dbcinds'],
-                dbcvals=femp['dbcvals'])
 
 
 # ---------------------------------------------------------------------------
@@ -176,7 +163,11 @@ def test_oracle_semi_implicit_euler_equals_reference_run(cyl1):
 
 
 # ---------------------------------------------------------------------------
-# live: the reference's own code beside the oracle (build container only)
+# live: the reference's own code beside the oracle.  The tests below that
+# run everywhere compare with `tests/golden/live_cases_cyl1.npz` (what the
+# oracle and the package return for the same inputs, `tests/golden/
+# make_golden.py`) and, where DNS_REFERENCE_ROOT names a checkout, also with
+# the reference itself
 # ---------------------------------------------------------------------------
 @needs_ref
 def test_live_reference_modules_are_the_reference_files():
@@ -191,16 +182,21 @@ def test_live_reference_modules_are_the_reference_files():
         'dolfin_navier_scipy.stokes_navier_utils'
 
 
-@needs_ref
 def test_live_reference_cnab_with_time_dependent_forcing(tmp_path):
     """`snu.solve_nse` -> `tiu.cnab` of the reference, Robin control at a
-    Reynolds number that is in no fixture, fresh step count"""
+    Reynolds number that is in no other fixture, fresh step count"""
     from oracle import snu as osnu
-    ref = rh.load()
-    sd = bcrob_soldict(1, 87.)
-    kw = dict(t0=0., tE=9./256, Nts=9, start_ssstokes=True,
-              return_vp_dict=True)
+    sd, kw = bcrob_soldict(1, lc.CNAB_RE), lc.CNAB_KW
     out = osnu.solve_nse(**dict(sd, **kw))
+    g = _gold('live_cases_cyl1.npz')
+    ts = sorted(out.keys())
+    assert np.array_equal(ts, g['cnab_t'])
+    for j, t in enumerate(ts):
+        assert _rel(out[t]['v'], g['cnab_v'][:, j:j+1]) <= TOL, t
+        assert _rel(out[t]['p'], g['cnab_p'][:, j:j+1]) <= TOL, t
+    if not rh.available():
+        return
+    ref = rh.load()
     got = ref['snu'].solve_nse(data_prfx=str(tmp_path/'r'), verbose=False,
                                paraviewoutput=False,
                                **rh.as_spmatrix(dict(sd, **kw)))
@@ -210,16 +206,18 @@ def test_live_reference_cnab_with_time_dependent_forcing(tmp_path):
         assert _rel(out[t]['p'], got[t]['p']) <= TOL, t
 
 
-@needs_ref
 def test_live_reference_blowup_flag(cyl1, tmp_path):
     """`check_ff` / `check_ff_maxv` (`tiu:94-103`)"""
     from oracle import snu as osnu
-    ref = rh.load()
     femp, sm, rhsd = cyl1
-    kw = dict(t0=0., tE=24./512, Nts=24, start_ssstokes=True,
-              return_final_vp=True, check_ff=True, check_ff_maxv=1e-3)
-    sd = soldict(femp, sm, rhsd, **kw)
+    sd = soldict(femp, sm, rhsd, **lc.BLOWUP_KW)
     (vo, po), fo = osnu.solve_nse(**sd)
+    g = _gold('live_cases_cyl1.npz')
+    assert fo == int(g['blowup_ff']) == 1
+    assert _rel(vo, g['blowup_v']) <= TOL and _rel(po, g['blowup_p']) <= TOL
+    if not rh.available():
+        return
+    ref = rh.load()
     (vr, pr), fr = ref['snu'].solve_nse(data_prfx=str(tmp_path/'r'),
                                         verbose=False, paraviewoutput=False,
                                         **rh.as_spmatrix(sd))
@@ -296,42 +294,43 @@ def test_host_hop_loop_equals_reference_run_with_callbacks(cyl1, scheme,
     assert _rel(p, g['p_' + scheme]) <= 1e-10
 
 
-@needs_ref
 def test_observer_discretisations_equal_the_reference():
     """`tiu.get_heunab_lti` / `get_heuntrpz_lti` (`tiu:148-257`): same outputs
     and the same memory trail as the reference's closures, mode by mode"""
     from dolfin_navier_scipy_b200 import time_int_utils as tiu
-    ref = rh.load()['tiu']
-    rng = np.random.default_rng(3)
-    ha = -2.*np.eye(4) + rng.standard_normal((4, 4))
-    hb, hc = rng.standard_normal((4, 2)), rng.standard_normal((3, 4))
-    x0 = rng.standard_normal((4, 1))
-    kw = dict(hb=hb, ha=ha, hc=hc, inihx=x0,
-              drift=lambda t: np.full((4, 1), np.sin(t)))
-    ts = np.linspace(0., .5, 6)
-    ys = [rng.standard_normal((2, 1)) for _ in ts]
-    for mine, theirs, extra in (
-            (tiu.get_heunab_lti, ref.get_heunab_lti, {}),
-            (tiu.get_heuntrpz_lti, ref.get_heuntrpz_lti,
-             dict(constdt=ts[1] - ts[0]))):
-        a, b = mine(**dict(kw, **extra)), theirs(**dict(kw, **extra))
-        ma, mb = {}, {}
-        seq = [(ts[0], 'init'), (ts[1], 'heunpred'), (ts[1], 'heuncorr')] + \
-            [(t, 'abtwo') for t in ts[2:]]
-        for k, (t, mode) in enumerate(seq):
-            ua, ma = a(t, vc=ys[min(k, 5)], memory=ma, mode=mode)
-            ub, mb = b(t, vc=ys[min(k, 5)], memory=mb, mode=mode)
-            assert np.allclose(ua, ub, rtol=1e-14, atol=0), (mode, k)
-            assert set(ma.keys()) == set(mb.keys())
+    inp = lc.observer_inputs()
+    g = _gold('live_cases_cyl1.npz')
+    ref = rh.load()['tiu'] if rh.available() else None
+    for name, extra in (('heunab', {}),
+                        ('heuntrpz', dict(constdt=inp['ts'][1] - inp['ts'][0]))):
+        mine = getattr(tiu, 'get_%s_lti' % name)
+        outs, keys = lc.observer_trail(mine, inp, **extra)
+        theirs = [(g[name + '_out'], list(g[name + '_keys']))]
+        if ref is not None:
+            theirs.append(lc.observer_trail(getattr(ref, 'get_%s_lti' % name),
+                                            inp, **extra))
+        for touts, tkeys in theirs:
+            for k, mode in enumerate(lc.OBSERVER_SEQ):
+                assert np.allclose(outs[k], touts[k], rtol=1e-14, atol=0), \
+                    (name, mode, k)
+                assert set(keys[k].split(',')) == set(tkeys[k].split(','))
 
 
-@needs_ref
 def test_live_reference_time_sections_are_broken_at_head(tmp_path):
     """`nsects` > 1 (`snu:1076-1087`): the reference's second time section dies
-    with `KeyError: None` (`snu:1425-1431`) -- the product's
-    `NotImplementedError` for `nsects`/`addfullsweep` mirrors a dead path"""
-    ref = rh.load()
+    with `KeyError: None` (`snu:1425-1431`, DESIGN.md section 2) -- the
+    product's `NotImplementedError` for `nsects`/`addfullsweep` mirrors a dead
+    path, raised before any device work"""
+    from dolfin_navier_scipy_b200 import stokes_navier_utils as snu
     femp, sm, rhsd = _cyl(1, 100)
+    sdp = soldict(femp, sm, rhsd, t0=0., tE=8./512, Nts=8, start_ssstokes=True)
+    for kw in (dict(nsects=2), dict(addfullsweep=True)):
+        with pytest.raises(NotImplementedError):
+            snu.solve_nse(treat_nonl_explicit=False, vel_pcrd_stps=1,
+                          vel_nwtn_stps=2, **kw, **sdp)
+    if not rh.available():
+        return
+    ref = rh.load()
     sd = rh.as_spmatrix(soldict(femp, sm, rhsd, t0=0., tE=8./512, Nts=8,
                                 start_ssstokes=True))
     kw = dict(verbose=False, paraviewoutput=False)
