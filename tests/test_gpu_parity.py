@@ -6,6 +6,8 @@ import pytest
 import scipy.sparse as sps
 
 from conftest import soldict
+from kernel_refs import cheb_np as _cheb_np
+from kernel_refs import ctx_with_env as _ctx_with_env
 
 pytestmark = pytest.mark.gpu
 
@@ -399,25 +401,6 @@ def test_spmm_all_batch_widths(cyl1, ctx, nb):
     JT = sps.csr_matrix(sm['JT'])
     P = rng.standard_normal((JT.shape[1], nb))
     assert _rel(ctx.csr(JT).spmm(P), JT@P) < 1e-13
-
-
-def _cheb_np(Fm, dinv, r, k, lmin, lmax):
-    """numpy restatement of the device Jacobi-Chebyshev smoother (zero guess)"""
-    th, de = .5*(lmax + lmin), .5*(lmax - lmin)
-    sigma = th/de
-    rho = 1./sigma
-    z = np.zeros_like(r)
-    res = r.copy()
-    d = dinv*res/th
-    for i in range(k):
-        z = z + d
-        if i == k - 1:
-            break
-        res = res - Fm@d
-        rho_n = 1./(2*sigma - rho)
-        d = rho_n*rho*d + 2*rho_n/de*(dinv*res)
-        rho = rho_n
-    return z
 
 
 @pytest.mark.parametrize('kind', ['stokes', 'picard'])
@@ -1027,23 +1010,6 @@ def test_steady_solver_outside_its_envelope_fails_loudly(cyl1, ctx):
                                   **soldict(femp, sm, rhsd))
 
 
-def _ctx_with_env(name, value, **more):
-    """a context created under environment switches (read at creation)"""
-    from dolfin_navier_scipy_b200 import _lib
-    env = dict(more)
-    env[name] = value
-    old = {k: os.environ.get(k) for k in env}
-    os.environ.update(env)
-    try:
-        return _lib.Context(0)
-    finally:
-        for k, v in old.items():
-            if v is None:
-                del os.environ[k]
-            else:
-                os.environ[k] = v
-
-
 @pytest.fixture
 def tc_ctx():
     """the tcgen05 Schur block (the default for nb >= 8) switched on explicitly"""
@@ -1056,7 +1022,7 @@ def f64_ctx():
     return _ctx_with_env('DNSB_SCHUR_TC', '0')
 
 
-@pytest.mark.parametrize('ncols', [64, 24, 8])
+@pytest.mark.parametrize('ncols', [256, 128, 64, 24, 8])
 def test_schur_tensor_core_block_against_numpy(cyl1, tc_ctx, ncols):
     """k_schur_tc (tcgen05.mma kind::tf32, TMA-fed, TMEM accumulators): the
     pressure part of one preconditioner application, z_p = -D r_p, against the
@@ -1436,7 +1402,9 @@ def test_projection_space_forms_agree_across_rebuilds(cyl1, ctx):
                                     'DNSB_TILE=0', 'DNSB_SCHUR_TC=0',
                                     'DNSB_GS_PYTH=0', 'DNSB_CHEB_F32=0',
                                     'DNSB_PROJ_T=0', 'DNSB_TAIL_WARPS=0',
-                                    'DNSB_PDL=0'])
+                                    'DNSB_PDL=0', 'DNSB_INIT_TILE=0',
+                                    'DNSB_TILEF_CTAS=1', 'DNSB_TILE_STAGES=2',
+                                    'DNSB_TILE_STAGES_F=2', 'DNSB_TC_CTAS=2'])
 def test_every_tuning_switch_gives_the_same_trajectory(cyl1, ctx, switch):
     """the environment switches select kernel VARIANTS of the same arithmetic
     (coloured scatter vs gather assembly -- the form `north_star` names --,
