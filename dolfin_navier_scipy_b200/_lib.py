@@ -84,6 +84,11 @@ SIGNATURES = {
     'dnsb_imex_reserve_snapshots': (_i, [_vp, _i]),
     'dnsb_imex_snapshots_host': (_i, [_vp, ctypes.POINTER(c_dbl_p),
                                       ctypes.POINTER(_i)]),
+    'dnsb_imex_set_outputs': (_i, [_vp, _vp, _vp]),
+    'dnsb_imex_set_force': (_i, [_vp, _i, c_int_p, _vp, _vp, _vp, c_dbl_p]),
+    'dnsb_imex_num_output_levels': (_i, [_vp]),
+    'dnsb_imex_get_outputs': (_i, [_vp, c_dbl_p, c_dbl_p]),
+    'dnsb_imex_reset_outputs': (_i, [_vp]),
     'dnsb_imex_stats': (_i, [_vp, ctypes.POINTER(_ll), ctypes.POINTER(_ll),
                              c_dbl_p]),
     'dnsb_imex_gram_dev': (_i, [_vp, _vp]),
@@ -612,6 +617,35 @@ class ImexEngine(object):
 
     def reset_snapshots(self):
         self.ctx.check(self.ctx.lib.dnsb_imex_reset_snapshots(self.h))
+
+    def set_outputs(self, cv=None, cp=None):
+        """linear output rows (`Csr`, device column numbering) or None; the
+        engine copies them"""
+        self.ctx.check(self.ctx.lib.dnsb_imex_set_outputs(
+            self.h, cv.h if cv is not None else None,
+            cp.h if cp is not None else None))
+
+    def set_force(self, dofs=None, fm=None, fa=None, fj=None, fa_bc=None):
+        """force rows (`Csr`) on the full-numbering ``dofs``; None: off"""
+        dofs = _i32(np.zeros(0) if dofs is None else dofs)
+        fa_bc = _f64(fa_bc, (-1,))
+        self.ctx.check(self.ctx.lib.dnsb_imex_set_force(
+            self.h, dofs.size, _ip(dofs), fm.h if fm is not None else None,
+            fa.h if fa is not None else None, fj.h if fj is not None else None,
+            _dp(fa_bc)))
+
+    def outputs(self, ny):
+        """``(y (levels, ny, nb), force (levels, 2, nb))``"""
+        nl = self.ctx.lib.dnsb_imex_num_output_levels(self.h)
+        y = np.empty((nl, ny, self.nb))
+        f = np.empty((nl, 2, self.nb))
+        if nl > 0:
+            self.ctx.check(self.ctx.lib.dnsb_imex_get_outputs(self.h, _dp(y),
+                                                              _dp(f)))
+        return y, f
+
+    def reset_outputs(self):
+        self.ctx.check(self.ctx.lib.dnsb_imex_reset_outputs(self.h))
 
     def stats(self):
         it, ns, rr = _ll(), _ll(), ctypes.c_double()

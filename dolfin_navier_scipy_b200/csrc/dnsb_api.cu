@@ -2558,6 +2558,18 @@ struct dnsb_imex {
   float last_run_ms = 0.f;
   bool have_state = false;
   bool p_stale = false;
+  // output functionals (dnsb_imex_set_outputs / dnsb_imex_set_force): ny linear rows + 2 force rows per
+  // time level.  The rows are kept on the host as given (either call rebuilds the device arrays), the
+  // record (levels, ny + 2, nb) grows at the start of a run like the snapshot store.
+  int ny = 0;
+  std::vector<int> cv_ptr, cv_idx, cp_ptr, cp_idx, fm_ptr, fm_idx, fa_ptr, fa_idx, fj_ptr, fj_idx, fdofs;
+  std::vector<double> cv_val, cp_val, fm_val, fa_val, fj_val;
+  double fbc[2] = {0.0, 0.0};
+  DBuf<int> o_vptr, o_vidx, o_pptr, o_pidx, o_fptr, o_fdofs;
+  DBuf<double> o_w1, o_w2, o_wp, o_fbc, o_csave, o_rec;
+  int nlev = 0, lev_cap = 0;
+  long long csave_level = -1;   // time level n whose Phi^T c(V_n) is in o_csave (-1: none)
+  bool outputs_on() const { return ny > 0 || !fdofs.empty(); }
 };
 
 extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
@@ -2654,6 +2666,9 @@ extern "C" void dnsb_imex_destroy(dnsb_imex *e) {
   e->gr.release(); e->partialh.release(); e->snaps.release();
   e->ptri.release(); e->py.release(); e->pgsum.release();
   e->normpart.release(); e->normout.release();
+  e->o_vptr.release(); e->o_vidx.release(); e->o_pptr.release(); e->o_pidx.release();
+  e->o_fptr.release(); e->o_fdofs.release(); e->o_w1.release(); e->o_w2.release(); e->o_wp.release();
+  e->o_fbc.release(); e->o_csave.release(); e->o_rec.release();
   delete e;
 }
 
@@ -2698,6 +2713,7 @@ extern "C" int dnsb_imex_set_state(dnsb_imex *e, const double *v0, const double 
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   e->step = 0; e->hist_cnt = 0; e->hist_pos = 0; e->nsnap = 0; e->pcnt = 0;
   e->force_t0 = 0;
+  e->nlev = 0; e->csave_level = -1;
   e->have_state = true;
   e->p_stale = false;
   return 0;
@@ -2792,6 +2808,114 @@ static int imex_snapshot(dnsb_imex *e) {
     e->stage_busy[q] = true;
   }
   e->nsnap++;
+  return 0;
+}
+
+// ---- output functionals ---------------------------------------------------
+// Row r of the (ny + 2) x nb values of one time level n:
+//   r < ny:      y_r = sum_k w1[k] vn[k] + ps sum_k wp[k] pn[k]                         (Cv v_n + Cp p_n)
+//   r = ny + c:  F_c = rdt sum_k w1[k] (vn - vp)[k] + nu_m (1/2 sum_k w2[k] (vn + vp)[k] + fbc[c])
+//                      - ps sum_k wp[k] pn[k] + 3/2 cc - 1/2 csave[c]
+// the CNAB residual tested with the indicator of component c of the force dofs (residual_checks.get_imex_res):
+// w1 = Phi^T M[:, inv], w2 = Phi^T A0[:, inv], wp = Phi^T JT, fbc = Phi^T A0[:, bc] u_bc, vp = v_{n-1}, and
+// cc = Phi^T c(V_{n-1}) summed from the element buffer E of K1a through the node -> cell lists (as
+// k_conv_gather does) or read from the full vector cfull (coloured K1a).  csave[c] holds Phi^T c(V_{n-2}) and
+// receives cc.  fvalid = 0: the force is NaN (no earlier level to difference against); out == null: only
+// csave is written (Heun start).  Block <-> (row, 32 members), lane <-> member: a warp reads 32 members of one
+// column; warp w takes the terms w, w + OUT_WARPS, ... and the warps' sums are added in warp order, so the
+// summation order is fixed and the result bit-reproducible.  The rows are short (a force row of cylinder_4:
+// ~800 velocity, ~190 pressure terms, ~190 dofs): the kernel is bound by the latency of the dependent index ->
+// value loads, hence many warps per row and unrolled loops (several loads in flight per warp).
+#define OUT_WARPS 32
+__global__ void __launch_bounds__(OUT_WARPS * 32)
+k_imex_outputs(int ny, int row0, const int *__restrict__ vptr, const int *__restrict__ vidx,
+               const double *__restrict__ w1, const double *__restrict__ w2, const int *__restrict__ pptr,
+               const int *__restrict__ pidx, const double *__restrict__ wp, const int *__restrict__ fptr,
+               const int *__restrict__ fdofs, const int *__restrict__ n2c_ptr, const int *__restrict__ n2c_idx,
+               const double *__restrict__ E, const double *__restrict__ cfull, const double *__restrict__ vn,
+               const double *__restrict__ vp, const double *__restrict__ pn, double ps, double rdt,
+               const double *__restrict__ nu, const double *__restrict__ fbc, int fvalid, double *csave,
+               double *__restrict__ out, int nb) {
+  dnsb_pdl_entry();
+  __shared__ double red[4][OUT_WARPS][32];
+  const int r = row0 + blockIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int m = blockIdx.y * 32 + lane;
+  const bool frow = r >= ny, act = m < nb;
+  const bool conv = frow && (E != nullptr || cfull != nullptr);
+  const bool sums = out != nullptr && (!frow || fvalid);
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+  if (act && sums) {
+    if (frow) {
+#pragma unroll 4
+      for (int k = vptr[r] + w; k < vptr[r + 1]; k += OUT_WARPS) {
+        const size_t o = (size_t)vidx[k] * nb + m;
+        const double a = vn[o], b = vp[o];
+        s0 += w1[k] * (a - b);
+        s1 += w2[k] * (a + b);
+      }
+    } else {
+#pragma unroll 4
+      for (int k = vptr[r] + w; k < vptr[r + 1]; k += OUT_WARPS) s0 += w1[k] * vn[(size_t)vidx[k] * nb + m];
+    }
+#pragma unroll 4
+    for (int k = pptr[r] + w; k < pptr[r + 1]; k += OUT_WARPS) s2 += wp[k] * pn[(size_t)pidx[k] * nb + m];
+  }
+  const int c = r - ny;
+  if (act && conv) {
+#pragma unroll 2
+    for (int q = fptr[c] + w; q < fptr[c + 1]; q += OUT_WARPS) {
+      const int dof = fdofs[q];
+      if (cfull) {
+        s3 += cfull[(size_t)dof * nb + m];
+      } else {
+        const int node = dof >> 1;
+        double s = 0.0;
+        for (int k = n2c_ptr[node]; k < n2c_ptr[node + 1]; ++k) s += E[((size_t)n2c_idx[k] * 2 + c) * nb + m];
+        s3 += s;
+      }
+    }
+  }
+  red[0][w][lane] = s0; red[1][w][lane] = s1; red[2][w][lane] = s2; red[3][w][lane] = s3;
+  __syncthreads();
+  if (w != 0 || !act) return;
+  double t0 = 0.0, t1 = 0.0, t2 = 0.0, t3 = 0.0;
+  for (int q = 0; q < OUT_WARPS; ++q) {
+    t0 += red[0][q][lane]; t1 += red[1][q][lane]; t2 += red[2][q][lane]; t3 += red[3][q][lane];
+  }
+  if (out) {
+    double val;
+    if (!frow) val = t0 + ps * t2;
+    else if (!fvalid) val = __longlong_as_double(0x7ff8000000000000ll);   // NaN
+    else val = rdt * t0 + nu[m] * (0.5 * t1 + fbc[c]) - ps * t2 + 1.5 * t3 - 0.5 * csave[(size_t)c * nb + m];
+    out[(size_t)r * nb + m] = val;
+  }
+  if (conv) csave[(size_t)c * nb + m] = t3;
+}
+
+// one launch of k_imex_outputs.  out_level: record the level into the next slot (vn, vp, pn, ps as in the
+// kernel; vp may be null when the force is not valid); false: only capture Phi^T c of the convection the
+// element buffer / cfull holds now (the caller says which level that is).  conv_level >= 0: the convection
+// source holds c(V_{conv_level}), which the force of level conv_level + 1 needs together with the saved
+// term of level conv_level - 1.
+static int imex_outputs(dnsb_imex *e, bool out_level, const double *vn, const double *vp, const double *pn,
+                        double ps, long long conv_level) {
+  dnsb_ctx *ctx = e->ctx;
+  const int nb = e->nb;
+  const bool force = !e->fdofs.empty() && conv_level >= 0;
+  const double *E = force && !g_conv_colours ? e->ctx->elem.p : nullptr;
+  const double *cf = force && g_conv_colours ? e->cfull.p : nullptr;
+  const int fvalid = force && out_level && e->csave_level == conv_level - 1 && vp != nullptr ? 1 : 0;
+  const int row0 = out_level ? 0 : e->ny;
+  const int nrows = out_level ? e->ny + 2 : 2;
+  if (!out_level && !force) return 0;
+  double *out = out_level ? e->o_rec.p + (size_t)e->nlev * (e->ny + 2) * nb : nullptr;
+  LAUNCH(ctx, k_imex_outputs, dim3(nrows, cdiv(nb, 32)), OUT_WARPS * 32, 0, e->ny, row0,
+         (const int *)e->o_vptr.p, (const int *)e->o_vidx.p, (const double *)e->o_w1.p, (const double *)e->o_w2.p,
+         (const int *)e->o_pptr.p, (const int *)e->o_pidx.p, (const double *)e->o_wp.p, (const int *)e->o_fptr.p,
+         (const int *)e->o_fdofs.p, (const int *)ctx->n2c_ptr.p, (const int *)ctx->n2c_idx.p, E, cf, vn, vp, pn, ps,
+         1.0 / e->dt, (const double *)e->nu.p, (const double *)e->o_fbc.p, fvalid, e->o_csave.p, out, nb);
+  if (force) e->csave_level = conv_level;
+  if (out_level) e->nlev++;
   return 0;
 }
 
@@ -3102,6 +3226,28 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     }
     if (e->step == 0) { int rc = imex_snapshot(e); if (rc) return rc; }
   }
+  // ---- output functionals: room for this run's levels, the current one first if the record is empty --
+  const bool outs = e->outputs_on();
+  if (outs) {
+    const size_t per = (size_t)(e->ny + 2) * nb;
+    const int need = e->nlev + (e->nlev == 0 ? 1 : 0) + nsteps;
+    if (need > e->lev_cap) {
+      DBuf<double> nr;
+      DNSB_CK(ctx, nr.alloc((size_t)need * per));
+      if (e->nlev > 0)
+        DNSB_CK(ctx, cudaMemcpyAsync(nr.p, e->o_rec.p, (size_t)e->nlev * per * sizeof(double),
+                                     cudaMemcpyDeviceToDevice, ctx->stream));
+      DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+      e->o_rec.release();
+      e->o_rec = nr;
+      e->lev_cap = need;
+    }
+    if (e->nlev == 0) {
+      imex_refresh_p(e);
+      int rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1);
+      if (rc) return rc;
+    }
+  }
   const long long it0 = e->sl->stat_iters, ns0 = e->sl->stat_solves;
   dnsb_solver *const run_solvers[3] = {e->sl, e->sp, e->sc};
   long long unc0 = 0;
@@ -3117,6 +3263,10 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     const double *u0 = useries_at(e, 0), *u1 = useries_at(e, 1);
     int rc = imex_nonl(e, e->v.p, e->nfc_c.p);                 // nfc(v0)
     if (rc) return rc;
+    if (outs && e->scheme == 0) {   // Phi^T c(V_0), before the predictor's convection overwrites it
+      rc = imex_outputs(e, false, nullptr, nullptr, nullptr, 0.0, 0);
+      if (rc) return rc;
+    }
     // predictor (IMEX Euler):  (M + dt A) tv = M v + dt f(t1) + dt nfc(v0)
     spmm_dev(ctx, e->M, nullptr, e->v.p, nullptr, e->b.p, nb, 1.0, 0.0);
     LAUNCH(ctx, k_rhs_combine, cdiv(nvb, 256), 256, 0, e->b.p, (const double *)e->nfc_c.p, dt,
@@ -3149,6 +3299,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     imex_refresh_p(e);
     e->step = 1;
     done = 1;
+    if (outs) { rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1); if (rc) return rc; }
     if (snap_stride > 0 && e->step % snap_stride == 0) { rc = imex_snapshot(e); if (rc) return rc; }
     // nfc_c holds nfc(v0): it becomes nfc_o in the first loop step
   }
@@ -3215,6 +3366,10 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     rc = solver_solve_dev(e->sl, e->b.p, e->x.p, tol, maxit, false);
     if (rc) return rc;
     e->p_stale = true;
+    if (outs) {   // level n from [v_n; q_n] = x, v_{n-1} = v and c(V_{n-1}) of this step's imex_nonl
+      rc = imex_outputs(e, true, e->x.p, e->v.p, e->x.p + nvb, -1.0 / dt, e->scheme == 0 ? n - 1 : -1);
+      if (rc) return rc;
+    }
     rc = imex_push_history(e, guess);
     if (rc) return rc;
     if (e->scheme == 1)
@@ -3354,6 +3509,139 @@ extern "C" int dnsb_imex_reserve_snapshots(dnsb_imex *e, int nsnap) {
   DNSB_REQUIRE(ctx, nsnap >= 0, "bad count");
   DNSB_CK(ctx, dnsb_enter(ctx));
   return imex_reserve_host(e, nsnap);
+}
+
+// ---- output functionals: host side --------------------------------------------
+static void rows_copy(const dnsb_csr *a, std::vector<int> &ptr, std::vector<int> &idx, std::vector<double> &val) {
+  if (!a) { ptr.clear(); idx.clear(); val.clear(); return; }
+  ptr = a->h_indptr; idx = a->h_indices; val = a->h_v1;
+}
+
+// device arrays of k_imex_outputs from the rows kept on the host: velocity rows (Cv | union of the
+// patterns of Phi^T M and Phi^T A0), pressure rows (Cp | Phi^T JT), force dofs by component
+static int outputs_upload(dnsb_imex *e) {
+  dnsb_ctx *ctx = e->ctx;
+  const int ny = e->ny;
+  std::vector<int> vptr(1, 0), vidx, pptr(1, 0), pidx;
+  std::vector<double> w1, w2, wp;
+  for (int r = 0; r < ny; ++r) {
+    if (!e->cv_ptr.empty())
+      for (int k = e->cv_ptr[r]; k < e->cv_ptr[r + 1]; ++k) {
+        vidx.push_back(e->cv_idx[k]); w1.push_back(e->cv_val[k]); w2.push_back(0.0);
+      }
+    vptr.push_back((int)vidx.size());
+    if (!e->cp_ptr.empty())
+      for (int k = e->cp_ptr[r]; k < e->cp_ptr[r + 1]; ++k) { pidx.push_back(e->cp_idx[k]); wp.push_back(e->cp_val[k]); }
+    pptr.push_back((int)pidx.size());
+  }
+  const bool force = !e->fdofs.empty();
+  std::vector<double> dm(force ? e->nv : 0), da(force ? e->nv : 0);
+  std::vector<char> hit(force ? e->nv : 0);
+  for (int c = 0; c < 2; ++c) {
+    if (force) {
+      std::fill(dm.begin(), dm.end(), 0.0); std::fill(da.begin(), da.end(), 0.0);
+      std::fill(hit.begin(), hit.end(), 0);
+      for (int k = e->fm_ptr[c]; k < e->fm_ptr[c + 1]; ++k) { dm[e->fm_idx[k]] += e->fm_val[k]; hit[e->fm_idx[k]] = 1; }
+      for (int k = e->fa_ptr[c]; k < e->fa_ptr[c + 1]; ++k) { da[e->fa_idx[k]] += e->fa_val[k]; hit[e->fa_idx[k]] = 1; }
+      for (int i = 0; i < e->nv; ++i)
+        if (hit[i]) { vidx.push_back(i); w1.push_back(dm[i]); w2.push_back(da[i]); }
+      for (int k = e->fj_ptr[c]; k < e->fj_ptr[c + 1]; ++k) { pidx.push_back(e->fj_idx[k]); wp.push_back(e->fj_val[k]); }
+    }
+    vptr.push_back((int)vidx.size());
+    pptr.push_back((int)pidx.size());
+  }
+  // force dofs: unique, x components first, ascending
+  std::vector<int> fd, fptr(3, 0);
+  for (int c = 0; c < 2; ++c) {
+    for (int d : e->fdofs) if ((d & 1) == c) fd.push_back(d);
+    std::sort(fd.begin() + fptr[c], fd.end());
+    fd.erase(std::unique(fd.begin() + fptr[c], fd.end()), fd.end());
+    fptr[c + 1] = (int)fd.size();
+  }
+  // empty lists still get a valid pointer
+  if (vidx.empty()) { vidx.push_back(0); w1.push_back(0.0); w2.push_back(0.0); }
+  if (pidx.empty()) { pidx.push_back(0); wp.push_back(0.0); }
+  if (fd.empty()) fd.push_back(0);
+  DNSB_CK(ctx, e->o_vptr.upload(vptr.data(), vptr.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_vidx.upload(vidx.data(), vidx.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_w1.upload(w1.data(), w1.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_w2.upload(w2.data(), w2.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_pptr.upload(pptr.data(), pptr.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_pidx.upload(pidx.data(), pidx.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_wp.upload(wp.data(), wp.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_fptr.upload(fptr.data(), fptr.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_fdofs.upload(fd.data(), fd.size(), ctx->stream));
+  DNSB_CK(ctx, e->o_fbc.upload(e->fbc, 2, ctx->stream));
+  DNSB_CK(ctx, e->o_csave.alloc((size_t)2 * e->nb));
+  // a new layout starts a new record
+  e->nlev = 0; e->lev_cap = 0; e->o_rec.release();
+  return 0;
+}
+
+extern "C" int dnsb_imex_set_outputs(dnsb_imex *e, dnsb_csr *cv, dnsb_csr *cp) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_REQUIRE(ctx, !cv || cv->ncols == e->nv, "Cv must have nv columns (inner velocity)");
+  DNSB_REQUIRE(ctx, !cp || cp->ncols == e->np, "Cp must have np columns (pressure)");
+  DNSB_REQUIRE(ctx, !cv || !cp || cv->nrows == cp->nrows, "Cv and Cp must have the same number of rows");
+  DNSB_CK(ctx, dnsb_enter(ctx));
+  e->ny = cv ? cv->nrows : cp ? cp->nrows : 0;
+  rows_copy(cv, e->cv_ptr, e->cv_idx, e->cv_val);
+  rows_copy(cp, e->cp_ptr, e->cp_idx, e->cp_val);
+  return outputs_upload(e);
+}
+
+extern "C" int dnsb_imex_set_force(dnsb_imex *e, int ndofs, const int32_t *dofs, dnsb_csr *fm, dnsb_csr *fa,
+                                   dnsb_csr *fj, const double *fa_bc) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_REQUIRE(ctx, ndofs >= 0, "bad number of force dofs");
+  if (ndofs > 0) {
+    DNSB_REQUIRE(ctx, e->scheme == 0,
+                 "forces are the CNAB residual (scheme 0); SBDF2 / IMEX Euler have no force functional");
+    DNSB_REQUIRE(ctx, dofs && fm && fa && fj && fa_bc, "null force arguments");
+    DNSB_REQUIRE(ctx, fm->nrows == 2 && fm->ncols == e->nv, "Phi^T M must be 2 x nv");
+    DNSB_REQUIRE(ctx, fa->nrows == 2 && fa->ncols == e->nv, "Phi^T A0 must be 2 x nv");
+    DNSB_REQUIRE(ctx, fj->nrows == 2 && fj->ncols == e->np, "Phi^T JT must be 2 x np");
+    for (int k = 0; k < ndofs; ++k)
+      DNSB_REQUIRE(ctx, dofs[k] >= 0 && dofs[k] < e->nvf, "force dof out of range (full velocity numbering)");
+  }
+  DNSB_CK(ctx, dnsb_enter(ctx));
+  if (ndofs > 0) e->fdofs.assign(dofs, dofs + ndofs); else e->fdofs.clear();
+  rows_copy(ndofs ? fm : nullptr, e->fm_ptr, e->fm_idx, e->fm_val);
+  rows_copy(ndofs ? fa : nullptr, e->fa_ptr, e->fa_idx, e->fa_val);
+  rows_copy(ndofs ? fj : nullptr, e->fj_ptr, e->fj_idx, e->fj_val);
+  e->fbc[0] = ndofs ? fa_bc[0] : 0.0;
+  e->fbc[1] = ndofs ? fa_bc[1] : 0.0;
+  e->csave_level = -1;
+  return outputs_upload(e);
+}
+
+extern "C" int dnsb_imex_num_output_levels(dnsb_imex *e) { return e ? e->nlev : -2; }
+
+extern "C" int dnsb_imex_reset_outputs(dnsb_imex *e) {
+  if (!e) return -2;
+  e->nlev = 0;
+  return 0;
+}
+
+extern "C" int dnsb_imex_get_outputs(dnsb_imex *e, double *y, double *force) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_CK(ctx, dnsb_enter(ctx));
+  const int nb = e->nb, nr = e->ny + 2;
+  if (e->nlev == 0) return 0;
+  std::vector<double> h((size_t)e->nlev * nr * nb);
+  DNSB_CK(ctx, cudaMemcpyAsync(h.data(), e->o_rec.p, h.size() * sizeof(double), cudaMemcpyDeviceToHost,
+                               ctx->stream));
+  DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  const size_t ly = (size_t)e->ny * nb, lf = (size_t)2 * nb;
+  for (int l = 0; l < e->nlev; ++l) {
+    const double *src = h.data() + (size_t)l * nr * nb;
+    if (y && ly) memcpy(y + l * ly, src, ly * sizeof(double));
+    if (force) memcpy(force + l * lf, src + ly, lf * sizeof(double));
+  }
+  return 0;
 }
 
 extern "C" int dnsb_imex_stats(dnsb_imex *e, long long *total_iters, long long *nsolves,

@@ -5,7 +5,9 @@ wake with penalised Robin control (`tests/time_dep_nse_bcrob.py:26-34`):
 ``A_m = nu_m*A0 + Arob/palpha``, ``f_m(t) = nu_m*fv_bc + u(t)*(B_1 - B_2)/palpha``.
 Members are independent: they are sharded over the GPUs with *no* collective
 on the step path; the only exchange is the all-reduce of the POD snapshot Gram
-matrix ``G = sum_m X_m^T M X_m`` (additive over members, SURVEY.md 8e).
+matrix ``G = sum_m X_m^T M X_m`` (additive over members, SURVEY.md 8e),
+and the one-off all-gather of the recorded output functionals
+(`gather_outputs`).
 """
 import numpy as np
 
@@ -13,7 +15,7 @@ from . import problem_setups as dnsps
 from . import time_int_utils as tiu
 
 __all__ = ['cylinder_ensemble', 'shard_members', 'bind_to_gpu_cpus',
-           'gram_allreduce',
+           'gram_allreduce', 'gather_outputs',
            'allreduce_gram', 'pod_from_gram', 'pod_modes']
 
 
@@ -57,11 +59,17 @@ def shard_members(nmembers, rank, world):
 def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
                       dt=1./512, scheme='cnab', palpha=1e-5, bccontrol=True,
                       control=np.sin, ntimes=513, t0=0., ctx=None, mesh=None,
-                      cheb_steps=4, restart=40, schur_poly=2, coarse_max=4096):
+                      cheb_steps=4, restart=40, schur_poly=2, coarse_max=4096,
+                      force=False, cv_mat=None, cp_mat=None):
     """device integrator for this rank's shard of a Re-sweep ensemble
 
     Returns ``(integ, info)``; ``integ`` is a `time_int_utils.DeviceImex` with
     forcing and members set, ``info`` holds sizes and the host operators.
+    ``force=True`` records the raw drag/lift on the whole cylinder
+    (``ldsbcinds``, control patches included) and ``cv_mat`` / ``cp_mat`` the
+    linear outputs at every time level (`DeviceImex.set_outputs`); the drag
+    coefficient is ``2/(rho L Um^2)`` times the x force
+    (`residual_checks.lift_drag_via_residual`).
     """
     Re_all = np.linspace(Res[0], Res[1], nmembers)
     lo, hi = shard_members(nmembers, rank, world)
@@ -94,6 +102,11 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
     if bccontrol:
         U[:, 1, :] = control(trange)[:, None]
     integ.set_forcing(B, U)
+    if force or cv_mat is not None or cp_mat is not None:
+        integ.set_outputs(cv_mat, cp_mat,
+                          force_dofs=femp['ldsbcinds'] if force else None,
+                          force_ops=dict(M=sm['Mfull'], A=sm['Afull'],
+                                         JT=sm['JTfull']))
     info = dict(femp=femp, sm=sm, nus=nus, Re=Re, NV=NV, NP=NP, B=B, U=U,
                 Arob=Arob, fp=rhs_bc['fp'] + rhs_vf['fp'], trange=trange,
                 members=(lo, hi))
@@ -124,6 +137,49 @@ def gram_allreduce(integ, group=None):
     torch.cuda.synchronize(dev)
     integ.engine.gram_dev(G.data_ptr())
     return allreduce_gram(G, group)
+
+
+def gather_outputs(integ, group=None):
+    """output functionals of the whole ensemble on every rank
+
+    ``integ.outputs()`` of each rank's shard (`DeviceImex.outputs`), put
+    together along the member axis in rank order -- the contiguous, possibly
+    uneven shards of `shard_members` -- by one ``all_gather`` (NCCL on the
+    device, gloo on the host).  Returns ``dict(y=(levels, ny, nmembers),
+    force=(levels, 2, nmembers))`` as numpy arrays; every rank must have
+    recorded the same levels.
+    """
+    import torch
+    import torch.distributed as dist
+    out = integ.outputs()
+    if not (dist.is_available() and dist.is_initialized()) \
+            or dist.get_world_size(group) == 1:
+        return out
+    world = dist.get_world_size(group)
+    rank = dist.get_rank(group)
+    dev = torch.device('cuda', torch.cuda.current_device()) \
+        if dist.get_backend(group) == 'nccl' else torch.device('cpu')
+    nb = out['force'].shape[2]
+    cnt = torch.tensor([nb], dtype=torch.int64, device=dev)
+    dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=group)
+    nmembers = int(cnt.item())
+    sizes = [hi - lo for lo, hi in (shard_members(nmembers, r, world)
+                                    for r in range(world))]
+    if sizes[rank] != nb:
+        raise ValueError('rank {0} holds {1} members, shard_members gives it '
+                         '{2}'.format(rank, nb, sizes[rank]))
+    per = max(sizes)
+    res = {}
+    for key in ('y', 'force'):
+        a = np.asarray(out[key], dtype=float)
+        pad = np.zeros(a.shape[:2] + (per,))
+        pad[:, :, :nb] = a
+        t = torch.from_numpy(pad).to(dev)
+        parts = [torch.empty_like(t) for _ in range(world)]
+        dist.all_gather(parts, t, group=group)
+        res[key] = np.concatenate([p.cpu().numpy()[:, :, :sizes[r]]
+                                   for r, p in enumerate(parts)], axis=2)
+    return res
 
 
 def pod_from_gram(G, energy=0.9999, kmax=None):

@@ -15,11 +15,13 @@ indicator of the obstacle's dofs gives drag and lift
 (`tests/steadystate_schaefer-turek_2D-1.py:71-85`).
 """
 import numpy as np
+import scipy.sparse as sps
 
 from . import dolfin_to_sparrays as dts
 from . import fem
 
-__all__ = ['get_steady_state_res', 'get_imex_res', 'lift_drag_via_residual']
+__all__ = ['get_steady_state_res', 'get_imex_res', 'get_imex_force_rows',
+           'lift_drag_via_residual']
 
 
 def _flat(vec):
@@ -84,6 +86,48 @@ def get_imex_res(V=None, outflowds=None, gradvsymmtrc=True, nu=None,
         return _test(res, phi)
 
     return imex_res
+
+
+def get_imex_force_rows(V=None, invinds=None, dbcinds=None, dbcvals=None,
+                        ldsbcinds=None, force_ops=None, outflowds=None,
+                        gradvsymmtrc=True):
+    """the drag/lift functional of `get_imex_res` (crni/abtw) as fixed rows
+
+    Testing the residual with the indicator ``phi`` of the x (row 0) and y
+    (row 1) components of the dofs ``ldsbcinds`` gives, for full velocities
+    whose Dirichlet values ``u_bc`` are the same at every level,
+
+        F = fm (v - vl)/dt + nu (fa (v + vl)/2 + fa_bc) - fj p
+            + phi^T (3/2 c(vl) - 1/2 c(vo))
+
+    with ``v``, ``vl`` the inner velocities (``invinds`` order) of the current
+    and the last level: ``fm = phi^T M[:, inv]``, ``fa = phi^T A[:, inv]``
+    (2 x NV), ``fj = phi^T JT`` (2 x NP), ``fa_bc = phi^T A[:, bc] u_bc`` (the
+    mass part of the boundary values cancels).  ``force_ops``: the uncondensed
+    nu = 1 operators ``dict(M=, A=, JT=)`` of `dts.get_stokessysmats`, built
+    from ``V`` if omitted.  Only the convection depends on the state nonlinearly;
+    it stays a vector.  Returns ``dict(fm, fa, fj, fa_bc, dofs, phi)``.
+    """
+    sm = force_ops if force_ops is not None else \
+        _operators(V, outflowds, gradvsymmtrc, 1., False)
+    M, A, JT = (sps.csr_matrix(sm[k]) for k in ('M', 'A', 'JT'))
+    nvf = M.shape[0]
+    dofs = np.unique(np.asarray(ldsbcinds, dtype=np.int64).reshape(-1))
+    if dofs.size and (dofs[0] < 0 or dofs[-1] >= nvf):
+        raise ValueError('force dofs out of range (full velocity numbering, '
+                         '{0} dofs)'.format(nvf))
+    phi = sps.csr_matrix((np.ones(dofs.size), (dofs % 2, dofs)),
+                         shape=(2, nvf))
+    aux = {}                    # Dirichlet data: last write wins (`dts:534-535`)
+    for i, v in zip(dbcinds, dbcvals):
+        aux[int(i)] = float(v)
+    bci = np.array(sorted(aux.keys()), dtype=np.int64)
+    ubc = np.array([aux[i] for i in bci], dtype=float)
+    inv = np.asarray(invinds, dtype=np.int64)
+    pM, pA = (phi@M).tocsc(), (phi@A).tocsc()
+    return dict(fm=pM[:, inv].tocsr(), fa=pA[:, inv].tocsr(),
+                fj=(phi@JT).tocsr(), fa_bc=pA[:, bci]@ubc, dofs=dofs,
+                phi=phi)
 
 
 def lift_drag_via_residual(steady_state_res, vel, pres, ldsbcinds, rho=1.,

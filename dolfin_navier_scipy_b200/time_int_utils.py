@@ -160,6 +160,8 @@ class DeviceImex(object):
             aux[int(i)] = float(v)
         bci = np.array(sorted(aux.keys()), dtype=np.int32)
         bcv = np.array([aux[i] for i in bci], dtype=float)
+        self._bcs = (bci, bcv)
+        self.ny = 0
         self.dev = _lib.device_for(V, self.ctx)
         ctx = self.ctx
         self.mmat = ctx.csr(Mp)
@@ -230,6 +232,71 @@ class DeviceImex(object):
         (valid until the next run)"""
         s = self.engine.snapshots() if copy else self.engine.snapshots_view()
         return s[:, :self.NV, :], s[:, self.NV:, :]
+
+    def set_outputs(self, cv_mat=None, cp_mat=None, force_dofs=None,
+                    force_ops=None):
+        """record output functionals at every time level inside the loop
+
+        ``y_n = cv_mat v_n + cp_mat p_n`` (``cv_mat`` ny x NV on the inner
+        velocity, ``cp_mat`` ny x NP, the caller's numbering; the reference's
+        ``cv_mat.dot(v)``) and, with ``force_dofs`` (full velocity dofs such
+        as ``ldsbcinds``; CNAB only), the raw x / y force: the CNAB residual
+        of `residual_checks.get_imex_res` with ``nu = nus[m]`` tested with
+        their indicator.  ``force_ops``: the uncondensed nu = 1 ``M``, ``A``,
+        ``JT`` (`dts.get_stokessysmats`), built from ``V`` if omitted.  No
+        argument switches the outputs off.  Read them with `outputs`.
+        """
+        from . import residual_checks
+        cv = None if cv_mat is None else sps.csr_matrix(cv_mat)
+        cp = None if cp_mat is None else sps.csr_matrix(cp_mat)
+        if cv is not None and cv.shape[1] != self.NV:
+            raise ValueError('cv_mat must have NV = {0} columns, not {1}'.
+                             format(self.NV, cv.shape[1]))
+        if cp is not None and cp.shape[1] != self.NP:
+            raise ValueError('cp_mat must have NP = {0} columns, not {1}'.
+                             format(self.NP, cp.shape[1]))
+        if cv is not None and cp is not None and cv.shape[0] != cp.shape[0]:
+            raise ValueError('cv_mat and cp_mat must have the same rows')
+        if force_dofs is not None and self.scheme != 'cnab':
+            raise NotImplementedError(
+                'forces are the CNAB residual (`get_imex_res`, crni/abtw); '
+                'scheme {0!r} has none'.format(self.scheme))
+        rows = None
+        if force_dofs is not None:
+            rows = residual_checks.get_imex_force_rows(
+                V=self.V, invinds=self.invinds, dbcinds=self._bcs[0],
+                dbcvals=self._bcs[1], ldsbcinds=force_dofs,
+                force_ops=force_ops)
+        ctx, pv, pp = self.ctx, self.pv, self.pp
+        mats = [None if cv is None else ctx.csr(cv[:, pv]),
+                None if cp is None else ctx.csr(cp[:, pp])]
+        if rows is not None:
+            mats += [ctx.csr(rows['fm'][:, pv]), ctx.csr(rows['fa'][:, pv]),
+                     ctx.csr(rows['fj'][:, pp])]
+        try:
+            self.engine.set_outputs(*mats[:2])
+            if rows is None:
+                self.engine.set_force()
+            else:
+                self.engine.set_force(rows['dofs'], *mats[2:],
+                                      fa_bc=rows['fa_bc'])
+        finally:
+            for m in mats:              # the engine keeps its own copy
+                if m is not None:
+                    m.close()
+        self.ny = 0 if cv is None and cp is None else \
+            (cv if cv is not None else cp).shape[0]
+
+    def outputs(self):
+        """``dict(y=(levels, ny, nb), force=(levels, 2, nb))`` recorded since
+        `set_state` / `reset_outputs` (members in the order of ``nus``; the
+        force is NaN at levels 0 and 1)"""
+        y, f = self.engine.outputs(self.ny)
+        return dict(y=y, force=f)
+
+    def reset_outputs(self):
+        """start a new record (the next run first records the current state)"""
+        self.engine.reset_outputs()
 
     def reserve_snapshots(self, nsnap):
         self.engine.reserve_snapshots(nsnap)

@@ -233,6 +233,34 @@ int dnsb_imex_set_output_order(dnsb_imex *e, const int32_t *vmap, const int32_t 
  * zero-copy view for the ctypes caller. */
 int dnsb_imex_reserve_snapshots(dnsb_imex *e, int nsnap);
 int dnsb_imex_snapshots_host(dnsb_imex *e, const double **ptr, int *nsnap);
+/* Output functionals recorded inside the loop at every time level (the
+ * initial state and the Heun level included), for all members, by one kernel
+ * per step that only reads the state; the values stay on the device until
+ * dnsb_imex_get_outputs.  A record holds (levels, ny + 2, nb) values: ny
+ * linear outputs and the x / y force.  It starts empty at dnsb_imex_set_state,
+ * dnsb_imex_reset_outputs and whenever the rows change, and a run appends to
+ * it (a run on an empty record first records the current state).
+ * Linear outputs  y_n = Cv v_n + Cp p_n  (the reference's `cv_mat.dot(v)`,
+ * stokes_navier_utils.py:1144-1150): `cv` ny x nv on the inner velocity, `cp`
+ * ny x np, columns in the device numbering; either may be NULL, both NULL = no
+ * linear outputs. */
+int dnsb_imex_set_outputs(dnsb_imex *e, dnsb_csr *cv, dnsb_csr *cp);
+/* Force (CNAB only): the CNAB weak residual of residual_checks.get_imex_res
+ * (crni/abtw, nu = nu[m]) tested with the indicator Phi of the x / y
+ * components of the `ndofs` full-numbering velocity dofs `dofs`:
+ *   F_n = Phi^T [ M (V_n - V_{n-1})/dt + nu_m A0 (V_n + V_{n-1})/2
+ *                 + 3/2 c(V_{n-1}) - 1/2 c(V_{n-2}) - JT p_n ]
+ * with the uncondensed nu = 1 operators reduced to rows: fm = Phi^T M[:, inv]
+ * and fa = Phi^T A0[:, inv] (2 x nv), fj = Phi^T JT (2 x np), fa_bc[2] =
+ * Phi^T A0[:, bc] u_bc (scaled by nu_m).  Defined for n >= 2 (NaN at levels 0
+ * and 1 and at the first level after the rows were set mid-run).  ndofs = 0
+ * switches the force off; scheme != 0 is refused. */
+int dnsb_imex_set_force(dnsb_imex *e, int ndofs, const int32_t *dofs, dnsb_csr *fm,
+                        dnsb_csr *fa, dnsb_csr *fj, const double *fa_bc);
+int dnsb_imex_num_output_levels(dnsb_imex *e);
+/* y: (levels, ny, nb), force: (levels, 2, nb); either may be NULL */
+int dnsb_imex_get_outputs(dnsb_imex *e, double *y, double *force);
+int dnsb_imex_reset_outputs(dnsb_imex *e);
 /* solver statistics of the last run: total FGMRES iterations (max over
  * members per solve, summed over the loop solves), number of loop solves, and
  * the LARGEST final relative residual over all solves of the run (every
