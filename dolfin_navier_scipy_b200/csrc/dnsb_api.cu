@@ -64,6 +64,43 @@
     c_->launches++;                                                            \
   } while (0)
 
+// Runtime flags and values to template arguments.  Each instantiation gets a LAUNCH of its own because
+// #kern, spelled as written here, is the kernel's name in the profile, which bench.py and the tests match on.
+//   LAUNCH_IF(ctx, c, K1, K0, ...)            K1 if c, else K0
+//   LAUNCH_B(ctx, K, b, ...)                  K<b>
+//   LAUNCH_BB(ctx, K, b0, b1, ...)            (K<b0, b1>)
+//   LAUNCH_XBB(ctx, K, X, b0, b1, ...)        (K<X, b0, b1>) for a constant X
+//   LAUNCH_BBB(ctx, K, b0, b1, b2, ...)       (K<b0, b1, b2>)
+//   LAUNCH_N3(ctx, K, c0, a, c1, b, c, ...)   K<a> if c0, else K<b> if c1, else K<c>; LAUNCH_N4 likewise
+#define LAUNCH_IF(ctx, c, K1, K0, ...) \
+  do { if (c) LAUNCH(ctx, K1, __VA_ARGS__); else LAUNCH(ctx, K0, __VA_ARGS__); } while (0)
+#define LAUNCH_B(ctx, K, b, ...) LAUNCH_IF(ctx, b, K<true>, K<false>, __VA_ARGS__)
+#define LAUNCH_BB(ctx, K, b0, b1, ...)                                                   \
+  do {                                                                                   \
+    if (b0) LAUNCH_IF(ctx, b1, (K<true, true>), (K<true, false>), __VA_ARGS__);         \
+    else LAUNCH_IF(ctx, b1, (K<false, true>), (K<false, false>), __VA_ARGS__);          \
+  } while (0)
+#define LAUNCH_XBB(ctx, K, X, b0, b1, ...)                                               \
+  do {                                                                                   \
+    if (b0) LAUNCH_IF(ctx, b1, (K<X, true, true>), (K<X, true, false>), __VA_ARGS__);   \
+    else LAUNCH_IF(ctx, b1, (K<X, false, true>), (K<X, false, false>), __VA_ARGS__);    \
+  } while (0)
+#define LAUNCH_BBB(ctx, K, b0, b1, b2, ...)                                              \
+  do {                                                                                   \
+    if (b0) LAUNCH_XBB(ctx, K, true, b1, b2, __VA_ARGS__);                               \
+    else LAUNCH_XBB(ctx, K, false, b1, b2, __VA_ARGS__);                                 \
+  } while (0)
+#define LAUNCH_N3(ctx, K, c0, a, c1, b, c, ...)                                          \
+  do {                                                                                   \
+    if (c0) LAUNCH(ctx, K<a>, __VA_ARGS__);                                              \
+    else LAUNCH_IF(ctx, c1, K<b>, K<c>, __VA_ARGS__);                                    \
+  } while (0)
+#define LAUNCH_N4(ctx, K, c0, a, c1, b, c2, c, d, ...)                                   \
+  do {                                                                                   \
+    if (c0) LAUNCH(ctx, K<a>, __VA_ARGS__);                                              \
+    else LAUNCH_N3(ctx, K, c1, b, c2, c, d, __VA_ARGS__);                                \
+  } while (0)
+
 static inline int pow2_floor(int x) {
   int p = 1;
   while (2 * p <= x) p *= 2;
@@ -443,12 +480,8 @@ static void spt_launch_epi(dnsb_ctx *ctx, const dnsb_csr *A, const double *coef,
                            const SptEpi &ep) {
   const SptPlan &p = A->spt;
   const unsigned grid = (unsigned)std::min(p.ntiles, ctx->sm_count * p.ctas_per_sm);
-  if (A->has2 && coef)
-    LAUNCH(ctx, (k_spmv_tma<true, EPI>), grid, SPT_THREADS, p.smem, A->view(), coef, x, ep, p.ntiles,
-           p.cap, p.stages, p.rt);
-  else
-    LAUNCH(ctx, (k_spmv_tma<false, EPI>), grid, SPT_THREADS, p.smem, A->view(), coef, x, ep, p.ntiles,
-           p.cap, p.stages, p.rt);
+  LAUNCH_IF(ctx, A->has2 && coef, (k_spmv_tma<true, EPI>), (k_spmv_tma<false, EPI>), grid, SPT_THREADS, p.smem,
+            A->view(), coef, x, ep, p.ntiles, p.cap, p.stages, p.rt);
 }
 static void spt_launch(dnsb_ctx *ctx, const dnsb_csr *A, const double *coef, const double *x,
                        const double *z, double *y, double alpha, double beta) {
@@ -478,12 +511,8 @@ static void spmm_dev(dnsb_ctx *ctx, const dnsb_csr *A, const double *coef,
       const TileDev tv = A->tile_view();
       const int ntw = row_begin < A->nrows ? g_tail_warps : 0;
       const int threads_ = TILE_THREADS + 32 * ntw;
-      if (beta != 0.0)
-        LAUNCH(ctx, k_spmm_tile<true>, grid_, threads_, A->tile.smem, tv, coef, x, z, y, alpha, beta, A->view(),
-               row_begin);
-      else
-        LAUNCH(ctx, k_spmm_tile<false>, grid_, threads_, A->tile.smem, tv, coef, x, z, y, alpha, beta, A->view(),
-               row_begin);
+      LAUNCH_B(ctx, k_spmm_tile, beta != 0.0, grid_, threads_, A->tile.smem, tv, coef, x, z, y, alpha, beta,
+               A->view(), row_begin);
       if (row_begin < A->nrows && ntw == 0)
         LAUNCH(ctx, k_spmm_b2<true>, spb2_grid(A->nrows - row_begin, nb), SPB_THREADS, 0, A->view(), coef, D2C(x),
                D2C(z), D2(y), nb, row_begin, alpha, beta);
@@ -491,35 +520,19 @@ static void spmm_dev(dnsb_ctx *ctx, const dnsb_csr *A, const double *coef,
       // paired rows and a tail of single rows (K = [F JT; J 0]) in one launch
       const unsigned tb = spb2_grid(A->nrows - row_begin, nb);
       const unsigned grid = tb + spp_grid(npairs, nb);
-      if (h2)
-        LAUNCH(ctx, k_spmm_k2<true>, grid, SPB_THREADS, 0, A->view(), coef, D2C(x), D2C(z), D2(y), nb,
-               npairs, (int)tb, alpha, beta);
-      else
-        LAUNCH(ctx, k_spmm_k2<false>, grid, SPB_THREADS, 0, A->view(), coef, D2C(x), D2C(z), D2(y), nb,
-               npairs, (int)tb, alpha, beta);
+      LAUNCH_B(ctx, k_spmm_k2, h2, grid, SPB_THREADS, 0, A->view(), coef, D2C(x), D2C(z), D2(y), nb, npairs,
+               (int)tb, alpha, beta);
     } else if (npairs > 0) {
-      if (h2)
-        LAUNCH(ctx, k_spmm_p2<true>, spp_grid(npairs, nb), SPB_THREADS, 0, A->view(), coef, D2C(x),
-               D2C(z), D2(y), nb, npairs, alpha, beta);
-      else
-        LAUNCH(ctx, k_spmm_p2<false>, spp_grid(npairs, nb), SPB_THREADS, 0, A->view(), coef, D2C(x),
-               D2C(z), D2(y), nb, npairs, alpha, beta);
+      LAUNCH_B(ctx, k_spmm_p2, h2, spp_grid(npairs, nb), SPB_THREADS, 0, A->view(), coef, D2C(x), D2C(z), D2(y),
+               nb, npairs, alpha, beta);
     } else {
-      if (h2)
-        LAUNCH(ctx, k_spmm_b2<true>, spb2_grid(A->nrows, nb), SPB_THREADS, 0, A->view(),
-               coef, D2C(x), D2C(z), D2(y), nb, 0, alpha, beta);
-      else
-        LAUNCH(ctx, k_spmm_b2<false>, spb2_grid(A->nrows, nb), SPB_THREADS, 0, A->view(),
-               coef, D2C(x), D2C(z), D2(y), nb, 0, alpha, beta);
+      LAUNCH_B(ctx, k_spmm_b2, h2, spb2_grid(A->nrows, nb), SPB_THREADS, 0, A->view(), coef, D2C(x), D2C(z),
+               D2(y), nb, 0, alpha, beta);
     }
   } else if (batched_ok(A, nb)) {
     const int gpc = spb_gpc(ctx, A->nrows, nb);
-    if (A->has2 && coef)
-      LAUNCH(ctx, k_spmm_b<true>, spb_grid(A->nrows, nb, gpc), SPB_THREADS, 0, A->view(), coef,
-             x, z, y, nb, gpc, alpha, beta);
-    else
-      LAUNCH(ctx, k_spmm_b<false>, spb_grid(A->nrows, nb, gpc), SPB_THREADS, 0, A->view(), coef,
-             x, z, y, nb, gpc, alpha, beta);
+    LAUNCH_B(ctx, k_spmm_b, A->has2 && coef, spb_grid(A->nrows, nb, gpc), SPB_THREADS, 0, A->view(), coef, x, z,
+             y, nb, gpc, alpha, beta);
   } else if (nb == 1) {
     const size_t threads = (size_t)A->nrows * 8;
     LAUNCH(ctx, k_spmm<8>, cdiv(threads, 256), 256, 0, A->view(), coef, x, z, y,
@@ -566,17 +579,14 @@ static void fill_tabulation(double phi[7][6], double dphi[7][6][3], double qw[7]
   X(g_dmma) X(g_schur_tf32) X(g_schur_tc) X(g_tile) X(g_gs_pyth) X(g_schur_l2keep) X(g_tile_stages)             \
   X(g_tile_stages_f) X(g_tail_warps) X(g_pkeep) X(g_proj_t) X(g_cheb_f32) X(g_conv_colours) X(g_rowpair)         \
   X(g_graphs) X(g_dense_ctas_per_sm) X(g_tilef_ctas) X(g_tc_ctas) X(g_init_tile)
-static void switches_store(int *sw) {
-  int k = 0;
-#define X(name) sw[k++] = name;
-  DNSB_SWITCH_LIST(X)
+#define X(name) &name,
+static int *const g_switches[] = {DNSB_SWITCH_LIST(X)};
 #undef X
+static void switches_store(int *sw) {
+  for (const int *v : g_switches) *sw++ = *v;
 }
 static void switches_load(const int *sw) {
-  int k = 0;
-#define X(name) name = sw[k++];
-  DNSB_SWITCH_LIST(X)
-#undef X
+  for (int *v : g_switches) *v = *sw++;
 }
 static const dnsb_ctx *g_switch_owner = nullptr;
 static inline cudaError_t dnsb_enter(const dnsb_ctx *ctx) {
@@ -585,6 +595,14 @@ static inline cudaError_t dnsb_enter(const dnsb_ctx *ctx) {
 }
 
 extern "C" int dnsb_version(void) { return DNSB_VERSION; }
+
+// lets each kernel use up to `bytes` of dynamic shared memory
+template <class... K>
+static cudaError_t smem_optin(int bytes, K *...kern) {
+  for (const void *k : {(const void *)kern...})
+    if (const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)) return e;
+  return cudaSuccess;
+}
 
 extern "C" int dnsb_ctx_create(int device, dnsb_ctx **out) {
   if (!out) return -2;
@@ -642,35 +660,24 @@ extern "C" int dnsb_ctx_create(int device, dnsb_ctx **out) {
   DNSB_CK(ctx, cudaMemcpyToSymbol(c_dphi, dphi, sizeof dphi));
   DNSB_CK(ctx, cudaMemcpyToSymbol(c_qw, qw, sizeof qw));
   DNSB_CK(ctx, cudaMemcpyToSymbol(c_lam, lam, sizeof lam));
-  // k_mdot_b keeps (nvec+1) x 256 partial sums in dynamic shared memory
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_mdot_b, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_gs_tma<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_gs_tma<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-#define SPT_ATTR(E)                                                                                  \
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_spmv_tma<true, E>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                    (int)SPT_SMEM_OPTIN));                                           \
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_spmv_tma<false, E>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                    (int)SPT_SMEM_OPTIN));
-  SPT_ATTR(SPT_AXPBY) SPT_ATTR(SPT_CHEB_INIT) SPT_ATTR(SPT_CHEB_STEP) SPT_ATTR(SPT_CHEB_STEP_FIRST)
-  SPT_ATTR(SPT_CHEB_STEP_LAST) SPT_ATTR(SPT_CHEB_STEP_ONLY)
-#undef SPT_ATTR
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_dense_dmma_streamk, cudaFuncAttributeMaxDynamicSharedMemorySize, DMM_SMEM_BYTES));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_dense_tf32_streamk<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TFM_SMEM_BYTES));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_dense_tf32_streamk<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TFM_SMEM_BYTES));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_dense_tf32_streamk<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TFM_SMEM_BYTES));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_schur_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_gmres_givens, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tile<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tile<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tile<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tile<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_spmm_tile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_spmm_tile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_init_tilef, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tilef<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tilef<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tilef<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
-  DNSB_CK(ctx, cudaFuncSetAttribute(k_cheb_step_tilef<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TILE_SMEM_OPTIN));
+  // every kernel that takes more than 48 KB of dynamic shared memory, by the most it takes
+  DNSB_CK(ctx, smem_optin(200 * 1024, k_mdot_b));   // (nvec+1) x 256 partial sums
+  DNSB_CK(ctx, smem_optin(112 * 1024, k_gs_tma<false>, k_gs_tma<true>));
+  DNSB_CK(ctx, smem_optin((int)SPT_SMEM_OPTIN, k_spmv_tma<true, SPT_AXPBY>, k_spmv_tma<false, SPT_AXPBY>,
+                          k_spmv_tma<true, SPT_CHEB_INIT>, k_spmv_tma<false, SPT_CHEB_INIT>,
+                          k_spmv_tma<true, SPT_CHEB_STEP>, k_spmv_tma<false, SPT_CHEB_STEP>,
+                          k_spmv_tma<true, SPT_CHEB_STEP_FIRST>, k_spmv_tma<false, SPT_CHEB_STEP_FIRST>,
+                          k_spmv_tma<true, SPT_CHEB_STEP_LAST>, k_spmv_tma<false, SPT_CHEB_STEP_LAST>,
+                          k_spmv_tma<true, SPT_CHEB_STEP_ONLY>, k_spmv_tma<false, SPT_CHEB_STEP_ONLY>));
+  DNSB_CK(ctx, smem_optin(DMM_SMEM_BYTES, k_dense_dmma_streamk));
+  DNSB_CK(ctx, smem_optin(TFM_SMEM_BYTES, k_dense_tf32_streamk<1>, k_dense_tf32_streamk<2>, k_dense_tf32_streamk<3>));
+  DNSB_CK(ctx, smem_optin(TC_SMEM_OPTIN, k_schur_tc));
+  DNSB_CK(ctx, smem_optin(96 * 1024, k_gmres_givens));
+  DNSB_CK(ctx, smem_optin(TILE_SMEM_OPTIN, k_cheb_step_tile<true, true>, k_cheb_step_tile<true, false>,
+                          k_cheb_step_tile<false, true>, k_cheb_step_tile<false, false>, k_spmm_tile<true>,
+                          k_spmm_tile<false>, k_cheb_init_tilef, k_cheb_step_tilef<true, true>,
+                          k_cheb_step_tilef<true, false>, k_cheb_step_tilef<false, true>,
+                          k_cheb_step_tilef<false, false>));
   return 0;
 }
 
@@ -1582,14 +1589,9 @@ static int dense_apply(dnsb_solver *s, MgLevel *L, const double *x,
            (size_t)p.mtiles * TC_BM * p.np_, p.np_, x, y, n, nb, alpha, ad, as);
     return 0;
   }
-  if (nb <= 1)
-    LAUNCH(ctx, k_dense_gemv<1>, cdiv((size_t)n * 32, 256), 256, 0, L->dinv_dense.p, x, y, n, nb, alpha, ad, as);
-  else if (nb <= 2)
-    LAUNCH(ctx, k_dense_gemv<2>, cdiv((size_t)n * 32, 256), 256, 0, L->dinv_dense.p, x, y, n, nb, alpha, ad, as);
-  else if (nb <= 4)
-    LAUNCH(ctx, k_dense_gemv<4>, cdiv((size_t)n * 32, 256), 256, 0, L->dinv_dense.p, x, y, n, nb, alpha, ad, as);
-  else if (nb <= 8)
-    LAUNCH(ctx, k_dense_gemv<8>, cdiv((size_t)n * 32, 256), 256, 0, L->dinv_dense.p, x, y, n, nb, alpha, ad, as);
+  if (nb <= 8)
+    LAUNCH_N4(ctx, k_dense_gemv, nb <= 1, 1, nb <= 2, 2, nb <= 4, 4, 8, cdiv((size_t)n * 32, 256), 256, 0,
+              L->dinv_dense.p, x, y, n, nb, alpha, ad, as);
   else {
     int tn;
     DenseSplit sp;
@@ -1597,21 +1599,13 @@ static int dense_apply(dnsb_solver *s, MgLevel *L, const double *x,
     const dim3 grid(sp.nctas, cdiv(nb, tn));
     if (g_schur_tf32 && L->dinv_f32.p && L->x_f32.p && tn == 64) {
       LAUNCH(ctx, k_f64_to_f32, cdiv((size_t)n * nb, 256), 256, 0, x, L->x_f32.p, (size_t)n, (size_t)nb, (size_t)nb);
-const float *df_ = L->dinv_f32.p, *xf_ = L->x_f32.p;
-      if (g_schur_tf32 == 1)
-        LAUNCH(ctx, k_dense_tf32_streamk<3>, grid, 128, TFM_SMEM_BYTES, df_, L->ldf, xf_, L->gpart.p, n, nb, sp);
-      else if (g_schur_tf32 == 2)
-        LAUNCH(ctx, k_dense_tf32_streamk<2>, grid, 128, TFM_SMEM_BYTES, df_, L->ldf, xf_, L->gpart.p, n, nb, sp);
-      else
-        LAUNCH(ctx, k_dense_tf32_streamk<1>, grid, 128, TFM_SMEM_BYTES, df_, L->ldf, xf_, L->gpart.p, n, nb, sp);
+      LAUNCH_N3(ctx, k_dense_tf32_streamk, g_schur_tf32 == 1, 3, g_schur_tf32 == 2, 2, 1, grid, 128, TFM_SMEM_BYTES,
+                (const float *)L->dinv_f32.p, L->ldf, (const float *)L->x_f32.p, L->gpart.p, n, nb, sp);
     } else if (g_dmma && nb > 32 && n % 2 == 0 && nb % 2 == 0)
       LAUNCH(ctx, k_dense_dmma_streamk, grid, 128, DMM_SMEM_BYTES, L->dinv_dense.p, x, L->gpart.p, n, nb, sp);
-    else if (tn == 16)
-      LAUNCH(ctx, k_dense_gemm_streamk<16>, grid, 128, 0, L->dinv_dense.p, x, L->gpart.p, n, nb, sp);
-    else if (tn == 32)
-      LAUNCH(ctx, k_dense_gemm_streamk<32>, grid, 128, 0, L->dinv_dense.p, x, L->gpart.p, n, nb, sp);
     else
-      LAUNCH(ctx, k_dense_gemm_streamk<64>, grid, 128, 0, L->dinv_dense.p, x, L->gpart.p, n, nb, sp);
+      LAUNCH_N3(ctx, k_dense_gemm_streamk, tn == 16, 16, tn == 32, 32, 64, grid, 128, 0, L->dinv_dense.p, x,
+                L->gpart.p, n, nb, sp);
     LAUNCH(ctx, k_dense_epilogue, cdiv((size_t)n * nb, 256), 256, 0, (const double *)L->gpart.p, sp, x,
            y, n, nb, alpha, ad, as);
   }
@@ -1638,9 +1632,10 @@ static void cheb_run(dnsb_solver *s, const dnsb_csr *A, const double *coef,
   const bool pair = pair_ok(A, nb) && (!C || pair_ok(C, nb));
   // all rows pair up (both components of every node are unknowns)?
   const bool rowpair = pair && rowpairs_of(A, nb) * 2 == n;
-  if (g_cheb_f32 && C && A == s->F && s->cf_res.p && rowpair && has2 && nb == TILE_NB && A->tile.ok && k >= 2 &&
-      rowpairs_of(C, nb) * 2 == n) {
-    // fp32 smoother (dnsb_tile.cuh): fp64 in (r, zc), fp64 out (z), work vectors and matrix values fp32
+  // fp32 smoother (dnsb_tile.cuh): fp64 in (r, zc), fp64 out (z), work vectors and matrix values fp32
+  const bool f32 = g_cheb_f32 && C && A == s->F && s->cf_res.p && rowpair && has2 && nb == TILE_NB && A->tile.ok &&
+                   k >= 2 && rowpairs_of(C, nb) * 2 == n;
+  if (f32) {
     if (g_init_tile && C->tile.ok && C->tile.npairs == n / 2) {
       const TilePlan &cp = C->tile;
       const int per_sm_i = 2 * (cp.smem + 2048) <= (size_t)227 * 1024 ? 2 : 1;
@@ -1650,26 +1645,7 @@ static void cheb_run(dnsb_solver *s, const dnsb_csr *A, const double *coef,
       LAUNCH(ctx, k_cheb_init_p2f, spp_grid(n / 2, nb), SPB_THREADS, 0, C->view(), D2C(zc), D2C(r),
              (const float2 *)s->cf_dinv.p, (float2 *)s->cf_res.p, (float2 *)s->cf_d0.p, nb, n / 2, (float)(1.0 / theta));
     }
-    float *dcf = s->cf_d0.p, *dnf = s->cf_d1.p;
-    const int per_sm_ = (g_tilef_ctas >= 2 && 2 * (A->tile.smem_f + 2048) <= (size_t)227 * 1024) ? 2 : 1;
-    const unsigned grid_ = std::min(A->tile.ntiles, per_sm_ * ctx->sm_count);
-    const TileDevF tv = A->tile_view_f();
-    for (int i = 0; i + 1 < k; ++i) {
-      const double rho_n = 1.0 / (2.0 * sigma - rho);
-      const float c1 = (float)(rho_n * rho), c2 = (float)(2.0 * rho_n / delta);
-      const bool first = i == 0, last = i + 2 == k;
-#define CHEB_ARGS_F tv, coef, (const float *)dcf, (const float *)s->cf_dinv.p, s->cf_res.p, dnf, s->cf_z.p, z, c1, c2
-      if (first && last) LAUNCH(ctx, (k_cheb_step_tilef<true, true>), grid_, TILE_THREADS, A->tile.smem_f, CHEB_ARGS_F);
-      else if (first) LAUNCH(ctx, (k_cheb_step_tilef<true, false>), grid_, TILE_THREADS, A->tile.smem_f, CHEB_ARGS_F);
-      else if (last) LAUNCH(ctx, (k_cheb_step_tilef<false, true>), grid_, TILE_THREADS, A->tile.smem_f, CHEB_ARGS_F);
-      else LAUNCH(ctx, (k_cheb_step_tilef<false, false>), grid_, TILE_THREADS, A->tile.smem_f, CHEB_ARGS_F);
-#undef CHEB_ARGS_F
-      std::swap(dcf, dnf);
-      rho = rho_n;
-    }
-    return;
-  }
-  if (C) {
+  } else if (C) {
     if (pair && rowpairs_of(C, nb) * 2 == n)
       LAUNCH(ctx, k_cheb_init_p2, spp_grid(n / 2, nb), SPB_THREADS, 0, C->view(), D2C(zc), D2C(r),
              D2C(dinv), D2(res), D2(dfirst), nb, n / 2, 1.0 / theta);
@@ -1692,84 +1668,43 @@ static void cheb_run(dnsb_solver *s, const dnsb_csr *A, const double *coef,
     LAUNCH(ctx, k_cheb_init_plain, cdiv(nn, 256), 256, 0, r, dinv, res, dfirst, nn, 1.0 / theta);
   }
   double *dc = d0, *dn = d1;
+  float *dcf = s->cf_d0.p, *dnf = s->cf_d1.p;
   for (int i = 0; i + 1 < k; ++i) {
     const double rho_n = 1.0 / (2.0 * sigma - rho);
     const double c1 = rho_n * rho, c2 = 2.0 * rho_n / delta;
     const bool first = i == 0, last = i + 2 == k;
-#define CHEB_ARGS A->view(), coef, (const double *)dc, dinv, res, dn, z, nb, c1, c2
-#define CHEB_ARGS_B A->view(), coef, (const double *)dc, dinv, res, dn, z, nb, gpc, c1, c2
-#define CHEB_DISPATCH_B(HAS2)                                                                       \
-    do {                                                                                            \
-      const unsigned grid_ = spb_grid(n, nb, gpc);                                                  \
-      if (first && last) LAUNCH(ctx, (k_cheb_step_b<HAS2, true, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_B);   \
-      else if (first) LAUNCH(ctx, (k_cheb_step_b<HAS2, true, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_B);     \
-      else if (last) LAUNCH(ctx, (k_cheb_step_b<HAS2, false, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_B);      \
-      else LAUNCH(ctx, (k_cheb_step_b<HAS2, false, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_B);               \
-    } while (0)
-#define CHEB_DISPATCH(KERN, GRID, BLK, ...)                                              \
-    do {                                                                                 \
-      if (first && last) LAUNCH(ctx, (KERN<__VA_ARGS__, true, true>), GRID, BLK, 0, CHEB_ARGS);       \
-      else if (first) LAUNCH(ctx, (KERN<__VA_ARGS__, true, false>), GRID, BLK, 0, CHEB_ARGS);         \
-      else if (last) LAUNCH(ctx, (KERN<__VA_ARGS__, false, true>), GRID, BLK, 0, CHEB_ARGS);          \
-      else LAUNCH(ctx, (KERN<__VA_ARGS__, false, false>), GRID, BLK, 0, CHEB_ARGS);                   \
-    } while (0)
-    if (rowpair) {
-#define CHEB_ARGS_R A->view(), coef, D2C(dc), D2C(dinv), D2(res), D2(dn), D2(z), nb, n / 2, c1, c2
-#define CHEB_DISPATCH_R(HAS2)                                                                       \
-    do {                                                                                            \
-      const unsigned grid_ = spp_grid(n / 2, nb);                                                   \
-      if (first && last) LAUNCH(ctx, (k_cheb_step_p2<HAS2, true, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_R);   \
-      else if (first) LAUNCH(ctx, (k_cheb_step_p2<HAS2, true, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_R);     \
-      else if (last) LAUNCH(ctx, (k_cheb_step_p2<HAS2, false, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_R);      \
-      else LAUNCH(ctx, (k_cheb_step_p2<HAS2, false, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_R);               \
-    } while (0)
-      if (has2 && nb == TILE_NB && A->tile.ok) {
-        // everything staged by TMA (dnsb_tile.cuh): persistent CTAs, one per SM
-        const unsigned grid_ = std::min(A->tile.ntiles, ctx->sm_count);
-        const TileDev tv = A->tile_view();
-#define CHEB_ARGS_T tv, coef, (const double *)dc, dinv, res, dn, z, c1, c2
-        if (first && last) LAUNCH(ctx, (k_cheb_step_tile<true, true>), grid_, TILE_THREADS, A->tile.smem, CHEB_ARGS_T);
-        else if (first) LAUNCH(ctx, (k_cheb_step_tile<true, false>), grid_, TILE_THREADS, A->tile.smem, CHEB_ARGS_T);
-        else if (last) LAUNCH(ctx, (k_cheb_step_tile<false, true>), grid_, TILE_THREADS, A->tile.smem, CHEB_ARGS_T);
-        else LAUNCH(ctx, (k_cheb_step_tile<false, false>), grid_, TILE_THREADS, A->tile.smem, CHEB_ARGS_T);
-#undef CHEB_ARGS_T
-      } else if (has2) CHEB_DISPATCH_R(true);
-      else CHEB_DISPATCH_R(false);
-#undef CHEB_DISPATCH_R
-#undef CHEB_ARGS_R
+    if (f32) {
+      const int per_sm = (g_tilef_ctas >= 2 && 2 * (A->tile.smem_f + 2048) <= (size_t)227 * 1024) ? 2 : 1;
+      LAUNCH_BB(ctx, k_cheb_step_tilef, first, last, std::min(A->tile.ntiles, per_sm * ctx->sm_count), TILE_THREADS,
+                A->tile.smem_f, A->tile_view_f(), coef, (const float *)dcf, (const float *)s->cf_dinv.p, s->cf_res.p,
+                dnf, s->cf_z.p, z, (float)c1, (float)c2);
+    } else if (rowpair && has2 && nb == TILE_NB && A->tile.ok) {
+      // everything staged by TMA (dnsb_tile.cuh): persistent CTAs, one per SM
+      LAUNCH_BB(ctx, k_cheb_step_tile, first, last, std::min(A->tile.ntiles, ctx->sm_count), TILE_THREADS,
+                A->tile.smem, A->tile_view(), coef, (const double *)dc, dinv, res, dn, z, c1, c2);
+    } else if (rowpair) {
+      LAUNCH_BBB(ctx, k_cheb_step_p2, has2, first, last, spp_grid(n / 2, nb), SPB_THREADS, 0, A->view(), coef,
+                 D2C(dc), D2C(dinv), D2(res), D2(dn), D2(z), nb, n / 2, c1, c2);
     } else if (pair) {
-#define CHEB_ARGS_P A->view(), coef, D2C(dc), D2C(dinv), D2(res), D2(dn), D2(z), nb, c1, c2
-#define CHEB_DISPATCH_P(HAS2)                                                                       \
-    do {                                                                                            \
-      const unsigned grid_ = spb2_grid(n, nb);                                                      \
-      if (first && last) LAUNCH(ctx, (k_cheb_step_b2<HAS2, true, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_P);   \
-      else if (first) LAUNCH(ctx, (k_cheb_step_b2<HAS2, true, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_P);     \
-      else if (last) LAUNCH(ctx, (k_cheb_step_b2<HAS2, false, true>), grid_, SPB_THREADS, 0, CHEB_ARGS_P);      \
-      else LAUNCH(ctx, (k_cheb_step_b2<HAS2, false, false>), grid_, SPB_THREADS, 0, CHEB_ARGS_P);               \
-    } while (0)
-      if (has2) CHEB_DISPATCH_P(true);
-      else CHEB_DISPATCH_P(false);
-#undef CHEB_DISPATCH_P
-#undef CHEB_ARGS_P
+      LAUNCH_BBB(ctx, k_cheb_step_b2, has2, first, last, spb2_grid(n, nb), SPB_THREADS, 0, A->view(), coef,
+                 D2C(dc), D2C(dinv), D2(res), D2(dn), D2(z), nb, c1, c2);
     } else if (batched) {
-      if (has2) CHEB_DISPATCH_B(true);
-      else CHEB_DISPATCH_B(false);
+      LAUNCH_BBB(ctx, k_cheb_step_b, has2, first, last, spb_grid(n, nb, gpc), SPB_THREADS, 0, A->view(), coef,
+                 (const double *)dc, dinv, res, dn, z, nb, gpc, c1, c2);
     } else if (spt_ok(A, nb)) {
-      SptEpi ep{nullptr, dinv, res, dn, z, c1, c2};
-      if (first && last) spt_launch_epi<SPT_CHEB_STEP_ONLY>(ctx, A, coef, dc, ep);
-      else if (first) spt_launch_epi<SPT_CHEB_STEP_FIRST>(ctx, A, coef, dc, ep);
-      else if (last) spt_launch_epi<SPT_CHEB_STEP_LAST>(ctx, A, coef, dc, ep);
-      else spt_launch_epi<SPT_CHEB_STEP>(ctx, A, coef, dc, ep);
+      static constexpr decltype(&spt_launch_epi<SPT_CHEB_STEP>) step[2][2] = {
+          {spt_launch_epi<SPT_CHEB_STEP>, spt_launch_epi<SPT_CHEB_STEP_LAST>},
+          {spt_launch_epi<SPT_CHEB_STEP_FIRST>, spt_launch_epi<SPT_CHEB_STEP_ONLY>}};   // [first][last]
+      step[first][last](ctx, A, coef, dc, SptEpi{nullptr, dinv, res, dn, z, c1, c2});
     } else if (nb == 1) {
-      CHEB_DISPATCH(k_cheb_step, cdiv((size_t)n * 8, 256), 256, 8);
+      LAUNCH_XBB(ctx, k_cheb_step, 8, first, last, cdiv((size_t)n * 8, 256), 256, 0, A->view(), coef,
+                 (const double *)dc, dinv, res, dn, z, nb, c1, c2);
     } else {
-      CHEB_DISPATCH(k_cheb_step, cdiv(nn, 256), 256, 1);
+      LAUNCH_XBB(ctx, k_cheb_step, 1, first, last, cdiv(nn, 256), 256, 0, A->view(), coef, (const double *)dc, dinv,
+                 res, dn, z, nb, c1, c2);
     }
-#undef CHEB_DISPATCH
-#undef CHEB_DISPATCH_B
-#undef CHEB_ARGS
-#undef CHEB_ARGS_B
     std::swap(dc, dn);
+    std::swap(dcf, dnf);
     rho = rho_n;
   }
 }
