@@ -32,6 +32,7 @@ SIGNATURES = {
     'dnsb_launch_count_reset': (None, [_vp]),
     'dnsb_profile_begin': (_i, [_vp, _i]),
     'dnsb_profile_end': (_i, [_vp, ctypes.c_char_p, _i]),
+    'dnsb_live_bytes': (None, [ctypes.POINTER(_ll), ctypes.POINTER(_ll)]),
     'dnsb_set_mesh': (_i, [_vp, _i, _i, c_int_p, c_dbl_p, _i, c_int_p]),
     'dnsb_set_conv_pattern': (_i, [_vp, c_int_p, c_int_p, c_int_p]),
     'dnsb_convvec': (_i, [_vp, c_dbl_p, c_dbl_p, c_dbl_p, _i]),
@@ -156,12 +157,14 @@ class Context(object):
         self.lib = load()
         h = ctypes.c_void_p()
         rc = self.lib.dnsb_ctx_create(int(device), ctypes.byref(h))
-        self.h = h
-        self.device = int(device)
         if rc != 0:
+            # a failed create still returns its context, for the message
             msg = self.lib.dnsb_last_error(h).decode() if h else 'no context'
+            self.lib.dnsb_ctx_destroy(h)
             raise DnsbError('dnsb_ctx_create(device={0}) failed: {1}'.
                             format(device, msg))
+        self.h = h
+        self.device = int(device)
         self._keep = []
 
     def check(self, rc):
@@ -211,6 +214,14 @@ class Context(object):
     # -- CSR ----------------------------------------------------------------
     def csr(self, mat, vals2=None):
         return Csr(self, mat, vals2)
+
+
+def live_bytes():
+    """``(device, pinned)`` bytes the library holds in this process"""
+    lib = load()
+    dev, pinned = _ll(), _ll()
+    lib.dnsb_live_bytes(ctypes.byref(dev), ctypes.byref(pinned))
+    return dev.value, pinned.value
 
 
 _CTX = {}

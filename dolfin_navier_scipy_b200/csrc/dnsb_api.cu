@@ -8,7 +8,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <ctime>
+#include <memory>
 #include <new>
 
 #include "dnsb_common.cuh"
@@ -218,6 +218,7 @@ struct dnsb_csr {
     a.v1 = v1.p; a.v2 = has2 ? v2.p : nullptr;
     return a;
   }
+  ~dnsb_csr() { cudaStreamSynchronize(ctx->stream); }   // no buffer is freed under a running kernel
 };
 
 template <typename T>
@@ -267,15 +268,15 @@ static SptPlan spt_plan(int nrows, const int32_t *indptr, bool h2) {
 
 static int csr_build(dnsb_ctx *ctx, int nrows, int ncols, const int32_t *indptr,
                      const int32_t *indices, const double *vals1,
-                     const double *vals2, dnsb_csr **out) {
-  DNSB_REQUIRE(ctx, nrows >= 0 && ncols >= 0 && indptr && out, "bad csr args");
+                     const double *vals2, std::unique_ptr<dnsb_csr> &out) {
+  DNSB_REQUIRE(ctx, nrows >= 0 && ncols >= 0 && indptr, "bad csr args");
   const int nnz = indptr[nrows];
   DNSB_REQUIRE(ctx, nnz >= 0 && (nnz == 0 || (indices && vals1)), "bad csr data");
   for (int i = 0; i < nrows; ++i)
     DNSB_REQUIRE(ctx, indptr[i] <= indptr[i + 1], "indptr not monotone");
   for (int k = 0; k < nnz; ++k)
     DNSB_REQUIRE(ctx, indices[k] >= 0 && indices[k] < ncols, "column index out of range");
-  dnsb_csr *m = new (std::nothrow) dnsb_csr();
+  std::unique_ptr<dnsb_csr> m(new (std::nothrow) dnsb_csr());
   DNSB_REQUIRE(ctx, m != nullptr, "out of host memory");
   m->ctx = ctx; m->nrows = nrows; m->ncols = ncols; m->nnz = nnz;
   m->has2 = vals2 != nullptr;
@@ -289,18 +290,12 @@ static int csr_build(dnsb_ctx *ctx, int nrows, int ncols, const int32_t *indptr,
   m->h_indices.assign(indices, indices + nnz);
   m->h_v1.assign(vals1, vals1 + nnz);
   if (vals2) m->h_v2.assign(vals2, vals2 + nnz);
-  cudaError_t e;
   // the bulk copies of the staged kernels read whole 16-byte groups: pad the arrays
-  if ((e = upload_padded(m->indptr, indptr, nrows + 1, 8, ctx->stream)) != cudaSuccess ||
-      (e = upload_padded(m->indices, indices, nnz, 4, ctx->stream)) != cudaSuccess ||
-      (e = upload_padded(m->v1, vals1, nnz, 4, ctx->stream)) != cudaSuccess ||
-      (vals2 && (e = upload_padded(m->v2, vals2, nnz, 4, ctx->stream)) != cudaSuccess)) {
-    ctx->fail(std::string("csr upload: ") + cudaGetErrorString(e), __FILE__, __LINE__);
-    m->indptr.release(); m->indices.release(); m->v1.release(); m->v2.release();
-    delete m;
-    return -1;
-  }
-  *out = m;
+  DNSB_CK(ctx, upload_padded(m->indptr, indptr, nrows + 1, 8, ctx->stream));
+  DNSB_CK(ctx, upload_padded(m->indices, indices, nnz, 4, ctx->stream));
+  DNSB_CK(ctx, upload_padded(m->v1, vals1, nnz, 4, ctx->stream));
+  if (vals2) DNSB_CK(ctx, upload_padded(m->v2, vals2, nnz, 4, ctx->stream));
+  out = std::move(m);
   return 0;
 }
 
@@ -411,14 +406,6 @@ static int tile_setup(dnsb_ctx *ctx, dnsb_csr *m, bool single = false) {
   }
   p.ok = true;
   return 0;
-}
-
-static void csr_free(dnsb_csr *m) {
-  if (!m) return;
-  m->t_uptr.release(); m->t_rptr.release(); m->t_runs.release(); m->t_pidx.release(); m->t_pval.release();
-  m->t_pidxf.release(); m->t_pvalf.release(); m->t_truns.release(); m->t_tdesc.release(); m->t_pdesc.release();
-  m->indptr.release(); m->indices.release(); m->v1.release(); m->v2.release();
-  delete m;
 }
 
 // the batched row kernels pre-multiply column indices by nb in int32
@@ -685,15 +672,12 @@ extern "C" void dnsb_ctx_destroy(dnsb_ctx *ctx) {
   if (!ctx) return;
   dnsb_enter(ctx);
   g_switch_owner = nullptr;
-  if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-  ctx->cn.release(); ctx->geom.release();
-  ctx->n2c_ptr.release(); ctx->n2c_idx.release(); ctx->elem.release();
-  ctx->cindptr.release(); ctx->cindices.release(); ctx->cslots.release();
-  ctx->cslot_ptr.release(); ctx->cslot_src.release(); ctx->en1.release(); ctx->en2.release();
-  ctx->stage_a.release(); ctx->stage_b.release();
-  ctx->stage_c.release(); ctx->stage_d.release();
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete ctx;
+}
+
+extern "C" void dnsb_live_bytes(long long *device, long long *pinned) {
+  if (device) *device = g_live_bytes[0];
+  if (pinned) *pinned = g_live_bytes[1];
 }
 
 extern "C" const char *dnsb_last_error(dnsb_ctx *ctx) {
@@ -717,8 +701,7 @@ extern "C" int dnsb_sync(dnsb_ctx *ctx) {
 extern "C" int dnsb_profile_begin(dnsb_ctx *ctx, int max_records) {
   if (!ctx) return -2;
   DNSB_CK(ctx, dnsb_enter(ctx));
-  for (ProfRec &r : ctx->recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
-  ctx->recs.clear();
+  ctx->drop_recs();
   ctx->prof_cap = max_records > 0 ? (size_t)max_records : 0;
   ctx->prof = max_records > 0;
   return 0;
@@ -741,9 +724,8 @@ extern "C" int dnsb_profile_end(dnsb_ctx *ctx, char *buf, int buflen) {
     for (; k < names.size(); ++k) if (names[k] == r.name) break;
     if (k == names.size()) { names.push_back(r.name); tot.push_back(0.0); cnt.push_back(0); work.push_back(0); }
     tot[k] += ms; cnt[k] += 1; work[k] += r.work;
-    cudaEventDestroy(r.e0); cudaEventDestroy(r.e1);
   }
-  ctx->recs.clear();
+  ctx->drop_recs();
   std::vector<size_t> order(names.size());
   for (size_t k = 0; k < order.size(); ++k) order[k] = k;
   std::sort(order.begin(), order.end(), [&](size_t a, size_t b) { return tot[a] > tot[b]; });
@@ -991,46 +973,35 @@ extern "C" int dnsb_assemble_stokes(dnsb_ctx *ctx, double nu, int symgrad, int j
   const size_t nnz = ctx->cnnz;
   DBuf<double> ej, emp, dm, da, dj, dmp;
   DBuf<int> jp, js, pp, ps;
-  int rc = 0;
-  do {
-    cudaError_t e;
-    if ((e = ctx->en1.alloc((size_t)36 * ncell)) != cudaSuccess || (e = ctx->en2.alloc((size_t)144 * ncell)) != cudaSuccess ||
-        (e = dm.alloc(nnz)) != cudaSuccess || (e = da.alloc(nnz)) != cudaSuccess ||
-        (j_vals && ((e = ej.alloc((size_t)36 * ncell)) != cudaSuccess || (e = dj.alloc(jnnz)) != cudaSuccess)) ||
-        (mp_vals && ((e = emp.alloc((size_t)9 * ncell)) != cudaSuccess || (e = dmp.alloc(mpnnz)) != cudaSuccess))) {
-      ctx->fail(std::string("assemble_stokes alloc: ") + cudaGetErrorString(e), __FILE__, __LINE__);
-      rc = -1;
-      break;
-    }
-    if (j_vals && (rc = slot_lists(ctx, 36, jnnz, jslots, jp, js))) break;
-    if (mp_vals && (rc = slot_lists(ctx, 9, mpnnz, mpslots, pp, ps))) break;
-    LAUNCH(ctx, k_stokes_elem, cdiv((size_t)ncell, CME_CELLS), 6 * CME_CELLS, 0, ncell,
-           (const double *)ctx->geom.p, nu, symgrad, ctx->en1.p, ctx->en2.p, j_vals ? ej.p : (double *)nullptr,
-           mp_vals ? emp.p : (double *)nullptr);
-    LAUNCH(ctx, k_convmats_gather, cdiv(nnz, 256), 256, 0, (int)nnz, ncell, (const int *)ctx->cslot_ptr.p,
-           (const int *)ctx->cslot_src.p, (const double *)ctx->en1.p, (const double *)ctx->en2.p, dm.p, da.p);
-    if (j_vals)
-      LAUNCH(ctx, k_slot_gather, cdiv((size_t)jnnz, 256), 256, 0, jnnz, (const int *)jp.p, (const int *)js.p,
-             (const double *)ej.p, dj.p);
-    if (mp_vals)
-      LAUNCH(ctx, k_slot_gather, cdiv((size_t)mpnnz, 256), 256, 0, mpnnz, (const int *)pp.p, (const int *)ps.p,
-             (const double *)emp.p, dmp.p);
-    cudaError_t ce = cudaMemcpyAsync(m_vals, dm.p, nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(a_vals, da.p, nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (ce == cudaSuccess && j_vals)
-      ce = cudaMemcpyAsync(j_vals, dj.p, (size_t)jnnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (ce == cudaSuccess && mp_vals)
-      ce = cudaMemcpyAsync(mp_vals, dmp.p, (size_t)mpnnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-    if (ce == cudaSuccess) ce = cudaGetLastError();
-    if (ce != cudaSuccess) {
-      ctx->fail(std::string("assemble_stokes: ") + cudaGetErrorString(ce), __FILE__, __LINE__);
-      rc = -1;
-    }
-  } while (0);
-  ej.release(); emp.release(); dm.release(); da.release(); dj.release(); dmp.release();
-  jp.release(); js.release(); pp.release(); ps.release();
-  return rc;
+  DNSB_CK(ctx, ctx->en1.alloc((size_t)36 * ncell));
+  DNSB_CK(ctx, ctx->en2.alloc((size_t)144 * ncell));
+  DNSB_CK(ctx, dm.alloc(nnz));
+  DNSB_CK(ctx, da.alloc(nnz));
+  if (j_vals) { DNSB_CK(ctx, ej.alloc((size_t)36 * ncell)); DNSB_CK(ctx, dj.alloc(jnnz)); }
+  if (mp_vals) { DNSB_CK(ctx, emp.alloc((size_t)9 * ncell)); DNSB_CK(ctx, dmp.alloc(mpnnz)); }
+  if (j_vals) { int rc = slot_lists(ctx, 36, jnnz, jslots, jp, js); if (rc) return rc; }
+  if (mp_vals) { int rc = slot_lists(ctx, 9, mpnnz, mpslots, pp, ps); if (rc) return rc; }
+  LAUNCH(ctx, k_stokes_elem, cdiv((size_t)ncell, CME_CELLS), 6 * CME_CELLS, 0, ncell,
+         (const double *)ctx->geom.p, nu, symgrad, ctx->en1.p, ctx->en2.p, j_vals ? ej.p : (double *)nullptr,
+         mp_vals ? emp.p : (double *)nullptr);
+  LAUNCH(ctx, k_convmats_gather, cdiv(nnz, 256), 256, 0, (int)nnz, ncell, (const int *)ctx->cslot_ptr.p,
+         (const int *)ctx->cslot_src.p, (const double *)ctx->en1.p, (const double *)ctx->en2.p, dm.p, da.p);
+  if (j_vals)
+    LAUNCH(ctx, k_slot_gather, cdiv((size_t)jnnz, 256), 256, 0, jnnz, (const int *)jp.p, (const int *)js.p,
+           (const double *)ej.p, dj.p);
+  if (mp_vals)
+    LAUNCH(ctx, k_slot_gather, cdiv((size_t)mpnnz, 256), 256, 0, mpnnz, (const int *)pp.p, (const int *)ps.p,
+           (const double *)emp.p, dmp.p);
+  DNSB_CK(ctx, cudaMemcpyAsync(m_vals, dm.p, nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  DNSB_CK(ctx, cudaMemcpyAsync(a_vals, da.p, nnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  if (j_vals)
+    DNSB_CK(ctx, cudaMemcpyAsync(j_vals, dj.p, (size_t)jnnz * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  if (mp_vals)
+    DNSB_CK(ctx, cudaMemcpyAsync(mp_vals, dmp.p, (size_t)mpnnz * sizeof(double), cudaMemcpyDeviceToHost,
+                                 ctx->stream));
+  DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  DNSB_CK(ctx, cudaGetLastError());
+  return 0;
 }
 
 extern "C" int dnsb_convmats(dnsb_ctx *ctx, const double *u0, double *n1_data,
@@ -1068,14 +1039,21 @@ extern "C" int dnsb_csr_create(dnsb_ctx *ctx, int nrows, int ncols,
                                const int32_t *indptr, const int32_t *indices,
                                const double *vals1, const double *vals2,
                                dnsb_csr **out) {
+  if (out) *out = nullptr;
   if (!ctx) return -2;
+  DNSB_REQUIRE(ctx, out != nullptr, "bad csr args");
   DNSB_CK(ctx, dnsb_enter(ctx));
-  return csr_build(ctx, nrows, ncols, indptr, indices, vals1, vals2, out);
+  std::unique_ptr<dnsb_csr> m;
+  int rc = csr_build(ctx, nrows, ncols, indptr, indices, vals1, vals2, m);
+  if (rc) return rc;
+  *out = m.release();
+  return 0;
 }
 
 extern "C" void dnsb_csr_destroy(dnsb_csr *mat) {
-  if (mat) dnsb_enter(mat->ctx);
-  csr_free(mat);
+  if (!mat) return;
+  dnsb_enter(mat->ctx);
+  delete mat;
 }
 
 extern "C" int dnsb_spmm_dev(dnsb_csr *mat, const double *coef_dev,
@@ -1139,7 +1117,7 @@ struct dnsb_solver {
   int nv = 0, np = 0, ntot = 0, nb = 1, mr = 30, kF = 3;
   double lmin = 0, lmax = 0;
   dnsb_csr *F = nullptr, *J = nullptr, *JT = nullptr;
-  dnsb_csr *K = nullptr;   // owned: [F JT; J 0]
+  std::unique_ptr<dnsb_csr> K;   // [F JT; J 0]
   DBuf<double> coef;       // nb (device copy)
   bool has_coef = false;
   DBuf<double> dinv;       // nv*nb
@@ -1154,9 +1132,9 @@ struct dnsb_solver {
   DBuf<int> gdone, gits, gittot, gflags;
   DBuf<double> grelmax;
   GmresState gs;
-  int *h_flags = nullptr;   // pinned
-  std::vector<MgLevel *> levels;    // Schur (pressure) hierarchy
-  std::vector<MgLevel *> vlevels;   // velocity hierarchy; [0] = F itself
+  PinnedBuf<int> h_flags;
+  std::vector<std::unique_ptr<MgLevel>> levels;    // Schur (pressure) hierarchy
+  std::vector<std::unique_ptr<MgLevel>> vlevels;   // velocity hierarchy; [0] = F itself
   DBuf<double> mp_dinv, mp_scale;
   bool has_mass = false;
   // least-squares-commutator Schur approximation (Stokes / Oseen / Newton)
@@ -1180,6 +1158,10 @@ struct dnsb_solver {
   bool use_pyth = false, igraph_pyth = false;
   long long stat_iters = 0, stat_solves = 0, stat_launched = 0;
   long long stat_unconverged = 0;   // solves that stopped at maxit above tol
+  ~dnsb_solver() {
+    cudaStreamSynchronize(ctx->stream);   // no buffer is freed under a running kernel
+    for (cudaGraphExec_t g : igraph) if (g) cudaGraphExecDestroy(g);
+  }
 };
 
 static void solver_drop_graphs(dnsb_solver *s);
@@ -1198,6 +1180,7 @@ extern "C" int dnsb_solver_create(dnsb_ctx *ctx, dnsb_csr *fmat, dnsb_csr *jmat,
                                   dnsb_csr *jtmat, const double *coef, int nb,
                                   int restart, int cheb_steps, double lmin,
                                   double lmax, dnsb_solver **out) {
+  if (out) *out = nullptr;
   if (!ctx) return -2;
   DNSB_REQUIRE(ctx, fmat && jmat && jtmat && out, "null matrices");
   DNSB_REQUIRE(ctx, nb >= 1 && nb <= 256, "nb must be in 1..256");
@@ -1209,12 +1192,11 @@ extern "C" int dnsb_solver_create(dnsb_ctx *ctx, dnsb_csr *fmat, dnsb_csr *jmat,
                jtmat->ncols == np, "inconsistent block shapes");
   DNSB_REQUIRE(ctx, !(fmat->has2 && !coef), "fmat has two value arrays: coef required");
   DNSB_CK(ctx, dnsb_enter(ctx));
-  dnsb_solver *s = new (std::nothrow) dnsb_solver();
+  std::unique_ptr<dnsb_solver> s(new (std::nothrow) dnsb_solver());
   DNSB_REQUIRE(ctx, s != nullptr, "out of host memory");
   s->ctx = ctx; s->nv = nv; s->np = np; s->ntot = nv + np; s->nb = nb;
   s->mr = restart; s->kF = cheb_steps; s->lmin = lmin; s->lmax = lmax;
   s->F = fmat; s->J = jmat; s->JT = jtmat;
-  *out = s;
   // ---- block matrix K = [F JT; J 0] on the host, then upload -------------
   {
     const int ntot = s->ntot;
@@ -1245,9 +1227,9 @@ extern "C" int dnsb_solver_create(dnsb_ctx *ctx, dnsb_csr *fmat, dnsb_csr *jmat,
       ip[nv + j + 1] = (int)ix.size();
     }
     int rc = csr_build(ctx, ntot, ntot, ip.data(), ix.data(), a1.data(),
-                       fmat->has2 ? a2.data() : nullptr, &s->K);
+                       fmat->has2 ? a2.data() : nullptr, s->K);
     if (rc) return rc;
-    if (nb == TILE_NB && coef) { int rct = tile_setup(ctx, s->K); if (rct) return rct; }
+    if (nb == TILE_NB && coef) { int rct = tile_setup(ctx, s->K.get()); if (rct) return rct; }
     // the block matrix is only needed on the device
     std::vector<int>().swap(s->K->h_indptr); std::vector<int>().swap(s->K->h_indices);
     std::vector<double>().swap(s->K->h_v1); std::vector<double>().swap(s->K->h_v2);
@@ -1272,15 +1254,15 @@ extern "C" int dnsb_solver_create(dnsb_ctx *ctx, dnsb_csr *fmat, dnsb_csr *jmat,
     LAUNCH(ctx, k_f64_to_f32, cdiv(nvb, 256), 256, 0, (const double *)s->dinv.p, s->cf_dinv.p, (size_t)1, nvb, nvb);
   }
   {
-    MgLevel *V0 = new (std::nothrow) MgLevel();
+    std::unique_ptr<MgLevel> V0(new (std::nothrow) MgLevel());
     DNSB_REQUIRE(ctx, V0 != nullptr, "out of host memory");
     V0->A = fmat; V0->coef = s->has_coef ? s->coef.p : nullptr;
     V0->n = nv; V0->nsmooth = s->kF; V0->kind = MG_SMOOTH;
     V0->lmin = lmin; V0->lmax = lmax; V0->dinv = s->dinv.p;
-    s->vlevels.push_back(V0);
     DNSB_CK(ctx, V0->b.alloc(nvb)); DNSB_CK(ctx, V0->r.alloc(nvb));
     DNSB_CK(ctx, V0->d0.alloc(nvb)); DNSB_CK(ctx, V0->d1.alloc(nvb));
     DNSB_CK(ctx, V0->t.alloc(nvb));
+    s->vlevels.push_back(std::move(V0));
   }
   DNSB_CK(ctx, s->Vb.alloc(ntb * (s->mr + 1)));
   DNSB_CK(ctx, s->Zb.alloc(ntb * s->mr));
@@ -1314,9 +1296,10 @@ extern "C" int dnsb_solver_create(dnsb_ctx *ctx, dnsb_csr *fmat, dnsb_csr *jmat,
   s->gs.h = s->gh.p; s->gs.invh = s->ginvh.p; s->gs.bnorm = s->gbnorm.p;
   s->gs.resid = s->gresid.p; s->gs.done = s->gdone.p; s->gs.its = s->gits.p;
   s->gs.ittot = s->gittot.p; s->gs.flags = s->gflags.p; s->gs.relmax = s->grelmax.p; s->gs.mr = mr;
-  DNSB_CK(ctx, cudaMallocHost((void **)&s->h_flags, 4 * sizeof(int)));
+  DNSB_CK(ctx, s->h_flags.alloc(4));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   DNSB_CK(ctx, cudaGetLastError());
+  *out = s.release();
   return 0;
 }
 
@@ -1392,46 +1375,9 @@ static cudaError_t tc_setup(dnsb_ctx *ctx, MgLevel *L, int n, int nb) {
   return cudaSuccess;
 }
 
-static void level_free(MgLevel *L) {
-  if (!L) return;
-  L->dinv_dense.release(); L->gpart.release(); L->dinv_f32.release(); L->x_f32.release(); L->xt.release(); L->tcpart.release(); L->dinv_own.release(); L->b.release(); L->x.release();
-  L->r.release(); L->d0.release(); L->d1.release(); L->t.release();
-  delete L;
-}
-
 extern "C" void dnsb_solver_destroy(dnsb_solver *s) {
   if (!s) return;
   dnsb_enter(s->ctx);
-  const bool trace = getenv("DNSB_TRACE_DESTROY") != nullptr;
-  auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
-  double t0 = now();
-  auto lap = [&](const char *what) { if (trace) { double t = now(); fprintf(stderr, "[destroy] %-12s %.2f ms\n", what, 1e3 * (t - t0)); t0 = t; } };
-  cudaStreamSynchronize(s->ctx->stream);
-  lap("sync");
-  for (cudaGraphExec_t g : s->igraph) if (g) cudaGraphExecDestroy(g);
-  s->igraph.clear();
-  lap("graphs");
-  csr_free(s->K);
-  lap("K");
-  s->coef.release(); s->dinv.release(); s->diagpos.release();
-  s->Vb.release(); s->Zb.release(); s->w.release();
-  lap("bases");
-  s->cf_res.release(); s->cf_d0.release(); s->cf_d1.release(); s->cf_z.release(); s->cf_dinv.release();
-  s->cres.release(); s->cd0.release(); s->cd1.release();
-  s->partial.release(); s->partial2.release(); s->red.release();
-  s->gR.release(); s->gcs.release(); s->gsn.release(); s->gg.release(); s->gh.release(); s->gh2.release();
-  s->ginvh.release(); s->gbnorm.release(); s->gresid.release(); s->grelmax.release();
-  s->gdone.release(); s->gits.release(); s->gittot.release(); s->gflags.release();
-  s->mp_dinv.release(); s->mp_scale.release(); s->sb.release(); s->sx.release();
-  s->zero_p.release();
-  s->lsc_dinv.release(); s->lsc_t1.release(); s->lsc_t2.release(); s->lsc_p1.release(); s->lsc_p2.release();
-  lap("small");
-  for (MgLevel *L : s->levels) level_free(L);
-  lap("levels");
-  for (MgLevel *L : s->vlevels) level_free(L);
-  lap("vlevels");
-  if (s->h_flags) cudaFreeHost(s->h_flags);
-  lap("pinned");
   delete s;
 }
 
@@ -1441,76 +1387,70 @@ static int solver_add_level(dnsb_solver *s, int block, dnsb_csr *amat, dnsb_csr 
                             const double *dense_inv) {
   dnsb_ctx *ctx = s->ctx;
   DNSB_CK(ctx, dnsb_enter(ctx));
-  std::vector<MgLevel *> &lv = block == 0 ? s->levels : s->vlevels;
+  std::vector<std::unique_ptr<MgLevel>> &lv = block == 0 ? s->levels : s->vlevels;
   solver_drop_graphs(s);   // the preconditioner changes: captured launch sequences are stale
   int nexpect;
   if (lv.empty()) {
     DNSB_REQUIRE(ctx, block == 0, "velocity level 0 is the matrix F itself");
     nexpect = s->np;
   } else {
-    MgLevel *up = lv.back();
+    const MgLevel *up = lv.back().get();
     DNSB_REQUIRE(ctx, up->kind == MG_MULTI && up->P, "previous level is terminal");
     nexpect = up->P->ncols;
   }
-  MgLevel *L = new (std::nothrow) MgLevel();
+  std::unique_ptr<MgLevel> L(new (std::nothrow) MgLevel());
   DNSB_REQUIRE(ctx, L != nullptr, "out of host memory");
   L->n = nexpect;
-  cudaError_t e = cudaSuccess;
   if (dense_inv) {
     L->kind = MG_DENSE;
-    e = L->dinv_dense.upload(dense_inv, (size_t)nexpect * nexpect, ctx->stream);
-    if (e == cudaSuccess && s->nb > 8) {
+    DNSB_CK(ctx, L->dinv_dense.upload(dense_inv, (size_t)nexpect * nexpect, ctx->stream));
+    if (s->nb > 8) {
       int tn;
       DenseSplit sp;
       dense_split(ctx, nexpect, s->nb, &tn, &sp);
-      e = L->gpart.alloc((size_t)sp.nctas * sp.maxseg * DGK_TM * s->nb);
-      if (e == cudaSuccess && g_schur_tf32 && s->nb % 4 == 0) {
+      DNSB_CK(ctx, L->gpart.alloc((size_t)sp.nctas * sp.maxseg * DGK_TM * s->nb));
+      if (g_schur_tf32 && s->nb % 4 == 0) {
         L->ldf = (nexpect + 3) & ~3;
-        if ((e = L->dinv_f32.alloc((size_t)nexpect * L->ldf)) == cudaSuccess &&
-            (e = L->x_f32.alloc((size_t)nexpect * s->nb)) == cudaSuccess)
-          LAUNCH(ctx, k_f64_to_f32, cdiv((size_t)nexpect * L->ldf, 256), 256, 0, (const double *)L->dinv_dense.p,
-                 L->dinv_f32.p, (size_t)nexpect, (size_t)nexpect, (size_t)L->ldf);
+        DNSB_CK(ctx, L->dinv_f32.alloc((size_t)nexpect * L->ldf));
+        DNSB_CK(ctx, L->x_f32.alloc((size_t)nexpect * s->nb));
+        LAUNCH(ctx, k_f64_to_f32, cdiv((size_t)nexpect * L->ldf, 256), 256, 0, (const double *)L->dinv_dense.p,
+               L->dinv_f32.p, (size_t)nexpect, (size_t)nexpect, (size_t)L->ldf);
       }
     }
-    if (e == cudaSuccess && g_schur_tc && !g_schur_tf32) {
-      e = tc_setup(ctx, L, nexpect, s->nb);
-      if (e == cudaSuccess && !L->tc.ok) {   // block does not qualify: the fp64 kernels serve it
+    if (g_schur_tc && !g_schur_tf32) {
+      DNSB_CK(ctx, tc_setup(ctx, L.get(), nexpect, s->nb));
+      if (!L->tc.ok) {   // block does not qualify: the fp64 kernels serve it
         DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
         L->dinv_f32.release(); L->xt.release(); L->tcpart.release();
       }
     }
-    if (e != cudaSuccess) { level_free(L); DNSB_CK(ctx, e); }
   } else {
     bool ok = amat && amat->nrows == nexpect && amat->ncols == nexpect && lmax > lmin &&
               lmin > 0 && nsmooth >= 1 && !amat->has2;
     if (ok && (pmat || rmat))
       ok = pmat && rmat && pmat->nrows == nexpect && rmat->ncols == nexpect &&
            rmat->nrows == pmat->ncols;
-    if (!ok) { delete L; DNSB_REQUIRE(ctx, false, "inconsistent multigrid level"); }
+    DNSB_REQUIRE(ctx, ok, "inconsistent multigrid level");
     L->kind = pmat ? MG_MULTI : MG_SMOOTH;
     L->A = amat; L->P = pmat; L->R = rmat;
     L->nsmooth = nsmooth; L->lmin = lmin; L->lmax = lmax;
     std::vector<int> dp;
-    if (find_diagpos(ctx, amat, dp)) { delete L; return -2; }
-    DBuf<int> dpd;
-    e = dpd.upload(dp.data(), dp.size(), ctx->stream);
-    if (e != cudaSuccess) { level_free(L); DNSB_CK(ctx, e); }
-    const size_t nn = (size_t)nexpect * s->nb;
-    if ((e = L->dinv_own.alloc(nn)) != cudaSuccess) { level_free(L); dpd.release(); DNSB_CK(ctx, e); }
-    LAUNCH(ctx, k_diag_inv, cdiv(nn, 256), 256, 0, amat->view(), dpd.p,
-           (const double *)nullptr, L->dinv_own.p, s->nb);
-    cudaStreamSynchronize(ctx->stream);
-    dpd.release();
+    if (find_diagpos(ctx, amat, dp)) return -2;
+    {
+      DBuf<int> dpd;
+      DNSB_CK(ctx, dpd.upload(dp.data(), dp.size(), ctx->stream));
+      const size_t nn = (size_t)nexpect * s->nb;
+      DNSB_CK(ctx, L->dinv_own.alloc(nn));
+      LAUNCH(ctx, k_diag_inv, cdiv(nn, 256), 256, 0, amat->view(), dpd.p,
+             (const double *)nullptr, L->dinv_own.p, s->nb);
+      cudaStreamSynchronize(ctx->stream);
+    }
     L->dinv = L->dinv_own.p;
   }
   const size_t nn = (size_t)L->n * s->nb;
-  if ((e = L->b.alloc(nn)) != cudaSuccess || (e = L->x.alloc(nn)) != cudaSuccess ||
-      (e = L->r.alloc(nn)) != cudaSuccess || (e = L->d0.alloc(nn)) != cudaSuccess ||
-      (e = L->d1.alloc(nn)) != cudaSuccess || (e = L->t.alloc(nn)) != cudaSuccess) {
-    level_free(L);
-    DNSB_CK(ctx, e);
-  }
-  lv.push_back(L);
+  DNSB_CK(ctx, L->b.alloc(nn)); DNSB_CK(ctx, L->x.alloc(nn)); DNSB_CK(ctx, L->r.alloc(nn));
+  DNSB_CK(ctx, L->d0.alloc(nn)); DNSB_CK(ctx, L->d1.alloc(nn)); DNSB_CK(ctx, L->t.alloc(nn));
+  lv.push_back(std::move(L));
   return 0;
 }
 
@@ -1729,10 +1669,10 @@ __global__ void k_rowscale_mul(const double *a, const double *rowscale, double *
 
 // x = Vcycle(b) on level l of hierarchy `lv` (b, x: n_l*nb device vectors,
 // b is not modified)
-static void mg_vcycle(dnsb_solver *s, std::vector<MgLevel *> &lv, size_t l,
+static void mg_vcycle(dnsb_solver *s, const std::vector<std::unique_ptr<MgLevel>> &lv, size_t l,
                       const double *b, double *x) {
   dnsb_ctx *ctx = s->ctx;
-  MgLevel *L = lv[l];
+  MgLevel *L = lv[l].get();
   const int nb = s->nb;
   if (L->kind == MG_DENSE) {
     dense_apply(s, L, b, x, 1.0, false);
@@ -1743,7 +1683,7 @@ static void mg_vcycle(dnsb_solver *s, std::vector<MgLevel *> &lv, size_t l,
     return;
   }
   const size_t nn = (size_t)L->n * nb;
-  MgLevel *C = lv[l + 1];
+  MgLevel *C = lv[l + 1].get();
   // pre-smoothing from a zero guess
   cheb_run(s, L->A, L->coef, L->dinv, nullptr, nullptr, b, x, L->r.p, L->d0.p, L->d1.p, L->nsmooth, L->lmin, L->lmax);
   // residual and restriction
@@ -1763,7 +1703,7 @@ static void mg_vcycle(dnsb_solver *s, std::vector<MgLevel *> &lv, size_t l,
 static void schur_levels_apply(dnsb_solver *s, const double *b, double *x, double alpha) {
   dnsb_ctx *ctx = s->ctx;
   const size_t npb = (size_t)s->np * s->nb;
-  MgLevel *L0 = s->levels[0];
+  MgLevel *L0 = s->levels[0].get();
   if (L0->kind == MG_DENSE) {
     dense_apply(s, L0, b, x, alpha, false);
   } else {
@@ -1789,7 +1729,7 @@ static int apply_prec(dnsb_solver *s, const double *r, double *z) {
                  "block-diagonal preconditioner: Chebyshev velocity block + dense Schur block only");
     DNSB_CK(ctx, s->zero_p.alloc(npb));
     DNSB_CK(ctx, s->zero_p.zero(ctx->stream));
-    dense_apply(s, s->levels[0], rp, zp, 1.0, s->has_mass);
+    dense_apply(s, s->levels[0].get(), rp, zp, 1.0, s->has_mass);
     cheb_run(s, s->F, s->has_coef ? s->coef.p : nullptr, s->dinv.p, s->JT, s->zero_p.p, rv, zv, s->cres.p,
              s->cd0.p, s->cd1.p, s->kF, s->lmin, s->lmax);
     return 0;
@@ -1811,7 +1751,7 @@ static int apply_prec(dnsb_solver *s, const double *r, double *z) {
     LAUNCH(ctx, k_scale_member, cdiv(npb, 256), 256, 0, rp, s->mp_scale.p, zp, (size_t)np, nb);
     LAUNCH(ctx, k_rowscale_mul, cdiv(npb, 256), 256, 0, zp, s->mp_dinv.p, zp, np, nb, -1.0);
   } else {
-    MgLevel *L0 = s->levels[0];
+    MgLevel *L0 = s->levels[0].get();
     if (L0->kind == MG_DENSE) {
       dense_apply(s, L0, rp, zp, -1.0, s->has_mass);
     } else {
@@ -1827,7 +1767,7 @@ static int apply_prec(dnsb_solver *s, const double *r, double *z) {
     }
   }
   // ---- zv = Fh^-1 (rv - JT zp) ---------------------------------------------
-  MgLevel *V0 = s->vlevels[0];
+  MgLevel *V0 = s->vlevels[0].get();
   if (V0->kind != MG_SMOOTH) {
     spmm_dev(ctx, s->JT, nullptr, zp, rv, V0->b.p, nb, -1.0, 1.0);
     mg_vcycle(s, s->vlevels, 0, V0->b.p, zv);
@@ -1853,7 +1793,7 @@ static int gmres_iteration_launch(dnsb_solver *s, int j, double tol) {
   double *Vj = s->Vb.p + (size_t)j * ntb;
   double *Zj = s->Zb.p + (size_t)j * ntb;
   if (apply_prec(s, Vj, Zj)) return -1;
-  spmm_dev(ctx, s->K, coef, Zj, nullptr, s->w.p, nb, 1.0, 0.0);
+  spmm_dev(ctx, s->K.get(), coef, Zj, nullptr, s->w.p, nb, 1.0, 0.0);
   // classical Gram-Schmidt; a second pass (CGS2) for long recurrences,
   // where one pass loses the orthogonality of the basis and FGMRES stalls
   // (the Oseen/Newton systems of the steady solver need 150-300 iterations)
@@ -1937,7 +1877,7 @@ static int gmres_iteration(dnsb_solver *s, int j, double tol) {
 
 static int read_flags(dnsb_solver *s) {
   dnsb_ctx *ctx = s->ctx;
-  DNSB_CK(ctx, cudaMemcpyAsync(s->h_flags, s->gs.flags, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  DNSB_CK(ctx, cudaMemcpyAsync(s->h_flags.p, s->gs.flags, 2 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   return 0;
 }
@@ -1964,7 +1904,7 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
     if (zero_guess && first)
       DNSB_CK(ctx, cudaMemcpyAsync(V0, b, ntb * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     else
-      spmm_dev(ctx, s->K, coef, x, b, V0, nb, -1.0, 1.0);
+      spmm_dev(ctx, s->K.get(), coef, x, b, V0, nb, -1.0, 1.0);
     LAUNCH(ctx, k_dot1, rc.nblocks, rc.threads, rc.smem, V0, V0, ntot, nb, rc.rpb, s->partial2.p);
     LAUNCH(ctx, k_reduce_partials2, cdiv(nb, 32), 1024, 0, (const double *)s->partial2.p, rc.nblocks, nb, s->red.p);
     LAUNCH(ctx, k_gmres_begin, 1, std::max(32, ((nb + 31) / 32) * 32), 0, s->gs, (const double *)s->red.p,
@@ -1972,7 +1912,7 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
     LAUNCH(ctx, k_scale_member, cdiv(ntb, 256), 256, 0, V0, s->gs.invh, V0, (size_t)ntot, nb);
     first = false;
     if (read_flags(s)) return -1;
-    if (s->h_flags[0] == 0) break;
+    if (s->h_flags.p[0] == 0) break;
     int j = 0;
     bool alldone = false;
     for (; j < mr && total < maxit; ++j, ++total) {
@@ -1980,7 +1920,7 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
       // convergence poll: skipped while far from the expected iteration count
       if (total + 1 >= expect - 1 || j + 1 == mr || total + 1 == maxit) {
         if (read_flags(s)) return -1;
-        if (s->h_flags[0] == 0) { alldone = true; ++j; ++total; break; }
+        if (s->h_flags.p[0] == 0) { alldone = true; ++j; ++total; break; }
       }
     }
     const int ncols = j;
@@ -1991,7 +1931,7 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
     }
     if (alldone || total >= maxit) break;
   }
-  if (s->h_flags[0] != 0) {
+  if (s->h_flags.p[0] != 0) {
     // stopped at maxit: the residual of the unfinished members enters the
     // running maximum, the solve is counted (callers decide what to do)
     LAUNCH(ctx, k_gmres_track_unconverged, 1, std::max(32, ((nb + 31) / 32) * 32), 0, s->gs, nb);
@@ -1999,7 +1939,7 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
   }
   // h_flags[1]: iteration at which the last member converged (<= total; the
   // difference are iterations launched between two convergence polls)
-  const int needed = std::min(total, std::max(0, s->h_flags[1]));
+  const int needed = std::min(total, std::max(0, s->h_flags.p[1]));
   s->expect_its = needed;
   s->stat_iters += needed;
   s->stat_launched += total;
@@ -2169,7 +2109,7 @@ struct dnsb_cnsweep {
   unsigned long long mesh_hash = 0;
   dnsb_solver *s = nullptr;
   dnsb_csr *M = nullptr;      // mass matrix (own pattern)
-  dnsb_csr *C = nullptr;      // owned: (A + N_c) on the pattern of F
+  std::unique_ptr<dnsb_csr> C;   // (A + N_c) on the pattern of F
   int nv = 0, np = 0, nvf = 0, nconv = 0, nbc = 0;
   DBuf<double> mv, av, nvn, nvc;          // value arrays on the pattern of F
   DBuf<int> src, pos, inv, bcinds;
@@ -2180,6 +2120,7 @@ struct dnsb_cnsweep {
   double max_relres = 0;      // of the last sweep (all step solves)
   long long unconverged = 0;
   int guess_mode = 1;         // 0: previous solution ('old'), 1: linear extrapolation ('upd')
+  ~dnsb_cnsweep() { cudaStreamSynchronize(ctx->stream); }   // no buffer is freed under a running kernel
 };
 
 extern "C" int dnsb_cnsweep_create(dnsb_solver *s, dnsb_csr *mmat, const double *mvals,
@@ -2187,6 +2128,7 @@ extern "C" int dnsb_cnsweep_create(dnsb_solver *s, dnsb_csr *mmat, const double 
                                    const int32_t *pos, const int32_t *invinds, int nbc,
                                    const int32_t *bcinds, const double *bcvals, const double *fv,
                                    const double *fp, dnsb_cnsweep **out) {
+  if (out) *out = nullptr;
   if (!s) return -2;
   dnsb_ctx *ctx = s->ctx;
   DNSB_REQUIRE(ctx, out && mmat && mvals && avals && src && pos && invinds && fv, "null arguments");
@@ -2200,13 +2142,12 @@ extern "C" int dnsb_cnsweep_create(dnsb_solver *s, dnsb_csr *mmat, const double 
   for (int i = 0; i < nv; ++i) DNSB_REQUIRE(ctx, invinds[i] >= 0 && invinds[i] < nvf, "invinds out of range");
   for (int i = 0; i < nbc; ++i) DNSB_REQUIRE(ctx, bcinds[i] >= 0 && bcinds[i] < nvf, "bcinds out of range");
   DNSB_CK(ctx, dnsb_enter(ctx));
-  dnsb_cnsweep *w = new (std::nothrow) dnsb_cnsweep();
+  std::unique_ptr<dnsb_cnsweep> w(new (std::nothrow) dnsb_cnsweep());
   DNSB_REQUIRE(ctx, w != nullptr, "out of host memory");
-  *out = w;
   w->ctx = ctx; w->mesh_hash = ctx->mesh_hash; w->s = s; w->M = mmat;
   w->nv = nv; w->np = np; w->nvf = nvf; w->nconv = nconv; w->nbc = nbc;
   {
-    int rc = csr_build(ctx, nv, nv, s->F->h_indptr.data(), s->F->h_indices.data(), avals, nullptr, &w->C);
+    int rc = csr_build(ctx, nv, nv, s->F->h_indptr.data(), s->F->h_indices.data(), avals, nullptr, w->C);
     if (rc) return rc;
   }
   DNSB_CK(ctx, w->mv.upload(mvals, nnz, ctx->stream));
@@ -2235,22 +2176,13 @@ extern "C" int dnsb_cnsweep_create(dnsb_solver *s, dnsb_csr *mmat, const double 
   RedCfg rc = red_cfg(ctx, nv, 1);
   DNSB_CK(ctx, w->npart.alloc(rc.nblocks)); DNSB_CK(ctx, w->nout.alloc(1));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  *out = w.release();
   return 0;
 }
 
 extern "C" void dnsb_cnsweep_destroy(dnsb_cnsweep *w) {
   if (!w) return;
   dnsb_enter(w->ctx);
-  cudaStreamSynchronize(w->ctx->stream);
-  csr_free(w->C);
-  w->mv.release(); w->av.release(); w->nvn.release(); w->nvc.release();
-  w->src.release(); w->pos.release(); w->inv.release(); w->bcinds.release();
-  w->bcvals.release(); w->ubc.release(); w->fv.release(); w->fp.release();
-  w->n1.release(); w->n2.release(); w->f3.release();
-  w->vfull.release(); w->fn.release(); w->fc.release(); w->b.release(); w->x.release();
-  w->xprev.release(); w->xguess.release();
-  w->y.release(); w->dvec.release(); w->mdv.release(); w->lin.release(); w->vtraj.release();
-  w->ptraj.release(); w->v.release(); w->p.release(); w->npart.release(); w->nout.release();
   delete w;
 }
 
@@ -2329,7 +2261,7 @@ extern "C" int dnsb_cnsweep_run(dnsb_cnsweep *w, int nsteps, const double *dts, 
     // rhs = M v + dt/2 (f_n + f_c - (A + N_c) v)
     LAUNCH(ctx, k_axpby, cdiv((size_t)nnz, 256), 256, 0, 1.0, (const double *)w->av.p, 1.0,
            (const double *)w->nvc.p, w->C->v1.p, (size_t)nnz);
-    spmm_dev(ctx, w->C, nullptr, w->v.p, nullptr, w->y.p, 1, 1.0, 0.0);
+    spmm_dev(ctx, w->C.get(), nullptr, w->v.p, nullptr, w->y.p, 1, 1.0, 0.0);
     spmm_dev(ctx, w->M, nullptr, w->v.p, nullptr, w->b.p, 1, 1.0, 0.0);
     LAUNCH(ctx, k_cn_rhs, cdiv(nv, 256), 256, 0, w->b.p, (const double *)w->fn.p, (const double *)w->fc.p,
            (const double *)w->y.p, 0.5 * dt, nv);
@@ -2433,7 +2365,7 @@ extern "C" int dnsb_solver_apply_k(dnsb_solver *s, const double *x, double *y) {
   DNSB_CK(ctx, s->sb.alloc(ntb));
   DNSB_CK(ctx, s->sx.alloc(ntb));
   DNSB_CK(ctx, cudaMemcpyAsync(s->sb.p, x, ntb * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
-  spmm_dev(ctx, s->K, s->has_coef ? s->coef.p : nullptr, s->sb.p, nullptr, s->sx.p, s->nb, 1.0, 0.0);
+  spmm_dev(ctx, s->K.get(), s->has_coef ? s->coef.p : nullptr, s->sb.p, nullptr, s->sx.p, s->nb, 1.0, 0.0);
   DNSB_CK(ctx, cudaMemcpyAsync(y, s->sx.p, ntb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   DNSB_CK(ctx, cudaGetLastError());
@@ -2449,7 +2381,7 @@ struct dnsb_imex {
   int scheme = 0, nb = 1, nv = 0, np = 0, nvf = 0, nbc = 0;
   double dt = 0;
   dnsb_csr *M = nullptr, *A = nullptr, *J = nullptr, *JT = nullptr;
-  dnsb_csr *Rm = nullptr;   // owned: CNAB rhs operator  M - dt/2*A_m
+  std::unique_ptr<dnsb_csr> Rm;   // CNAB rhs operator  M - dt/2*A_m
   dnsb_solver *sl = nullptr, *sp = nullptr, *sc = nullptr;
   DBuf<double> nu, coefR, coefA;   // nb
   DBuf<int> inv, bcinds;
@@ -2485,7 +2417,7 @@ struct dnsb_imex {
   cudaEvent_t ev_free[NSTAGE] = {nullptr, nullptr, nullptr, nullptr};
   bool stage_busy[NSTAGE] = {false, false, false, false};
   cudaStream_t cstream = nullptr;
-  double *h_snaps = nullptr;   // pinned, h_cap snapshots
+  PinnedBuf<double> h_snaps;   // h_cap snapshots
   int h_cap = 0;
   bool host_mirror = true;
   long long step = 0;   // steps done so far
@@ -2505,6 +2437,16 @@ struct dnsb_imex {
   int nlev = 0, lev_cap = 0;
   long long csave_level = -1;   // time level n whose Phi^T c(V_n) is in o_csave (-1: none)
   bool outputs_on() const { return ny > 0 || !fdofs.empty(); }
+  ~dnsb_imex() {
+    cudaStreamSynchronize(ctx->stream);   // no buffer is freed under a running kernel or copy
+    if (cstream) { cudaStreamSynchronize(cstream); cudaStreamDestroy(cstream); }
+    for (int q = 0; q < NSTAGE; ++q) {
+      if (ev_ready[q]) cudaEventDestroy(ev_ready[q]);
+      if (ev_free[q]) cudaEventDestroy(ev_free[q]);
+    }
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+  }
 };
 
 extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
@@ -2513,6 +2455,7 @@ extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
                                 const int32_t *invinds, int nv, int nbc,
                                 const int32_t *bcinds, const double *bcvals,
                                 const double *fv, const double *fp, dnsb_imex **out) {
+  if (out) *out = nullptr;
   if (!ctx) return -2;
   DNSB_REQUIRE(ctx, out && mmat && amat && jmat && jtmat && nu && invinds, "null arguments");
   DNSB_REQUIRE(ctx, scheme >= 0 && scheme <= 2, "scheme must be 0 (CNAB), 1 (SBDF2) or 2 (IMEX Euler)");
@@ -2529,9 +2472,8 @@ extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
   for (int i = 0; i < nbc; ++i)
     DNSB_REQUIRE(ctx, bcinds[i] >= 0 && bcinds[i] < nvf, "bcinds out of range");
   DNSB_CK(ctx, dnsb_enter(ctx));
-  dnsb_imex *e = new (std::nothrow) dnsb_imex();
+  std::unique_ptr<dnsb_imex> e(new (std::nothrow) dnsb_imex());
   DNSB_REQUIRE(ctx, e != nullptr, "out of host memory");
-  *out = e;
   e->ctx = ctx; e->scheme = scheme; e->nb = nb; e->dt = dt;
   e->mesh_hash = ctx->mesh_hash;
   e->nv = nv; e->np = jmat->nrows; e->nvf = nvf; e->nbc = nbc;
@@ -2553,10 +2495,10 @@ extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
     std::vector<double> r1(mmat->nnz);
     for (int k = 0; k < mmat->nnz; ++k) r1[k] = mmat->h_v1[k] - 0.5 * dt * amat->h_v1[k];
     int rc = csr_build(ctx, nv, nv, mmat->h_indptr.data(), mmat->h_indices.data(), r1.data(),
-                       amat->h_v2.data(), &e->Rm);
+                       amat->h_v2.data(), e->Rm);
     if (rc) return rc;
     // the right-hand side product R v of every step through the staged tile kernel as well (bit-identical)
-    if (nb == TILE_NB) { rc = tile_setup(ctx, e->Rm); if (rc) return rc; }
+    if (nb == TILE_NB) { rc = tile_setup(ctx, e->Rm.get()); if (rc) return rc; }
   }
   const size_t nvb = (size_t)nv * nb, npb = (size_t)e->np * nb, nfb = (size_t)nvf * nb;
   DNSB_CK(ctx, e->v.alloc(nvb)); DNSB_CK(ctx, e->vprev.alloc(nvb));
@@ -2573,37 +2515,13 @@ extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
            e->vfull.p, nbc, nb);
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   DNSB_CK(ctx, cudaGetLastError());
+  *out = e.release();
   return 0;
 }
 
 extern "C" void dnsb_imex_destroy(dnsb_imex *e) {
   if (!e) return;
   dnsb_enter(e->ctx);
-  cudaStreamSynchronize(e->ctx->stream);
-  csr_free(e->Rm);
-  if (e->cstream) { cudaStreamSynchronize(e->cstream); cudaStreamDestroy(e->cstream); }
-  for (int q = 0; q < dnsb_imex::NSTAGE; ++q) {
-    e->stage[q].release();
-    if (e->ev_ready[q]) cudaEventDestroy(e->ev_ready[q]);
-    if (e->ev_free[q]) cudaEventDestroy(e->ev_free[q]);
-  }
-  if (e->h_snaps) cudaFreeHost(e->h_snaps);
-  e->outmap.release();
-  if (e->ev0) cudaEventDestroy(e->ev0);
-  if (e->ev1) cudaEventDestroy(e->ev1);
-  e->nu.release(); e->coefR.release(); e->coefA.release(); e->inv.release();
-  e->bcinds.release(); e->bcvals.release(); e->fv.release(); e->fp.release();
-  e->Bk.release(); e->useries.release();
-  e->v.release(); e->vprev.release(); e->p.release(); e->vfull.release(); e->cfull.release();
-  e->nfc_c.release(); e->nfc_o.release(); e->nfc_t.release(); e->tmp.release();
-  e->b.release(); e->x.release(); e->xh.release(); e->bq.release(); e->xq.release(); e->x0.release();
-  e->pw0.release(); e->pw1.release(); e->pd0.release(); e->pd1.release(); e->pinv.release();
-  e->gr.release(); e->partialh.release(); e->snaps.release();
-  e->ptri.release(); e->py.release(); e->pgsum.release();
-  e->normpart.release(); e->normout.release();
-  e->o_vptr.release(); e->o_vidx.release(); e->o_pptr.release(); e->o_pidx.release();
-  e->o_fptr.release(); e->o_fdofs.release(); e->o_w1.release(); e->o_w2.release(); e->o_wp.release();
-  e->o_fbc.release(); e->o_csave.release(); e->o_rec.release();
   delete e;
 }
 
@@ -2702,14 +2620,13 @@ static int imex_reserve_host(dnsb_imex *e, int cap) {
   dnsb_ctx *ctx = e->ctx;
   if (cap <= e->h_cap) return 0;
   const size_t ntb = (size_t)(e->nv + e->np) * e->nb;
-  double *nh = nullptr;
-  DNSB_CK(ctx, cudaMallocHost((void **)&nh, (size_t)cap * ntb * sizeof(double)));
-  if (e->h_snaps) {
+  PinnedBuf<double> nh;
+  DNSB_CK(ctx, nh.alloc((size_t)cap * ntb));
+  if (e->h_snaps.p) {
     if (e->cstream) DNSB_CK(ctx, cudaStreamSynchronize(e->cstream));
-    memcpy(nh, e->h_snaps, (size_t)std::min(e->nsnap, e->h_cap) * ntb * sizeof(double));
-    cudaFreeHost(e->h_snaps);
+    memcpy(nh.p, e->h_snaps.p, (size_t)std::min(e->nsnap, e->h_cap) * ntb * sizeof(double));
   }
-  e->h_snaps = nh;
+  e->h_snaps = std::move(nh);
   e->h_cap = cap;
   return 0;
 }
@@ -2737,7 +2654,7 @@ static int imex_snapshot(dnsb_imex *e) {
            dst + nvb);
     DNSB_CK(ctx, cudaEventRecord(e->ev_ready[q], ctx->stream));
     DNSB_CK(ctx, cudaStreamWaitEvent(e->cstream, e->ev_ready[q], 0));
-    DNSB_CK(ctx, cudaMemcpyAsync(e->h_snaps + (size_t)e->nsnap * ntb, e->stage[q].p, ntb * sizeof(double),
+    DNSB_CK(ctx, cudaMemcpyAsync(e->h_snaps.p + (size_t)e->nsnap * ntb, e->stage[q].p, ntb * sizeof(double),
                                  cudaMemcpyDeviceToHost, e->cstream));
     DNSB_CK(ctx, cudaEventRecord(e->ev_free[q], e->cstream));
     e->stage_busy[q] = true;
@@ -2972,7 +2889,7 @@ static int proj_add(dnsb_imex *e, double *d, int npass) {
   const double *coef = sl->has_coef ? sl->coef.p : nullptr;
   RedCfg rc = red_cfg(ctx, ntot, nb);
   double *w = e->pw0.p, *w2 = e->pw1.p, *d2 = e->pd1.p;
-  spmm_dev(ctx, sl->K, coef, d, nullptr, w, nb, 1.0, 0.0);
+  spmm_dev(ctx, sl->K.get(), coef, d, nullptr, w, nb, 1.0, 0.0);
   const int k = e->pcnt;
   // |K d|^2 before the orthogonalisation (reference for the breakdown test)
   for (int pass = 0; pass < npass && k > 0; ++pass) {
@@ -3144,8 +3061,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
         DNSB_CK(ctx, cudaMemcpyAsync(ns.p, e->snaps.p, (size_t)e->nsnap * ntb * sizeof(double),
                                      cudaMemcpyDeviceToDevice, ctx->stream));
       DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
-      e->snaps.release();
-      e->snaps = ns;
+      e->snaps = std::move(ns);
       e->snap_cap = need;
     }
     if (e->host_mirror) {
@@ -3173,8 +3089,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
         DNSB_CK(ctx, cudaMemcpyAsync(nr.p, e->o_rec.p, (size_t)e->nlev * per * sizeof(double),
                                      cudaMemcpyDeviceToDevice, ctx->stream));
       DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
-      e->o_rec.release();
-      e->o_rec = nr;
+      e->o_rec = std::move(nr);
       e->lev_cap = need;
     }
     if (e->nlev == 0) {
@@ -3263,7 +3178,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
       std::swap(e->nfc_o.p, e->nfc_c.p);
       rc = imex_nonl(e, e->v.p, e->nfc_c.p);
       if (rc) return rc;
-      spmm_dev(ctx, e->Rm, e->coefR.p, e->v.p, nullptr, e->b.p, nb, 1.0, 0.0);
+      spmm_dev(ctx, e->Rm.get(), e->coefR.p, e->v.p, nullptr, e->b.p, nb, 1.0, 0.0);
       LAUNCH(ctx, k_rhs_combine, cdiv(nvb, 256), 256, 0, e->b.p, (const double *)e->nfc_c.p, 1.5 * dt,
              (const double *)e->nfc_o.p, -0.5 * dt, (const double *)e->fv.p, dt,
              (const double *)e->Bk.p, e->nk, uc, 0.5 * dt, un, 0.5 * dt, nv, nb);
@@ -3393,9 +3308,9 @@ extern "C" int dnsb_imex_get_snapshots(dnsb_imex *e, double *out) {
   DNSB_CK(ctx, dnsb_enter(ctx));
   const size_t ntb = (size_t)(e->nv + e->np) * e->nb;
   if (e->nsnap == 0) return 0;
-  if (e->host_mirror && e->h_snaps && e->nsnap <= e->h_cap) {
+  if (e->host_mirror && e->h_snaps.p && e->nsnap <= e->h_cap) {
     DNSB_CK(ctx, cudaStreamSynchronize(e->cstream));
-    memcpy(out, e->h_snaps, (size_t)e->nsnap * ntb * sizeof(double));
+    memcpy(out, e->h_snaps.p, (size_t)e->nsnap * ntb * sizeof(double));
     return 0;
   }
   DNSB_REQUIRE(ctx, !e->has_outmap, "host mirror disabled: no output order available");
@@ -3411,7 +3326,7 @@ extern "C" int dnsb_imex_snapshots_host(dnsb_imex *e, const double **ptr, int *n
   DNSB_REQUIRE(ctx, ptr && nsnap, "null output");
   DNSB_REQUIRE(ctx, e->host_mirror, "host mirror disabled");
   if (e->cstream) DNSB_CK(ctx, cudaStreamSynchronize(e->cstream));
-  *ptr = e->h_snaps;
+  *ptr = e->h_snaps.p;
   *nsnap = std::min(e->nsnap, e->h_cap);
   return 0;
 }
@@ -3623,15 +3538,10 @@ extern "C" int dnsb_imex_gram(dnsb_imex *e, double *g) {
   DBuf<double> gd;
   DNSB_CK(ctx, gd.alloc((size_t)e->nsnap * e->nsnap));
   int rc = imex_gram_impl(e, gd.p);
-  if (!rc) {
-    cudaError_t ce = cudaMemcpyAsync(g, gd.p, gd.n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-    gd.release();
-    DNSB_CK(ctx, ce);
-    return 0;
-  }
-  gd.release();
-  return rc;
+  if (rc) return rc;
+  DNSB_CK(ctx, cudaMemcpyAsync(g, gd.p, gd.n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
 }
 
 extern "C" int dnsb_imex_gram_dev(dnsb_imex *e, double *g_dev) { return imex_gram_impl(e, g_dev); }
@@ -3652,7 +3562,6 @@ static int imex_gram_impl(dnsb_imex *e, double *g_dev) {
   LAUNCH(ctx, k_gram_partial, dim3(nchunks, ns * ns), 256, 256 * sizeof(double), e->snaps.p, ntb, MX.p, ns, nvb, part.p);
   LAUNCH(ctx, k_reduce_partials2, cdiv((size_t)ns * ns, 32), 1024, 0, (const double *)part.p, nchunks, ns * ns, g_dev);
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
-  MX.release(); part.release();
   DNSB_CK(ctx, cudaGetLastError());
   return 0;
 }

@@ -6,6 +6,7 @@
 #define DNSB_L2_HINTS 2
 #endif
 #include <cuda_runtime.h>
+#include <atomic>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -59,20 +60,36 @@ __device__ __forceinline__ void dnsb_pdl_entry() {
     }                                                                         \
   } while (0)
 
-// plain device buffer; freed explicitly (no exceptions across the ABI)
-template <class T>
-struct DBuf {
+// bytes held by live device [0] / pinned host [1] buffers of the whole process (dnsb_live_bytes)
+static std::atomic<long long> g_live_bytes[2];
+
+// Buffer of n T's in device memory (DBuf) or pinned host memory (PinnedBuf), owned by the object that
+// holds it: the destructor frees it, a move hands it over, there are no copies.  Destructors do not
+// throw, so nothing crosses the ABI as an exception.
+template <class T, bool Pinned>
+struct OwnedBuf {
   T *p = nullptr;
   size_t n = 0;
+  OwnedBuf() = default;
+  OwnedBuf(const OwnedBuf &) = delete;
+  OwnedBuf &operator=(const OwnedBuf &) = delete;
+  OwnedBuf(OwnedBuf &&o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+  OwnedBuf &operator=(OwnedBuf &&o) noexcept {
+    if (this != &o) { release(); p = o.p; n = o.n; o.p = nullptr; o.n = 0; }
+    return *this;
+  }
+  ~OwnedBuf() { release(); }
   cudaError_t alloc(size_t count) {
     if (p && n == count) return cudaSuccess;   // reuse
     release();
     n = count;
     if (count == 0) return cudaSuccess;
-    cudaError_t e = cudaMalloc((void **)&p, count * sizeof(T));
+    cudaError_t e = Pinned ? cudaMallocHost((void **)&p, count * sizeof(T)) : cudaMalloc((void **)&p, count * sizeof(T));
     if (e != cudaSuccess) { p = nullptr; n = 0; }
+    else g_live_bytes[Pinned] += (long long)(count * sizeof(T));
     return e;
   }
+  // upload / zero: device buffers
   cudaError_t upload(const T *h, size_t count, cudaStream_t s) {
     cudaError_t e = alloc(count);
     if (e != cudaSuccess || count == 0) return e;
@@ -85,11 +102,16 @@ struct DBuf {
     return cudaMemsetAsync(p, 0, n * sizeof(T), s);
   }
   void release() {
-    if (p) cudaFree(p);
+    if (p) {
+      if (Pinned) cudaFreeHost(p); else cudaFree(p);
+      g_live_bytes[Pinned] -= (long long)(n * sizeof(T));
+    }
     p = nullptr;
     n = 0;
   }
 };
+template <class T> using DBuf = OwnedBuf<T, false>;
+template <class T> using PinnedBuf = OwnedBuf<T, true>;
 
 struct ProfRec {
   const char *name;
@@ -135,6 +157,15 @@ struct dnsb_ctx {
     char buf[64];
     snprintf(buf, sizeof buf, " (%s:%d)", file, line);
     err = what + buf;
+  }
+  void drop_recs() {
+    for (ProfRec &r : recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
+    recs.clear();
+  }
+  ~dnsb_ctx() {   // the caller has made the device current (dnsb_enter)
+    if (stream) cudaStreamSynchronize(stream);   // no buffer is freed under a running kernel
+    drop_recs();
+    if (stream) cudaStreamDestroy(stream);
   }
 };
 

@@ -16,6 +16,14 @@
  * reference's sparse-LU solve cannot fail this way).  Nothing throws across
  * the ABI.  One context = one device + one stream; a context is
  * not thread-safe.
+ *
+ * Handles: a dnsb_*_create sets *out only on success; on failure *out is NULL
+ * and nothing it allocated stays allocated.  The exception is
+ * dnsb_ctx_create, which returns its context on failure as well so that the
+ * message can be read with dnsb_last_error; the caller then destroys it.
+ * dnsb_*_destroy waits for the work queued on the handle's streams, then
+ * frees everything the handle owns (matrices and solvers passed in are
+ * borrowed and stay the caller's).
  */
 #ifndef DNSB_H
 #define DNSB_H
@@ -54,6 +62,11 @@ void dnsb_launch_count_reset(dnsb_ctx *ctx);
  * read), so that their average algorithmic bytes can be computed. */
 int dnsb_profile_begin(dnsb_ctx *ctx, int max_records);
 int dnsb_profile_end(dnsb_ctx *ctx, char *buf, int buflen);
+/* bytes of device memory and of pinned host memory held by the library in
+ * this process, over all contexts (either pointer may be NULL): a leak shows
+ * here exactly, unlike in the device's free memory, which other processes
+ * share */
+void dnsb_live_bytes(long long *device, long long *pinned);
 
 /* ---- mesh + convection assembly (K1a / K1b) ------------------------------
  * dnsb_set_mesh: P2 scalar cell dofmap (ncell*6, local order 3 vertices then

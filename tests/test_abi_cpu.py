@@ -236,6 +236,7 @@ def test_device_path_fails_loudly_without_a_gpu():
     from dolfin_navier_scipy_b200 import fem
     with pytest.raises(_lib.DnsbError):
         _lib.Context(0)
+    assert _lib.live_bytes() == (0, 0)     # the failed context was destroyed
     V = fem.VectorP2Space(fem.unit_square_mesh(2))
     with pytest.raises(RuntimeError):
         dts.get_convvec(V=V, u0_vec=np.zeros(V.dim()))
