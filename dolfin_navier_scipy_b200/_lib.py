@@ -76,6 +76,8 @@ SIGNATURES = {
     'dnsb_imex_set_state': (_i, [_vp, c_dbl_p, c_dbl_p]),
     'dnsb_imex_run': (_i, [_vp, _i, _i, _d, _i, _i, _d, _i,
                            ctypes.POINTER(_i)]),
+    'dnsb_imex_set_member_guard': (_i, [_vp, _i]),
+    'dnsb_imex_member_status': (_i, [_vp, c_int_p]),
     'dnsb_imex_last_run_ms': (_d, [_vp]),
     'dnsb_imex_get_state': (_i, [_vp, c_dbl_p, c_dbl_p]),
     'dnsb_imex_num_snapshots': (_i, [_vp]),
@@ -587,6 +589,17 @@ class ImexEngine(object):
         if not (allow_unconverged and rc == E_NOT_CONVERGED):
             self.ctx.check(rc)
         return ff.value
+
+    def set_member_guard(self, on):
+        """per-member blow-up guard (``dnsb_imex_set_member_guard``)"""
+        self.ctx.check(self.ctx.lib.dnsb_imex_set_member_guard(self.h,
+                                                               int(bool(on))))
+
+    def member_status(self):
+        """trip level of every member, -1 while it is live"""
+        t = np.empty(self.nb, dtype=np.int32)
+        self.ctx.check(self.ctx.lib.dnsb_imex_member_status(self.h, _ip(t)))
+        return t
 
     def last_run_ms(self):
         return float(self.ctx.lib.dnsb_imex_last_run_ms(self.h))

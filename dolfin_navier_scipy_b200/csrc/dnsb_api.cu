@@ -1950,12 +1950,17 @@ static int solver_solve_dev(dnsb_solver *s, const double *b, double *x, double t
 
 // max over members of the running maximum of the final relative residuals
 // since the last reset (NaN if any solve produced one); optionally reset
-static int solver_relmax(dnsb_solver *s, bool reset, double *out) {
+static int solver_relmax_members(dnsb_solver *s, std::vector<double> &h, bool reset = false) {
   dnsb_ctx *ctx = s->ctx;
-  std::vector<double> h(s->nb);
+  h.resize(s->nb);
   DNSB_CK(ctx, cudaMemcpyAsync(h.data(), s->grelmax.p, s->nb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   if (reset) DNSB_CK(ctx, s->grelmax.zero(ctx->stream));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  return 0;
+}
+static int solver_relmax(dnsb_solver *s, bool reset, double *out) {
+  std::vector<double> h;
+  if (solver_relmax_members(s, h, reset)) return -1;
   double mx = 0.0;
   for (int m = 0; m < s->nb; ++m) {
     if (h[m] != h[m]) { mx = h[m]; break; }   // NaN wins
@@ -2436,6 +2441,14 @@ struct dnsb_imex {
   DBuf<double> o_w1, o_w2, o_wp, o_fbc, o_csave, o_rec;
   int nlev = 0, lev_cap = 0;
   long long csave_level = -1;   // time level n whose Phi^T c(V_n) is in o_csave (-1: none)
+  // per-member blow-up guard (dnsb_imex_set_member_guard): trip level of every member (-1: live) on the
+  // host and on the device, and the frozen trip states (v, p lanes) of the retired members.  The device
+  // arrays exist from the first retirement on; nretired == 0 launches nothing of this machinery.
+  bool member_guard = false;
+  std::vector<int> trip;
+  int nretired = 0;
+  DBuf<int> d_trip;
+  DBuf<double> trip_v, trip_p;
   bool outputs_on() const { return ny > 0 || !fdofs.empty(); }
   ~dnsb_imex() {
     cudaStreamSynchronize(ctx->stream);   // no buffer is freed under a running kernel or copy
@@ -2475,6 +2488,7 @@ extern "C" int dnsb_imex_create(dnsb_ctx *ctx, int scheme, int nb, double dt,
   std::unique_ptr<dnsb_imex> e(new (std::nothrow) dnsb_imex());
   DNSB_REQUIRE(ctx, e != nullptr, "out of host memory");
   e->ctx = ctx; e->scheme = scheme; e->nb = nb; e->dt = dt;
+  e->trip.assign(nb, -1);
   e->mesh_hash = ctx->mesh_hash;
   e->nv = nv; e->np = jmat->nrows; e->nvf = nvf; e->nbc = nbc;
   e->M = mmat; e->A = amat; e->J = jmat; e->JT = jtmat;
@@ -2567,6 +2581,7 @@ extern "C" int dnsb_imex_set_state(dnsb_imex *e, const double *v0, const double 
   e->step = 0; e->hist_cnt = 0; e->hist_pos = 0; e->nsnap = 0; e->pcnt = 0;
   e->force_t0 = 0;
   e->nlev = 0; e->csave_level = -1;
+  e->trip.assign(e->nb, -1); e->nretired = 0;   // every member is live again
   e->have_state = true;
   e->p_stale = false;
   return 0;
@@ -2615,6 +2630,48 @@ __global__ void k_scatter_rows(const double *__restrict__ x, const int *__restri
   if (copy) copy[t] = v;
 }
 
+// ---- per-member blow-up guard: the lanes of retired members ----------------
+// trip[m] is the time level at which member m was retired, -1 while it is live.  Members are the fastest
+// index of every vector, so lane m of a vector of n rows is x[i*nb + m].
+// tv / tp lane m = v / p lane m for the members retired at `level`: their frozen trip state
+__global__ void k_retire_take(const double *__restrict__ v, const double *__restrict__ p, double *__restrict__ tv,
+                              double *__restrict__ tp, size_t nvb, size_t npb, int nb, const int *__restrict__ trip,
+                              long long level) {
+  dnsb_pdl_entry();
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= nvb + npb) return;
+  const size_t u = t < nvb ? t : t - nvb;
+  if (trip[u % nb] != level) return;
+  if (t < nvb) tv[u] = v[u]; else tp[u] = p[u];
+}
+// zero the retired lanes of the right-hand side b and the initial guess x (ntb each): such a lane enters
+// FGMRES with b = 0 and x = 0 and is done at iteration 0, whatever its history buffers hold
+__global__ void k_retire_zero(double *__restrict__ b, double *__restrict__ x, size_t ntb, int nb,
+                              const int *__restrict__ trip) {
+  dnsb_pdl_entry();
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= ntb || trip[t % nb] < 0) return;
+  b[t] = 0.0;
+  x[t] = 0.0;
+}
+// NaN in the lanes of the members retired before `level`, in a record of that level (x, and y if not null)
+__global__ void k_retire_nan(double *__restrict__ x, double *__restrict__ y, size_t n, int nb,
+                             const int *__restrict__ trip, long long level) {
+  dnsb_pdl_entry();
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int tl = trip[t % nb];
+  if (tl < 0 || level <= tl) return;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  x[t] = nan;
+  if (y) y[t] = nan;
+}
+static int retire_nan(dnsb_imex *e, double *x, double *y, size_t n, long long level) {
+  if (e->nretired == 0) return 0;
+  LAUNCH(e->ctx, k_retire_nan, cdiv(n, 256), 256, 0, x, y, n, e->nb, (const int *)e->d_trip.p, level);
+  return 0;
+}
+
 // pinned host mirror with room for `cap` snapshots (contents are kept)
 static int imex_reserve_host(dnsb_imex *e, int cap) {
   dnsb_ctx *ctx = e->ctx;
@@ -2643,6 +2700,8 @@ static int imex_snapshot(dnsb_imex *e) {
   if (!mirror) {
     DNSB_CK(ctx, cudaMemcpyAsync(dst, e->v.p, nvb * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     DNSB_CK(ctx, cudaMemcpyAsync(dst + nvb, e->p.p, npb * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+    int rc = retire_nan(e, dst, nullptr, ntb, e->step);
+    if (rc) return rc;
   }
   if (mirror) {   // the un-permuting kernels below fill the device-side store in the same pass
     const int q = e->nsnap % dnsb_imex::NSTAGE;
@@ -2652,6 +2711,8 @@ static int imex_snapshot(dnsb_imex *e) {
     LAUNCH(ctx, k_scatter_rows, cdiv(nvb, 256), 256, 0, (const double *)e->v.p, mv, e->stage[q].p, e->nv, e->nb, dst);
     LAUNCH(ctx, k_scatter_rows, cdiv(npb, 256), 256, 0, (const double *)e->p.p, mp, e->stage[q].p + nvb, e->np, e->nb,
            dst + nvb);
+    int rc = retire_nan(e, dst, e->stage[q].p, ntb, e->step);
+    if (rc) return rc;
     DNSB_CK(ctx, cudaEventRecord(e->ev_ready[q], ctx->stream));
     DNSB_CK(ctx, cudaStreamWaitEvent(e->cstream, e->ev_ready[q], 0));
     DNSB_CK(ctx, cudaMemcpyAsync(e->h_snaps.p + (size_t)e->nsnap * ntb, e->stage[q].p, ntb * sizeof(double),
@@ -2750,7 +2811,7 @@ k_imex_outputs(int ny, int row0, const int *__restrict__ vptr, const int *__rest
 // source holds c(V_{conv_level}), which the force of level conv_level + 1 needs together with the saved
 // term of level conv_level - 1.
 static int imex_outputs(dnsb_imex *e, bool out_level, const double *vn, const double *vp, const double *pn,
-                        double ps, long long conv_level) {
+                        double ps, long long conv_level, long long level) {
   dnsb_ctx *ctx = e->ctx;
   const int nb = e->nb;
   const bool force = !e->fdofs.empty() && conv_level >= 0;
@@ -2767,7 +2828,11 @@ static int imex_outputs(dnsb_imex *e, bool out_level, const double *vn, const do
          (const int *)e->o_fdofs.p, (const int *)ctx->n2c_ptr.p, (const int *)ctx->n2c_idx.p, E, cf, vn, vp, pn, ps,
          1.0 / e->dt, (const double *)e->nu.p, (const double *)e->o_fbc.p, fvalid, e->o_csave.p, out, nb);
   if (force) e->csave_level = conv_level;
-  if (out_level) e->nlev++;
+  if (out_level) {
+    int rc = retire_nan(e, out, nullptr, (size_t)(e->ny + 2) * nb, level);   // `level` is that of the record
+    if (rc) return rc;
+    e->nlev++;
+  }
   return 0;
 }
 
@@ -2986,8 +3051,10 @@ static int imex_push_history(dnsb_imex *e, int guess) {
   return 0;
 }
 
-// |v_m| > maxv or NaN for any member?  (time_int_utils.py:94-103)
-static int imex_blowup(dnsb_imex *e, const double *vc, double maxv, bool *bad) {
+// blow-up guard (time_int_utils.py:94-103) at the current time level: |v_m| > maxv or NaN?  Stop-all mode:
+// *stop if any member fails.  Member mode: the live members that fail are retired (their v / p lanes are
+// frozen into trip_v / trip_p, trip[m] = this level, *retired = true) and *stop only once none is left.
+static int imex_blowup(dnsb_imex *e, const double *vc, double maxv, bool *stop, bool *retired) {
   dnsb_ctx *ctx = e->ctx;
   const int nb = e->nb;
   RedCfg rcn = red_cfg(ctx, e->nv, nb);
@@ -2996,9 +3063,28 @@ static int imex_blowup(dnsb_imex *e, const double *vc, double maxv, bool *bad) {
   std::vector<double> hn(nb);
   DNSB_CK(ctx, cudaMemcpyAsync(hn.data(), e->normout.p, nb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
-  *bad = false;
+  *stop = false;
+  if (!e->member_guard) {
+    for (int m = 0; m < nb; ++m)
+      if (!(std::sqrt(hn[m]) <= maxv)) *stop = true;   // also catches NaN
+    return 0;
+  }
+  int fresh = 0;
   for (int m = 0; m < nb; ++m)
-    if (!(std::sqrt(hn[m]) <= maxv)) *bad = true;   // also catches NaN
+    if (e->trip[m] < 0 && !(std::sqrt(hn[m]) <= maxv)) { e->trip[m] = (int)e->step; ++fresh; }
+  if (fresh == 0) return 0;
+  *retired = true;
+  if (e->nretired == 0) {
+    DNSB_CK(ctx, e->trip_v.alloc((size_t)e->nv * nb));
+    DNSB_CK(ctx, e->trip_p.alloc((size_t)e->np * nb));
+  }
+  e->nretired += fresh;
+  DNSB_CK(ctx, e->d_trip.upload(e->trip.data(), nb, ctx->stream));
+  imex_refresh_p(e);
+  const size_t nvb = (size_t)e->nv * nb, npb = (size_t)e->np * nb;
+  LAUNCH(ctx, k_retire_take, cdiv(nvb + npb, 256), 256, 0, (const double *)e->v.p, (const double *)e->p.p,
+         e->trip_v.p, e->trip_p.p, nvb, npb, nb, (const int *)e->d_trip.p, e->step);
+  *stop = e->nretired == nb;
   return 0;
 }
 
@@ -3094,7 +3180,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     }
     if (e->nlev == 0) {
       imex_refresh_p(e);
-      int rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1);
+      int rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1, e->step);
       if (rc) return rc;
     }
   }
@@ -3114,7 +3200,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     int rc = imex_nonl(e, e->v.p, e->nfc_c.p);                 // nfc(v0)
     if (rc) return rc;
     if (outs && e->scheme == 0) {   // Phi^T c(V_0), before the predictor's convection overwrites it
-      rc = imex_outputs(e, false, nullptr, nullptr, nullptr, 0.0, 0);
+      rc = imex_outputs(e, false, nullptr, nullptr, nullptr, 0.0, 0, 0);
       if (rc) return rc;
     }
     // predictor (IMEX Euler):  (M + dt A) tv = M v + dt f(t1) + dt nfc(v0)
@@ -3149,7 +3235,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     imex_refresh_p(e);
     e->step = 1;
     done = 1;
-    if (outs) { rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1); if (rc) return rc; }
+    if (outs) { rc = imex_outputs(e, true, e->v.p, nullptr, e->p.p, 1.0, -1, 1); if (rc) return rc; }
     if (snap_stride > 0 && e->step % snap_stride == 0) { rc = imex_snapshot(e); if (rc) return rc; }
     // nfc_c holds nfc(v0): it becomes nfc_o in the first loop step
   }
@@ -3158,7 +3244,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
   // remainder slice (time_int_utils.py:94-103, 480-489)
   const int loopsteps = nsteps - done;
   const int lenofts = ntimeslices > 0 ? loopsteps / ntimeslices : 0;
-  bool blown = false;
+  bool blown = false, retired = false;
   for (int it = 0; it < loopsteps; ++it) {
     if (ntimeslices > 0) {
       bool check = false;
@@ -3166,7 +3252,7 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
         if (it == k * lenofts) check = true;
       if (check) {
         bool bad = false;
-        int rcb = imex_blowup(e, e->scheme == 1 ? e->vprev.p : e->v.p, check_ff_maxv, &bad);
+        int rcb = imex_blowup(e, e->scheme == 1 ? e->vprev.p : e->v.p, check_ff_maxv, &bad, &retired);
         if (rcb) return rcb;
         if (bad) { blown = true; break; }
       }
@@ -3211,13 +3297,15 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
       LAUNCH(ctx, k_axpby, cdiv(npb, 256), 256, 0, -dt, (const double *)e->p.p, 0.0,
              (const double *)nullptr, e->x.p + nvb, npb);
     }
+    if (e->nretired > 0)
+      LAUNCH(ctx, k_retire_zero, cdiv(ntb, 256), 256, 0, e->b.p, e->x.p, ntb, nb, (const int *)e->d_trip.p);
     if (guess >= 2 && rc != 2)   // rc == 2: imex_guess wrote x0 itself
       DNSB_CK(ctx, cudaMemcpyAsync(e->x0.p, e->x.p, ntb * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
     rc = solver_solve_dev(e->sl, e->b.p, e->x.p, tol, maxit, false);
     if (rc) return rc;
     e->p_stale = true;
     if (outs) {   // level n from [v_n; q_n] = x, v_{n-1} = v and c(V_{n-1}) of this step's imex_nonl
-      rc = imex_outputs(e, true, e->x.p, e->v.p, e->x.p + nvb, -1.0 / dt, e->scheme == 0 ? n - 1 : -1);
+      rc = imex_outputs(e, true, e->x.p, e->v.p, e->x.p + nvb, -1.0 / dt, e->scheme == 0 ? n - 1 : -1, n);
       if (rc) return rc;
     }
     rc = imex_push_history(e, guess);
@@ -3231,11 +3319,11 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
   if (!blown && ntimeslices > 0 && ntimeslices * lenofts == loopsteps) {
     // the (empty) remainder slice still runs the guard once
     bool bad = false;
-    int rcb = imex_blowup(e, e->scheme == 1 ? e->vprev.p : e->v.p, check_ff_maxv, &bad);
+    int rcb = imex_blowup(e, e->scheme == 1 ? e->vprev.p : e->v.p, check_ff_maxv, &bad, &retired);
     if (rcb) return rcb;
     if (bad) blown = true;
   }
-  if (blown && ffflag) *ffflag = 1;
+  if ((blown || retired) && ffflag) *ffflag = 1;
   imex_refresh_p(e);
   DNSB_CK(ctx, cudaEventRecord(e->ev1, ctx->stream));
   DNSB_CK(ctx, cudaEventSynchronize(e->ev1));
@@ -3244,14 +3332,21 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
   // convergence of the run: the largest final relative residual over ALL
   // solves and members (the device keeps the running maximum), and the number
   // of solves that stopped at `maxit` above `tol`
+  // (member mode: over the members live at the end of the run)
+  int live_failed = 0;
   {
     double mx = 0.0;
     long long unc = -unc0;
     for (dnsb_solver *sv : run_solvers)
       if (sv) {
-        double r = 0.0;
-        if (solver_relmax(sv, false, &r)) return -1;
-        if (mx == mx && !(r <= mx)) mx = r;
+        std::vector<double> h;
+        if (solver_relmax_members(sv, h)) return -1;
+        for (int m = 0; m < nb; ++m) {
+          if (e->member_guard && e->trip[m] >= 0) continue;
+          const double r = h[m];
+          if (mx == mx && !(r <= mx)) mx = r;   // NaN wins
+          if (!(r <= tol)) ++live_failed;
+        }
         unc += sv->stat_unconverged;
       }
     e->last_relres = mx;
@@ -3260,6 +3355,16 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
   e->run_iters = e->sl->stat_iters - it0;
   e->run_solves = e->sl->stat_solves - ns0;
   DNSB_CK(ctx, cudaGetLastError());
+  if (e->member_guard) {
+    // per-member verdict: a member retired in this run is forgiven its solves, a live one is not
+    if (live_failed == 0) return 0;
+    char msg[240];
+    snprintf(msg, sizeof msg, "a member live at the end of the run has a final relative residual above tol=%.1e "
+             "or a non-finite one (largest over the live members %.3e; FGMRES maxit=%d)", tol, e->last_relres,
+             maxit);
+    ctx->fail(msg, __FILE__, __LINE__);
+    return DNSB_E_NOT_CONVERGED;
+  }
   if (e->last_relres != e->last_relres && !blown) {
     // inf/NaN right-hand sides "converge" trivially (NaN compares false): a blown-up member with
     // the guard of time_int_utils.py:94-103 switched off (ntimeslices = 0) must not pass silently
@@ -3288,6 +3393,35 @@ extern "C" int dnsb_imex_get_state(dnsb_imex *e, double *v, double *p) {
   if (v) DNSB_CK(ctx, cudaMemcpyAsync(v, e->v.p, nvb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   if (p) DNSB_CK(ctx, cudaMemcpyAsync(p, e->p.p, npb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  if (e->nretired == 0) return 0;
+  // retired members: their frozen trip state
+  const int nb = e->nb;
+  std::vector<double> tv(v ? nvb : 0), tp(p ? npb : 0);
+  if (v) DNSB_CK(ctx, cudaMemcpyAsync(tv.data(), e->trip_v.p, nvb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  if (p) DNSB_CK(ctx, cudaMemcpyAsync(tp.data(), e->trip_p.p, npb * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  for (int m = 0; m < nb; ++m) {
+    if (e->trip[m] < 0) continue;
+    if (v) for (size_t i = 0; i < (size_t)e->nv; ++i) v[i * nb + m] = tv[i * nb + m];
+    if (p) for (size_t i = 0; i < (size_t)e->np; ++i) p[i * nb + m] = tp[i * nb + m];
+  }
+  return 0;
+}
+
+extern "C" int dnsb_imex_set_member_guard(dnsb_imex *e, int on) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_REQUIRE(ctx, on || e->nretired == 0,
+               "members are retired: dnsb_imex_set_state makes them live before the stop-all guard can return");
+  e->member_guard = on != 0;
+  return 0;
+}
+
+extern "C" int dnsb_imex_member_status(dnsb_imex *e, int32_t *trip_level) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_REQUIRE(ctx, trip_level != nullptr, "null output");
+  for (int m = 0; m < e->nb; ++m) trip_level[m] = e->trip[m];
   return 0;
 }
 
@@ -3505,10 +3639,11 @@ extern "C" int dnsb_imex_stats(dnsb_imex *e, long long *total_iters, long long *
 
 extern "C" long long dnsb_imex_unconverged(dnsb_imex *e) { return e ? e->run_unconverged : -2; }
 
-// G[a,b] = sum_m sum_i X_a[i,m] * (M X_b)[i,m]
+// G[a,b] = sum_m sum_i X_a[i,m] * (M X_b)[i,m]; trip != null: only the members m with trip[m] < 0 (live)
 __global__ void k_gram_partial(const double *__restrict__ X, size_t xstride,
                                const double *__restrict__ MX,
-                               int ns, size_t nvb, double *__restrict__ partial) {
+                               int ns, size_t nvb, double *__restrict__ partial,
+                               const int *__restrict__ trip, int nb) {
   dnsb_pdl_entry();
   // block (a, b) pair over blockIdx.y; grid-stride chunks over blockIdx.x
   extern __shared__ double sred[];
@@ -3518,7 +3653,12 @@ __global__ void k_gram_partial(const double *__restrict__ X, size_t xstride,
   const size_t chunk = (nvb + gridDim.x - 1) / gridDim.x;
   const size_t i0 = (size_t)blockIdx.x * chunk, i1 = min(nvb, i0 + chunk);
   double acc = 0.0;
-  for (size_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) acc += xa[i] * mb[i];
+  if (trip) {
+    for (size_t i = i0 + threadIdx.x; i < i1; i += blockDim.x)
+      if (trip[i % nb] < 0) acc += xa[i] * mb[i];   // a retired lane may hold NaN: skipped, not weighted
+  } else {
+    for (size_t i = i0 + threadIdx.x; i < i1; i += blockDim.x) acc += xa[i] * mb[i];
+  }
   sred[threadIdx.x] = acc;
   __syncthreads();
   for (int s = blockDim.x >> 1; s > 0; s >>= 1) {
@@ -3559,7 +3699,8 @@ static int imex_gram_impl(dnsb_imex *e, double *g_dev) {
     spmm_dev(ctx, e->M, nullptr, e->snaps.p + (size_t)a * ntb, nullptr, MX.p + (size_t)a * nvb, nb, 1.0, 0.0);
   const int nchunks = 32;
   DNSB_CK(ctx, part.alloc((size_t)nchunks * ns * ns));
-  LAUNCH(ctx, k_gram_partial, dim3(nchunks, ns * ns), 256, 256 * sizeof(double), e->snaps.p, ntb, MX.p, ns, nvb, part.p);
+  LAUNCH(ctx, k_gram_partial, dim3(nchunks, ns * ns), 256, 256 * sizeof(double), e->snaps.p, ntb, MX.p, ns, nvb, part.p,
+         e->nretired > 0 ? (const int *)e->d_trip.p : (const int *)nullptr, nb);
   LAUNCH(ctx, k_reduce_partials2, cdiv((size_t)ns * ns, 32), 1024, 0, (const double *)part.p, nchunks, ns * ns, g_dev);
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   DNSB_CK(ctx, cudaGetLastError());

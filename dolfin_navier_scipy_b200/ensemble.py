@@ -6,8 +6,8 @@ wake with penalised Robin control (`tests/time_dep_nse_bcrob.py:26-34`):
 Members are independent: they are sharded over the GPUs with *no* collective
 on the step path; the only exchange is the all-reduce of the POD snapshot Gram
 matrix ``G = sum_m X_m^T M X_m`` (additive over members, SURVEY.md 8e),
-and the one-off all-gather of the recorded output functionals
-(`gather_outputs`).
+and the one-off all-gathers of the recorded output functionals
+(`gather_outputs`) and of the members' trip levels (`gather_member_status`).
 """
 import numpy as np
 
@@ -15,7 +15,7 @@ from . import problem_setups as dnsps
 from . import time_int_utils as tiu
 
 __all__ = ['cylinder_ensemble', 'shard_members', 'bind_to_gpu_cpus',
-           'gram_allreduce', 'gather_outputs',
+           'gram_allreduce', 'gather_outputs', 'gather_member_status',
            'allreduce_gram', 'pod_from_gram', 'pod_modes']
 
 
@@ -60,7 +60,8 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
                       dt=1./512, scheme='cnab', palpha=1e-5, bccontrol=True,
                       control=np.sin, ntimes=513, t0=0., ctx=None, mesh=None,
                       cheb_steps=4, restart=40, schur_poly=2, coarse_max=4096,
-                      force=False, cv_mat=None, cp_mat=None):
+                      force=False, cv_mat=None, cp_mat=None,
+                      member_guard=False):
     """device integrator for this rank's shard of a Re-sweep ensemble
 
     Returns ``(integ, info)``; ``integ`` is a `time_int_utils.DeviceImex` with
@@ -69,7 +70,9 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
     (``ldsbcinds``, control patches included) and ``cv_mat`` / ``cp_mat`` the
     linear outputs at every time level (`DeviceImex.set_outputs`); the drag
     coefficient is ``2/(rho L Um^2)`` times the x force
-    (`residual_checks.lift_drag_via_residual`).
+    (`residual_checks.lift_drag_via_residual`).  ``member_guard=True``
+    retires a member that trips the blow-up guard and integrates the others
+    on (`DeviceImex.set_member_guard`).
     """
     Re_all = np.linspace(Res[0], Res[1], nmembers)
     lo, hi = shard_members(nmembers, rank, world)
@@ -102,6 +105,8 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
     if bccontrol:
         U[:, 1, :] = control(trange)[:, None]
     integ.set_forcing(B, U)
+    if member_guard:
+        integ.set_member_guard(True)
     if force or cv_mat is not None or cp_mat is not None:
         integ.set_outputs(cv_mat, cp_mat,
                           force_dofs=femp['ldsbcinds'] if force else None,
@@ -149,17 +154,25 @@ def gather_outputs(integ, group=None):
     force=(levels, 2, nmembers))`` as numpy arrays; every rank must have
     recorded the same levels.
     """
+    out = integ.outputs()
+    return {key: _gather_members(np.asarray(out[key], dtype=float), group)
+            for key in ('y', 'force')}
+
+
+def _gather_members(a, group):
+    """all-gather ``a`` (..., nb) of every rank's shard along the last axis
+    in rank order (the contiguous, possibly uneven shards of
+    `shard_members`); ``a`` itself for a single process"""
     import torch
     import torch.distributed as dist
-    out = integ.outputs()
     if not (dist.is_available() and dist.is_initialized()) \
             or dist.get_world_size(group) == 1:
-        return out
+        return a
     world = dist.get_world_size(group)
     rank = dist.get_rank(group)
     dev = torch.device('cuda', torch.cuda.current_device()) \
         if dist.get_backend(group) == 'nccl' else torch.device('cpu')
-    nb = out['force'].shape[2]
+    nb = a.shape[-1]
     cnt = torch.tensor([nb], dtype=torch.int64, device=dev)
     dist.all_reduce(cnt, op=dist.ReduceOp.SUM, group=group)
     nmembers = int(cnt.item())
@@ -168,18 +181,26 @@ def gather_outputs(integ, group=None):
     if sizes[rank] != nb:
         raise ValueError('rank {0} holds {1} members, shard_members gives it '
                          '{2}'.format(rank, nb, sizes[rank]))
-    per = max(sizes)
-    res = {}
-    for key in ('y', 'force'):
-        a = np.asarray(out[key], dtype=float)
-        pad = np.zeros(a.shape[:2] + (per,))
-        pad[:, :, :nb] = a
-        t = torch.from_numpy(pad).to(dev)
-        parts = [torch.empty_like(t) for _ in range(world)]
-        dist.all_gather(parts, t, group=group)
-        res[key] = np.concatenate([p.cpu().numpy()[:, :, :sizes[r]]
-                                   for r, p in enumerate(parts)], axis=2)
-    return res
+    pad = np.zeros(a.shape[:-1] + (max(sizes),), dtype=a.dtype)
+    pad[..., :nb] = a
+    t = torch.from_numpy(pad).to(dev)
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t, group=group)
+    return np.concatenate([p.cpu().numpy()[..., :sizes[r]]
+                           for r, p in enumerate(parts)], axis=-1)
+
+
+def gather_member_status(integ, group=None):
+    """trip levels of the whole ensemble on every rank, in member order
+
+    ``integ.member_status()['trip_level']`` of each rank's shard
+    (`DeviceImex.member_status`; -1 = live), put together by one
+    ``all_gather`` like `gather_outputs`.  Returns ``dict(trip_level=
+    (nmembers,) int, alive=(nmembers,) bool)``.
+    """
+    t = np.asarray(integ.member_status()['trip_level'], dtype=np.int64)
+    t = _gather_members(t, group)
+    return dict(trip_level=t, alive=t < 0)
 
 
 def pod_from_gram(G, energy=0.9999, kmax=None):

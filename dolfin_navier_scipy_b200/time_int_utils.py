@@ -222,7 +222,25 @@ class DeviceImex(object):
         self.dev.bind()       # the loop assembles the convection on this mesh
         return self.engine.run(nsteps, **kw)
 
+    def set_member_guard(self, on=True):
+        """per-member blow-up guard: a member whose ``|v|`` fails the
+        reference's check (``check_ff_maxv``, at the ``ntimeslices`` slice
+        starts of `run`) is retired at that time level -- its state is frozen
+        and `state` returns it, its later outputs and snapshots are NaN, it
+        leaves the Gram matrix -- and the others integrate on.  Retired
+        members stay retired until `set_state`.  Off (the default): the first
+        member that fails ends the run for all."""
+        self.engine.set_member_guard(on)
+
+    def member_status(self):
+        """``dict(trip_level=(nb,) int, alive=(nb,) bool)``; the trip level
+        is -1 for a live member"""
+        t = self.engine.member_status()
+        return dict(trip_level=t, alive=t < 0)
+
     def state(self):
+        """final ``(v (NV, nb), p (NP, nb))``; a retired member's columns
+        hold its state at its trip level"""
         v, p = self.engine.state()
         return v[self.ipv], p[self.ipp]
 
@@ -290,7 +308,8 @@ class DeviceImex(object):
     def outputs(self):
         """``dict(y=(levels, ny, nb), force=(levels, 2, nb))`` recorded since
         `set_state` / `reset_outputs` (members in the order of ``nus``; the
-        force is NaN at levels 0 and 1)"""
+        force is NaN at levels 0 and 1, and every output of a retired member
+        is NaN after its trip level)"""
         y, f = self.engine.outputs(self.ny)
         return dict(y=y, force=f)
 

@@ -218,10 +218,36 @@ int dnsb_imex_set_state(dnsb_imex *e, const double *v0, const double *p0);
  * are stored on the device every `snap_stride` steps (0 = none), including the
  * initial state.  tol/maxit: FGMRES controls; guess: 0 = previous solution,
  * 1 = linear extrapolation, k>=2 = projection onto the last k solutions.
- * ffflag (out): 1 if the blow-up guard tripped (time_int_utils.py:99-103). */
+ * ffflag (out): 1 if the blow-up guard tripped (time_int_utils.py:99-103);
+ * with the per-member guard: 1 if at least one member was retired in this run. */
 int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double tol,
                   int maxit, int guess, double check_ff_maxv, int ntimeslices,
                   int *ffflag);
+/* Per-member blow-up guard.  on = 0 (default): the reference's guard applied
+ * to the ensemble as a whole -- the first member with |v_m| > check_ff_maxv
+ * (or NaN) ends the run for all.  on = 1: the same test, at the same points
+ * (start of each of the ntimeslices slices and of the remainder slice; v_n for
+ * CNAB / IMEX Euler, v_c for SBDF2), is applied to every live member, and a
+ * member that fails is RETIRED: its state (v_n, p_n) is frozen at that time
+ * level (its trip level; what the reference's cnab / sbdftwo returns after
+ * its break) and the others integrate on.  A retired member stays retired
+ * across runs until dnsb_imex_set_state; the run ends at a check that leaves
+ * no member live.  For a retired member:
+ *   dnsb_imex_get_state        returns the frozen trip state;
+ *   dnsb_imex_get_outputs      gives NaN at every level after the trip level;
+ *   snapshots                  hold NaN in its lanes from the trip on (device
+ *                              store and pinned mirror alike);
+ *   dnsb_imex_gram(_dev)       sums over the members live when called only,
+ *                              sum_{m live} X_m^T M X_m, so no NaN of a member
+ *                              retired inside the snapshot window enters G.
+ * Run verdict in this mode: DNSB_E_NOT_CONVERGED only if a member live at the
+ * end of the run has a final relative residual above tol or a non-finite one;
+ * the solves of members retired in the same run are forgiven, no others.
+ * Allowed between runs; switching it off while members are retired is
+ * refused (dnsb_imex_set_state first). */
+int dnsb_imex_set_member_guard(dnsb_imex *e, int on);
+/* trip_level (nb entries): -1 for a live member, else its trip level */
+int dnsb_imex_member_status(dnsb_imex *e, int32_t *trip_level);
 /* device time of the last dnsb_imex_run, measured with CUDA events on the
  * context's stream (milliseconds) */
 double dnsb_imex_last_run_ms(dnsb_imex *e);
@@ -280,11 +306,15 @@ int dnsb_imex_reset_outputs(dnsb_imex *e);
  * member, start-up solves included; NaN if a solve produced one).
  * dnsb_imex_run returns DNSB_E_NOT_CONVERGED when a solve of the run stopped
  * at maxit above tol (unless the blow-up guard fired, which is reported through
- * ffflag like time_int_utils.py:94-103); dnsb_imex_unconverged = how many. */
+ * ffflag like time_int_utils.py:94-103); dnsb_imex_unconverged = how many.
+ * With the per-member guard, max_relres is the largest over the members live
+ * at the end of the run, and dnsb_imex_unconverged still counts every solve
+ * that stopped at maxit with any member above tol. */
 int dnsb_imex_stats(dnsb_imex *e, long long *total_iters, long long *nsolves,
                     double *max_relres);
 long long dnsb_imex_unconverged(dnsb_imex *e);
-/* local POD Gram matrix  G = sum_m X_m^T M X_m  (nsnap x nsnap, row-major)
+/* local POD Gram matrix  G = sum_m X_m^T M X_m  (nsnap x nsnap, row-major;
+ * with retired members the sum runs over the live ones only)
  * written to DEVICE memory g_dev (so that torch.distributed / NCCL can
  * all-reduce it in place) -- stokes_navier_utils.py:136-143 is the only
  * Gram-like op of the reference. */
