@@ -78,6 +78,12 @@ SIGNATURES = {
                            ctypes.POINTER(_i)]),
     'dnsb_imex_set_member_guard': (_i, [_vp, _i]),
     'dnsb_imex_member_status': (_i, [_vp, c_int_p]),
+    'dnsb_imex_set_statistics': (_i, [_vp, _i]),
+    'dnsb_imex_reset_statistics': (_i, [_vp]),
+    'dnsb_imex_get_statistics': (_i, [_vp, ctypes.POINTER(_ll),
+                                      ctypes.POINTER(_ll), ctypes.POINTER(_ll),
+                                      c_dbl_p, c_dbl_p, c_dbl_p, c_dbl_p,
+                                      c_dbl_p]),
     'dnsb_imex_last_run_ms': (_d, [_vp]),
     'dnsb_imex_get_state': (_i, [_vp, c_dbl_p, c_dbl_p]),
     'dnsb_imex_num_snapshots': (_i, [_vp]),
@@ -600,6 +606,34 @@ class ImexEngine(object):
         t = np.empty(self.nb, dtype=np.int32)
         self.ctx.check(self.ctx.lib.dnsb_imex_member_status(self.h, _ip(t)))
         return t
+
+    def set_statistics(self, on):
+        """in-loop field statistics (``dnsb_imex_set_statistics``)"""
+        self.ctx.check(self.ctx.lib.dnsb_imex_set_statistics(self.h,
+                                                             int(bool(on))))
+
+    def reset_statistics(self):
+        self.ctx.check(self.ctx.lib.dnsb_imex_reset_statistics(self.h))
+
+    def statistics(self, nnodes):
+        """``dnsb_imex_get_statistics`` in the device numbering: dict of
+        ``first``, ``last``, ``count`` (nb,), ``v_mean`` (nvf, nb), ``uvcov``
+        (3, nnodes, nb), ``p_mean`` / ``p_var`` (np, nb), ``c_mean`` (nv, nb)"""
+        nb = self.nb
+        first, last = _ll(), _ll()
+        count = np.empty(nb, dtype=np.int64)
+        out = dict(v_mean=np.empty((2*nnodes, nb)),
+                   uvcov=np.empty((3, nnodes, nb)),
+                   p_mean=np.empty((self.np_, nb)),
+                   p_var=np.empty((self.np_, nb)),
+                   c_mean=np.empty((self.nv, nb)))
+        self.ctx.check(self.ctx.lib.dnsb_imex_get_statistics(
+            self.h, ctypes.byref(first), ctypes.byref(last),
+            count.ctypes.data_as(ctypes.POINTER(_ll)), _dp(out['v_mean']),
+            _dp(out['uvcov']), _dp(out['p_mean']), _dp(out['p_var']),
+            _dp(out['c_mean'])))
+        out.update(first=first.value, last=last.value, count=count)
+        return out
 
     def last_run_ms(self):
         return float(self.ctx.lib.dnsb_imex_last_run_ms(self.h))

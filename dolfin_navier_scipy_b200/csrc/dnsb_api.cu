@@ -8,6 +8,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <memory>
 #include <new>
 
@@ -2449,6 +2450,12 @@ struct dnsb_imex {
   int nretired = 0;
   DBuf<int> d_trip;
   DBuf<double> trip_v, trip_p;
+  // in-loop statistics (dnsb_imex_set_statistics): Welford accumulators of the time levels st_first..st_last,
+  // members fastest: st_v (nvf: mean of V in full numbering), st_cov (3 x nnodes: co-moments uu, vv, uv of
+  // the two components of a node), st_pm / st_p2 (np: mean and M2 of p), st_c (nv: mean of c(V)[inv])
+  bool stats_on = false;
+  long long st_first = 0, st_last = -1;
+  DBuf<double> st_v, st_cov, st_pm, st_p2, st_c;
   bool outputs_on() const { return ny > 0 || !fdofs.empty(); }
   ~dnsb_imex() {
     cudaStreamSynchronize(ctx->stream);   // no buffer is freed under a running kernel or copy
@@ -2582,6 +2589,7 @@ extern "C" int dnsb_imex_set_state(dnsb_imex *e, const double *v0, const double 
   e->force_t0 = 0;
   e->nlev = 0; e->csave_level = -1;
   e->trip.assign(e->nb, -1); e->nretired = 0;   // every member is live again
+  e->st_first = 0; e->st_last = -1;
   e->have_state = true;
   e->p_stale = false;
   return 0;
@@ -2671,6 +2679,10 @@ static int retire_nan(dnsb_imex *e, double *x, double *y, size_t n, long long le
   LAUNCH(e->ctx, k_retire_nan, cdiv(n, 256), 256, 0, x, y, n, e->nb, (const int *)e->d_trip.p, level);
   return 0;
 }
+
+// fold time level `level` into the in-loop statistics (defined with its kernel at the end of the file, after
+// every other kernel: ptxas then emits the SASS of all the others exactly as without it)
+static int imex_stats(dnsb_imex *e, long long level, const double *nfc);
 
 // pinned host mirror with room for `cap` snapshots (contents are kept)
 static int imex_reserve_host(dnsb_imex *e, int cap) {
@@ -3199,6 +3211,8 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     const double *u0 = useries_at(e, 0), *u1 = useries_at(e, 1);
     int rc = imex_nonl(e, e->v.p, e->nfc_c.p);                 // nfc(v0)
     if (rc) return rc;
+    rc = imex_stats(e, 0, e->nfc_c.p);
+    if (rc) return rc;
     if (outs && e->scheme == 0) {   // Phi^T c(V_0), before the predictor's convection overwrites it
       rc = imex_outputs(e, false, nullptr, nullptr, nullptr, 0.0, 0, 0);
       if (rc) return rc;
@@ -3264,6 +3278,8 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
       std::swap(e->nfc_o.p, e->nfc_c.p);
       rc = imex_nonl(e, e->v.p, e->nfc_c.p);
       if (rc) return rc;
+      rc = imex_stats(e, n - 1, e->nfc_c.p);
+      if (rc) return rc;
       spmm_dev(ctx, e->Rm.get(), e->coefR.p, e->v.p, nullptr, e->b.p, nb, 1.0, 0.0);
       LAUNCH(ctx, k_rhs_combine, cdiv(nvb, 256), 256, 0, e->b.p, (const double *)e->nfc_c.p, 1.5 * dt,
              (const double *)e->nfc_o.p, -0.5 * dt, (const double *)e->fv.p, dt,
@@ -3271,6 +3287,8 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     } else if (e->scheme == 1) {
       std::swap(e->nfc_o.p, e->nfc_c.p);
       rc = imex_nonl(e, e->v.p, e->nfc_c.p);
+      if (rc) return rc;
+      rc = imex_stats(e, n - 1, e->nfc_c.p);
       if (rc) return rc;
       // rhs = 1/3 M (4 v_c - v_p) + 2/3 dt (2 nfc_c - nfc_p) + 2/3 dt f_n
       LAUNCH(ctx, k_axpby, cdiv(nvb, 256), 256, 0, 4.0 / 3.0, (const double *)e->v.p, -1.0 / 3.0,
@@ -3283,6 +3301,8 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
     } else {
       // IMEX Euler: (M + dt A) v+ = M v + dt (f(t+) + nfc(v))
       rc = imex_nonl(e, e->v.p, e->nfc_c.p);
+      if (rc) return rc;
+      rc = imex_stats(e, n - 1, e->nfc_c.p);
       if (rc) return rc;
       spmm_dev(ctx, e->M, nullptr, e->v.p, nullptr, e->b.p, nb, 1.0, 0.0);
       LAUNCH(ctx, k_rhs_combine, cdiv(nvb, 256), 256, 0, e->b.p, (const double *)e->nfc_c.p, dt,
@@ -3325,6 +3345,13 @@ extern "C" int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double t
   }
   if ((blown || retired) && ffflag) *ffflag = 1;
   imex_refresh_p(e);
+  if (e->stats_on && e->st_last < e->step) {
+    // the final level: its convection into e->tmp, which every step writes before it reads it
+    int rc = imex_nonl(e, e->v.p, e->tmp.p);
+    if (rc) return rc;
+    rc = imex_stats(e, e->step, e->tmp.p);
+    if (rc) return rc;
+  }
   DNSB_CK(ctx, cudaEventRecord(e->ev1, ctx->stream));
   DNSB_CK(ctx, cudaEventSynchronize(e->ev1));
   if (snap_stride > 0 && e->cstream) DNSB_CK(ctx, cudaStreamSynchronize(e->cstream));
@@ -3422,6 +3449,72 @@ extern "C" int dnsb_imex_member_status(dnsb_imex *e, int32_t *trip_level) {
   dnsb_ctx *ctx = e->ctx;
   DNSB_REQUIRE(ctx, trip_level != nullptr, "null output");
   for (int m = 0; m < e->nb; ++m) trip_level[m] = e->trip[m];
+  return 0;
+}
+
+extern "C" int dnsb_imex_set_statistics(dnsb_imex *e, int on) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_CK(ctx, dnsb_enter(ctx));
+  e->stats_on = false;
+  if (!on) {
+    for (DBuf<double> *b : {&e->st_v, &e->st_cov, &e->st_pm, &e->st_p2, &e->st_c}) b->release();
+    return 0;
+  }
+  const size_t nb = e->nb, nnodes = e->nvf / 2;
+  DNSB_CK(ctx, e->st_v.alloc((size_t)e->nvf * nb));
+  DNSB_CK(ctx, e->st_cov.alloc(3 * nnodes * nb));
+  DNSB_CK(ctx, e->st_pm.alloc((size_t)e->np * nb));
+  DNSB_CK(ctx, e->st_p2.alloc((size_t)e->np * nb));
+  DNSB_CK(ctx, e->st_c.alloc((size_t)e->nv * nb));
+  e->stats_on = true;
+  e->st_first = e->step; e->st_last = e->step - 1;
+  return 0;
+}
+
+extern "C" int dnsb_imex_reset_statistics(dnsb_imex *e) {
+  if (!e) return -2;
+  DNSB_REQUIRE(e->ctx, e->stats_on, "statistics are off (dnsb_imex_set_statistics)");
+  e->st_first = e->step; e->st_last = e->step - 1;
+  return 0;
+}
+
+extern "C" int dnsb_imex_get_statistics(dnsb_imex *e, long long *first, long long *last, long long *count,
+                                        double *v_mean, double *uvcov, double *p_mean, double *p_var,
+                                        double *c_mean) {
+  if (!e) return -2;
+  dnsb_ctx *ctx = e->ctx;
+  DNSB_REQUIRE(ctx, e->stats_on, "statistics are off (dnsb_imex_set_statistics)");
+  DNSB_CK(ctx, dnsb_enter(ctx));
+  const int nb = e->nb, nnodes = e->nvf / 2;
+  if (first) *first = e->st_first;
+  if (last) *last = e->st_last;
+  // levels of each member: a retired one stops at its trip level
+  std::vector<long long> cnt(nb);
+  const long long n = e->st_last - e->st_first + 1;
+  for (int m = 0; m < nb; ++m)
+    cnt[m] = e->trip[m] < 0 ? n : std::max(0LL, std::min(n, (long long)e->trip[m] - e->st_first + 1));
+  if (count) for (int m = 0; m < nb; ++m) count[m] = cnt[m];
+  struct Part { double *out; const DBuf<double> *src; size_t rows; bool moment; };
+  const Part parts[] = {{v_mean, &e->st_v, (size_t)e->nvf, false}, {uvcov, &e->st_cov, 3 * (size_t)nnodes, true},
+                        {p_mean, &e->st_pm, (size_t)e->np, false}, {p_var, &e->st_p2, (size_t)e->np, true},
+                        {c_mean, &e->st_c, (size_t)e->nv, false}};
+  for (const Part &q : parts)
+    if (q.out)
+      DNSB_CK(ctx, cudaMemcpyAsync(q.out, q.src->p, q.rows * nb * sizeof(double), cudaMemcpyDeviceToHost,
+                                   ctx->stream));
+  DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
+  // co-moments -> population (co)variances; a member without levels is NaN
+  const double nan = std::numeric_limits<double>::quiet_NaN();
+  for (const Part &q : parts) {
+    if (!q.out) continue;
+    for (size_t i = 0; i < q.rows; ++i)
+      for (int m = 0; m < nb; ++m) {
+        double &x = q.out[i * nb + m];
+        if (cnt[m] == 0) x = nan;
+        else if (q.moment) x /= (double)cnt[m];
+      }
+  }
   return 0;
 }
 
@@ -3704,5 +3797,121 @@ static int imex_gram_impl(dnsb_imex *e, double *g_dev) {
   LAUNCH(ctx, k_reduce_partials2, cdiv((size_t)ns * ns, 32), 1024, 0, (const double *)part.p, nchunks, ns * ns, g_dev);
   DNSB_CK(ctx, cudaStreamSynchronize(ctx->stream));
   DNSB_CK(ctx, cudaGetLastError());
+  return 0;
+}
+
+// ---- in-loop statistics ----------------------------------------------------
+// W consecutive members of row i of an (n, nb) array (W = 2: one 16-byte access)
+template <int W>
+__device__ __forceinline__ void st_load(const double *__restrict__ a, size_t i, int nb, int m, double (&r)[W]) {
+  if constexpr (W == 2) {
+    const double2 t = *reinterpret_cast<const double2 *>(a + i * nb + m);
+    r[0] = t.x; r[1] = t.y;
+  } else {
+    r[0] = a[i * nb + m];
+  }
+}
+template <int W>
+__device__ __forceinline__ void st_store(double *__restrict__ a, size_t i, int nb, int m, const double (&r)[W]) {
+  if constexpr (W == 2) *reinterpret_cast<double2 *>(a + i * nb + m) = make_double2(r[0], r[1]);
+  else a[i * nb + m] = r[0];
+}
+// Fold one time level into the accumulators by an elementwise Welford update with the count k of that level
+// (rk = 1/k; k == 1 writes the values themselves, so the buffers need no clearing).  One thread per W
+// consecutive members of one row of the concatenated index space [nnodes nodes | nv inner dofs | np pressures]:
+//   node i:   u = vfull[2i], v = vfull[2i+1]   ->  mean st_v[2i], st_v[2i+1]; co-moments cov[0|1|2][i] (uu, vv, uv)
+//   inner j:  c = -nfc[j]                      ->  mean cm[j]
+//   press. r: p = ps * pq[r]                   ->  mean pm[r], M2 p2[r]
+// A member retired before `level` (0 <= trip[m] < level) keeps its values.  No reduction: the result does not
+// depend on the launch shape and is bit-reproducible.
+template <int W>
+__global__ void k_imex_stats(const double *__restrict__ vfull, const double *__restrict__ nfc,
+                             const double *__restrict__ pq, double ps, double *__restrict__ vm,
+                             double *__restrict__ cov, double *__restrict__ cm, double *__restrict__ pm,
+                             double *__restrict__ p2, int nnodes, int nv, int np, int nb,
+                             const int *__restrict__ trip, long long level, bool first, double rk) {
+  dnsb_pdl_entry();
+  const int ng = nb / W;
+  const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (size_t)(nnodes + nv + np) * ng) return;
+  const size_t row = t / ng;
+  const int m = (int)(t % ng) * W;
+  bool live[W];
+  for (int w = 0; w < W; ++w) live[w] = !trip || trip[m + w] < 0 || trip[m + w] >= level;
+  if (row < (size_t)nnodes) {
+    const size_t i = row;
+    double u[W], v[W], mu[W], mv[W], cuu[W], cvv[W], cuv[W];
+    st_load<W>(vfull, 2 * i, nb, m, u);
+    st_load<W>(vfull, 2 * i + 1, nb, m, v);
+    st_load<W>(vm, 2 * i, nb, m, mu);
+    st_load<W>(vm, 2 * i + 1, nb, m, mv);
+    st_load<W>(cov, i, nb, m, cuu);
+    st_load<W>(cov, nnodes + i, nb, m, cvv);
+    st_load<W>(cov, 2 * (size_t)nnodes + i, nb, m, cuv);
+    for (int w = 0; w < W; ++w) {
+      if (!live[w]) continue;
+      if (first) {
+        mu[w] = u[w]; mv[w] = v[w]; cuu[w] = 0.0; cvv[w] = 0.0; cuv[w] = 0.0;
+        continue;
+      }
+      const double du = u[w] - mu[w], dv = v[w] - mv[w];
+      mu[w] += du * rk;
+      mv[w] += dv * rk;
+      const double eu = u[w] - mu[w], ev = v[w] - mv[w];
+      cuu[w] += du * eu;
+      cvv[w] += dv * ev;
+      cuv[w] += du * ev;
+    }
+    st_store<W>(vm, 2 * i, nb, m, mu);
+    st_store<W>(vm, 2 * i + 1, nb, m, mv);
+    st_store<W>(cov, i, nb, m, cuu);
+    st_store<W>(cov, nnodes + i, nb, m, cvv);
+    st_store<W>(cov, 2 * (size_t)nnodes + i, nb, m, cuv);
+  } else if (row < (size_t)(nnodes + nv)) {
+    const size_t j = row - nnodes;
+    double c[W], mc[W];
+    st_load<W>(nfc, j, nb, m, c);
+    st_load<W>(cm, j, nb, m, mc);
+    for (int w = 0; w < W; ++w) {
+      if (!live[w]) continue;
+      mc[w] = first ? -c[w] : mc[w] + (-c[w] - mc[w]) * rk;
+    }
+    st_store<W>(cm, j, nb, m, mc);
+  } else {
+    const size_t r = row - nnodes - nv;
+    double p[W], mp[W], q[W];
+    st_load<W>(pq, r, nb, m, p);
+    st_load<W>(pm, r, nb, m, mp);
+    st_load<W>(p2, r, nb, m, q);
+    for (int w = 0; w < W; ++w) {
+      if (!live[w]) continue;
+      const double x = ps * p[w];
+      if (first) { mp[w] = x; q[w] = 0.0; continue; }
+      const double d = x - mp[w];
+      mp[w] += d * rk;
+      q[w] += d * (x - mp[w]);
+    }
+    st_store<W>(pm, r, nb, m, mp);
+    st_store<W>(p2, r, nb, m, q);
+  }
+}
+// fold time level `level` into the statistics, once: vfull holds V_level (Dirichlet values included), nfc =
+// -c(V_level)[inv], and its pressure is e->p, or -q/dt in x while e->p is stale (nothing between the solve and
+// the next imex_guess writes x: imex_push_history / proj_add only read it)
+static int imex_stats(dnsb_imex *e, long long level, const double *nfc) {
+  if (!e->stats_on || level <= e->st_last) return 0;
+  dnsb_ctx *ctx = e->ctx;
+  const int nb = e->nb, nnodes = e->nvf / 2;
+  const size_t nvb = (size_t)e->nv * nb;
+  const double *pq = e->p_stale ? e->x.p + nvb : e->p.p;
+  const double ps = e->p_stale ? -1.0 / e->dt : 1.0;
+  const long long k = level - e->st_first + 1;
+  const int *trip = e->nretired > 0 ? (const int *)e->d_trip.p : (const int *)nullptr;
+  const bool pair = nb % 2 == 0;
+  const size_t nthr = (size_t)(nnodes + e->nv + e->np) * (pair ? nb / 2 : nb);
+  LAUNCH_IF(ctx, pair, k_imex_stats<2>, k_imex_stats<1>, cdiv(nthr, 256), 256, 0, (const double *)e->vfull.p, nfc,
+            pq, ps, e->st_v.p, e->st_cov.p, e->st_c.p, e->st_pm.p, e->st_p2.p, nnodes, e->nv, e->np, nb, trip, level,
+            k == 1, 1.0 / (double)k);
+  e->st_last = level;
   return 0;
 }

@@ -7,7 +7,8 @@ Members are independent: they are sharded over the GPUs with *no* collective
 on the step path; the only exchange is the all-reduce of the POD snapshot Gram
 matrix ``G = sum_m X_m^T M X_m`` (additive over members, SURVEY.md 8e),
 and the one-off all-gathers of the recorded output functionals
-(`gather_outputs`) and of the members' trip levels (`gather_member_status`).
+(`gather_outputs`), of the members' trip levels (`gather_member_status`) and
+of their field statistics (`gather_statistics`).
 """
 import numpy as np
 
@@ -16,6 +17,7 @@ from . import time_int_utils as tiu
 
 __all__ = ['cylinder_ensemble', 'shard_members', 'bind_to_gpu_cpus',
            'gram_allreduce', 'gather_outputs', 'gather_member_status',
+           'gather_statistics',
            'allreduce_gram', 'pod_from_gram', 'pod_modes']
 
 
@@ -61,7 +63,7 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
                       control=np.sin, ntimes=513, t0=0., ctx=None, mesh=None,
                       cheb_steps=4, restart=40, schur_poly=2, coarse_max=4096,
                       force=False, cv_mat=None, cp_mat=None,
-                      member_guard=False):
+                      member_guard=False, statistics=False):
     """device integrator for this rank's shard of a Re-sweep ensemble
 
     Returns ``(integ, info)``; ``integ`` is a `time_int_utils.DeviceImex` with
@@ -72,7 +74,10 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
     coefficient is ``2/(rho L Um^2)`` times the x force
     (`residual_checks.lift_drag_via_residual`).  ``member_guard=True``
     retires a member that trips the blow-up guard and integrates the others
-    on (`DeviceImex.set_member_guard`).
+    on (`DeviceImex.set_member_guard`).  ``statistics=True`` accumulates
+    the mean flow, the velocity and pressure fluctuation intensities and the
+    mean convection of every member inside the loop
+    (`DeviceImex.set_statistics`).
     """
     Re_all = np.linspace(Res[0], Res[1], nmembers)
     lo, hi = shard_members(nmembers, rank, world)
@@ -107,6 +112,8 @@ def cylinder_ensemble(N=4, Res=(60., 150.), nmembers=64, rank=0, world=1,
     integ.set_forcing(B, U)
     if member_guard:
         integ.set_member_guard(True)
+    if statistics:
+        integ.set_statistics(True)
     if force or cv_mat is not None or cp_mat is not None:
         integ.set_outputs(cv_mat, cp_mat,
                           force_dofs=femp['ldsbcinds'] if force else None,
@@ -201,6 +208,23 @@ def gather_member_status(integ, group=None):
     t = np.asarray(integ.member_status()['trip_level'], dtype=np.int64)
     t = _gather_members(t, group)
     return dict(trip_level=t, alive=t < 0)
+
+
+def gather_statistics(integ, group=None):
+    """field statistics of the whole ensemble on every rank, in member order
+
+    ``integ.statistics()`` of each rank's shard (`DeviceImex.statistics`),
+    every per-member array put together along the member axis by one
+    ``all_gather`` like `gather_outputs`; ``first_level`` and ``last_level``
+    are this rank's (every rank must have run the same levels).
+    """
+    s = integ.statistics()
+    out = dict(first_level=s['first_level'], last_level=s['last_level'])
+    out['count'] = _gather_members(np.asarray(s['count'], dtype=np.int64),
+                                   group)
+    for key in ('v_mean', 'uu', 'vv', 'uv', 'p_mean', 'p_var', 'c_mean'):
+        out[key] = _gather_members(np.asarray(s[key], dtype=float), group)
+    return out
 
 
 def pod_from_gram(G, energy=0.9999, kmax=None):

@@ -238,6 +238,48 @@ class DeviceImex(object):
         t = self.engine.member_status()
         return dict(trip_level=t, alive=t < 0)
 
+    def set_statistics(self, on=True):
+        """accumulate field statistics of every member inside the loop
+
+        From the current time level on (from level 0 after `set_state`),
+        every level a run passes through -- its final level included -- is
+        folded into per-member means and second moments by one device kernel
+        per level; nothing moves to the host until `statistics`.  ``on=True``
+        while on restarts the window; ``on=False`` frees the accumulators.
+        Off (the default) leaves the loop unchanged."""
+        self.engine.set_statistics(on)
+
+    def reset_statistics(self):
+        """restart the statistics window at the current time level"""
+        self.engine.reset_statistics()
+
+    def statistics(self):
+        """field statistics of the window, in the caller's numbering
+
+        ``dict(first_level, last_level, count=(nb,), v_mean=(NVf, nb),
+        uu, vv, uv=(nnodes, nb), p_mean, p_var=(NP, nb), c_mean=(NV, nb))``:
+        the mean of the full velocity (Dirichlet values included), the
+        population covariances of the two velocity components at each P2
+        node, mean and variance of the pressure and the mean of the
+        convection ``c(V)[invinds]`` (the sign of `dts.get_convvec`) over the
+        levels ``first_level..last_level``.  A member retired by the
+        per-member guard counts its levels up to its trip level only; a
+        member with ``count == 0`` has NaN fields."""
+        s = self.engine.statistics(self.dev.nvf//2)
+        cov = s['uvcov']
+        return dict(first_level=s['first'], last_level=s['last'],
+                    count=s['count'], v_mean=s['v_mean'], uu=cov[0],
+                    vv=cov[1], uv=cov[2], p_mean=s['p_mean'][self.ipp],
+                    p_var=s['p_var'][self.ipp], c_mean=s['c_mean'][self.ipv])
+
+    def mean_flow_forcing(self, stats=None):
+        """Reynolds-stress forcing ``mean(c(V)) - c(mean V)`` on the inner
+        dofs (NV, nb), from `statistics` (or ``stats``, its result): the
+        forcing under which the mean flow solves the steady equations"""
+        s = self.statistics() if stats is None else stats
+        cbar = self.dev.convvec(s['v_mean'])
+        return s['c_mean'] - cbar[self.invinds]
+
     def state(self):
         """final ``(v (NV, nb), p (NP, nb))``; a retired member's columns
         hold its state at its trip level"""

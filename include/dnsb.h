@@ -248,6 +248,35 @@ int dnsb_imex_run(dnsb_imex *e, int nsteps, int snap_stride, double tol,
 int dnsb_imex_set_member_guard(dnsb_imex *e, int on);
 /* trip_level (nb entries): -1 for a live member, else its trip level */
 int dnsb_imex_member_status(dnsb_imex *e, int32_t *trip_level);
+/* Field statistics of every member accumulated inside the loop, one
+ * elementwise Welford update per time level that only reads the state.
+ * on = 1 switches them on (or, when on already, restarts the window); on = 0
+ * (default) frees them, and with them off the loop is unchanged.
+ * Window: it starts at the current time level at dnsb_imex_set_statistics(1)
+ * and dnsb_imex_reset_statistics, and at level 0 at dnsb_imex_set_state.  After
+ * a run it holds every level from its first level through the run's final
+ * level, inclusive (first, last); a run that continues the trajectory
+ * continues the window without gap or double count.  When the stop-all guard
+ * trips, the run's final level is the state the run returns.  The Heun levels 0
+ * and 1 of CNAB / SBDF2 are ordinary levels.
+ * Per member m with count[m] levels (divisors are the count, population
+ * statistics):
+ *   v_mean (nvf*nb)        mean of the full velocity V (Dirichlet values
+ *                          included, full numbering 2*node + comp);
+ *   uvcov (3, nnodes, nb)  per P2 node, the covariances uu, vv, uv of its two
+ *                          components;
+ *   p_mean, p_var (np*nb)  mean and variance of the pressure p = -q/dt;
+ *   c_mean (nv*nb)         mean of the convection c(V)[inv] on the inner dofs
+ *                          (the sign of dts.get_convvec).
+ * p and c are in the device numbering.  A member retired by the per-member
+ * guard counts the levels up to its trip level only (0 if it was retired
+ * before the window); a member with count 0 has NaN fields.  Any output may be
+ * NULL; reset and get are refused while the statistics are off. */
+int dnsb_imex_set_statistics(dnsb_imex *e, int on);
+int dnsb_imex_reset_statistics(dnsb_imex *e);
+int dnsb_imex_get_statistics(dnsb_imex *e, long long *first, long long *last, long long *count,
+                             double *v_mean, double *uvcov, double *p_mean, double *p_var,
+                             double *c_mean);
 /* device time of the last dnsb_imex_run, measured with CUDA events on the
  * context's stream (milliseconds) */
 double dnsb_imex_last_run_ms(dnsb_imex *e);
